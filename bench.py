@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """Benchmark of the DFMI readout hot path (BASELINE.json: NLS fit buffers/s; demod HBM GB/s vs peak).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--no-configs]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--no-configs] [--dump-outputs DIR]
 
 Headline workload (config.workload): BASELINE config 2, "long single channel" -- f_mod = 1 kHz, f_samp = 1 MHz,
 3600 s of synthetic 'snr'-mode DFMI (m = 6, 40 dB), n = 20 periods per buffer (R = 20000 samples), N = 10
@@ -20,6 +20,11 @@ configs       (N = 1) the other four BASELINE configs measured in the same proce
               cfg 1, cfg 3 (one resident wave), cfg 4 (the whole 100 s, streamed slab by slab), cfg 5
 strong        (N > 1) ONE cfg-2 record, and one cfg-3 wave, split over the N GPUs: wall time incl. seed broadcast
               and row gather
+
+--dump-outputs DIR writes what the last timed step computed, rank 0's result columns (amp, m, phi, psi, dc, ssq,
+fitok: 180 000 float64 each, 10 MB in all) as DIR/<column>.npy.  The record is generated from a fixed seed, so two
+builds run with the same arguments can be compared output for output (on hosts with the same core count: the
+warm-start schedule, SCHED, follows it).
 """
 import argparse
 import json
@@ -708,6 +713,16 @@ def strong_scaling(torch, dist, ctx, local, rank, world, w0, opts, single_gpu_ms
 
 
 # ---- GPU arm --------------------------------------------------------------------------------------------
+def dump_outputs(out_dir, rows):
+    """The frame's columns of the row table (what StandardNLSFitter.fit returns for the record) as <column>.npy."""
+    import numpy as np
+    from deepfmkit_b200.fitters import RESULT_COLUMNS
+    os.makedirs(out_dir, exist_ok=True)
+    table = rows.cpu().numpy()
+    for i, name in enumerate(RESULT_COLUMNS):
+        np.save(os.path.join(out_dir, name + ".npy"), np.ascontiguousarray(table[:, i], dtype=np.float64))
+
+
 def run_gpu(args):
     import numpy as np
     import torch
@@ -774,6 +789,8 @@ def run_gpu(args):
         ctx.profile_enable(False)
         counters = ctx.lm_counters(reset=True)
         head = rows[:4096].cpu().numpy()
+        if args.dump_outputs and rank == 0:
+            dump_outputs(args.dump_outputs, rows)
         fp64_peak = ctx.probe_fp64_tflops() if rank == 0 else None
 
     # sanity: the timed work produced real fits
@@ -923,9 +940,13 @@ def main():
                     help="reference arm only: which BASELINE config's bounded CPU sample to time (default: the contract's cfg2)")
     ap.add_argument("--no-configs", action="store_true", help="skip the cfg 1/3/4/5 block of the N = 1 line")
     ap.add_argument("--no-strong", action="store_true", help="skip the strong-scaling block of the N > 1 line")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the last timed step's result columns (rank 0) to DIR/<column>.npy, float64")
     args = ap.parse_args()
     if args.steps < 1 or args.warmup < 0:
         raise SystemExit("--steps must be >= 1 and --warmup >= 0")
+    if args.dump_outputs and args.impl == "reference":
+        raise SystemExit("--dump-outputs applies to the GPU arm, not --impl reference")
     if args.impl == "reference":
         return run_reference(args)
     return run_gpu(args)

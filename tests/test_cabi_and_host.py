@@ -294,13 +294,13 @@ def test_bench_reference_arm_contract():
 
 
 def test_reference_facade_dispatches_to_b200_fitters(lib, tmp_path):
-    """INTEGRATION.md section 1 on the real thing: the unmodified reference (when its checkout is present, i.e. in the
-    build container) with its two fitter classes swapped for ours.  The facade reaches our C ABI: here, without a
-    GPU, that shows as the library's loud 'no CUDA device' error; the frame-level parity of the same call is what
-    `-m gpu` tests check against fixtures minted from this very reference."""
-    ref = os.environ.get("DFK_REFERENCE", "/root/reference")
-    if not os.path.isdir(ref):
-        pytest.skip("reference checkout not present on this machine")
+    """INTEGRATION.md section 1 on the real thing: the unmodified reference (a DeepFMKit checkout named by
+    DFK_REFERENCE; it is not part of this repository) with its two fitter classes swapped for ours.  The facade reaches
+    our C ABI: without a GPU, that shows as the library's loud 'no CUDA device' error; the frame-level parity of the
+    same call is what `-m gpu` tests check against fixtures minted from this very reference."""
+    ref = os.environ.get("DFK_REFERENCE")
+    if not ref or not os.path.isdir(ref):
+        pytest.skip("set DFK_REFERENCE to a DeepFMKit checkout to run this test")
     from unittest.mock import MagicMock
     saved = {k: sys.modules.get(k) for k in ("matplotlib", "matplotlib.pyplot", "matplotlib.colors",
                                              "matplotlib.dates", "matplotlib.cm", "pyplnoise")}
