@@ -399,7 +399,9 @@ __global__ void trial_stats_finish(const double* __restrict__ values, long long 
     r.std = cnt > 0.0 ? sqrt(q / cnt) : nan;
     r.min = cnt > 0.0 ? mn : nan;
     r.max = cnt > 0.0 ? mx : nan;
-    r.worst = cnt > 0.0 ? values[(point * ntrials + far_t) * col_stride + c] : nan;
+    // far < 0: no trial had a finite distance (a column holding both +inf and -inf has a NaN mean; a NaN centre),
+    // so far_t still holds its sentinel and there is no trial to report
+    r.worst = (cnt > 0.0 && far >= 0.0) ? values[(point * ntrials + far_t) * col_stride + c] : nan;
     r.count = cnt;
     out[i] = r;
 }

@@ -433,7 +433,9 @@ int launch_demod(dfk_ctx* ctx, const double* x, int64_t nbuf, int64_t bpc, int64
 int launch_demod_tm(dfk_ctx* ctx, const double* x, int64_t nbuf_t, int64_t C, int64_t R, int32_t N, double w0, double* qi,
                     double* dc, cudaStream_t st) {
     if (nbuf_t == 0 || C == 0) return DFK_OK;
-    const dfk::DemodPlan pl = dfk::make_demod_plan(R, w0, N);
+    dfk::DemodPlan pl = dfk::make_demod_plan(R, w0, N);
+    const int env_drift = dev_int("DFK_FOLD_DRIFT", -1);  // development override, as in launch_demod
+    if (env_drift >= 0) pl.drift = env_drift != 0;
     const int64_t Pc = pl.P * C, Rc = R * C;
     if (!pl.folded || (Pc & 1) || Pc > dfk::kMaxFoldPeriod || Rc > std::numeric_limits<int>::max() ||
         (reinterpret_cast<uintptr_t>(x) & 15u) != 0)

@@ -135,7 +135,9 @@ __global__ void stats_finish_kernel(const double* __restrict__ acc, long long C,
     stats[2 * c + 1] = acc[3 * c + 2] / acc[3 * c];
 }
 
-constexpr int kEkfStateStride = 32;  // doubles per channel in a carried state: x[5], P[25], r, spare
+// doubles per channel in a carried state: x at [0, 5), the covariance's upper triangle at [5, 20) in tri(i, j) order
+// (EkfState::P, the pending update applied), [20, 30) unused, r at [30], [31] unused
+constexpr int kEkfStateStride = 32;
 
 struct EkfLaunch {
     long long k0;   // absolute index of the first sample of this call (a multiple of R)

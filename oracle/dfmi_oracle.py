@@ -352,25 +352,28 @@ EKF_Q_DIAG = (1e-8, 1e-8, 1e-6, 1e-6, 1e-8)
 def ekf_track(x: np.ndarray, f_samp: float, f_mod: float, n: int,
               init_a: float = 1.6, init_m: float = 6.0, init_phi: float = 0.0, init_psi: float = 0.0,
               p0_diag=EKF_P0_DIAG, q_diag=EKF_Q_DIAG, r_val: float | None = None,
-              init_dc: float | None = None) -> np.ndarray:
+              init_dc: float | None = None, k0: int = 0, init_cov=None) -> np.ndarray:
     """5-state random-walk EKF with scalar measurement, state snapshot every R samples.
 
     State [a, m, phi, psi, dc]; time is absolute, t_k = k / f_samp (fitters.py:263).
     Returns rows[nbuf,7] with ssq = 0 and fitok = 1 (fitters.py:313-318).
+    k0 and init_cov are not reference options either: x is then the part of a longer record that starts at sample k0
+    (t_k = (k0 + k) / f_samp), and the filter resumes from the full 5x5 covariance init_cov instead of diag(p0_diag),
+    which is how a continuation slab of the GPU's streamed entry point is checked.
     """
     z = np.asarray(x, dtype=float).ravel()
     R, _, nbuf = buffer_geometry(len(z), f_samp, f_mod, n)
     # init_dc is not a reference option: it lets tests of the slab-wise GPU entry point start the filter from the
     # first slab's mean, as that entry point does (the reference always uses the whole record's mean).
     state = np.array([init_a, init_m, init_phi, init_psi, np.mean(z) if init_dc is None else init_dc])
-    cov = np.diag(p0_diag).astype(float)
+    cov = np.diag(p0_diag).astype(float) if init_cov is None else np.array(init_cov, dtype=float).reshape(5, 5)
     q_mat = np.diag(q_diag).astype(float)
     if r_val is None:
         r_val = np.var(z)
     r_mat = np.array([[r_val]])
     eye = np.eye(5)
     w_m = 2 * np.pi * f_mod
-    t_axis = np.arange(len(z)) / f_samp
+    t_axis = (int(k0) + np.arange(len(z))) / f_samp
     snaps = np.zeros((nbuf, 5))
     for k in range(len(z)):
         cov = eye @ cov @ eye.T + q_mat  # fitters.py:276 (F = I)

@@ -115,6 +115,18 @@ def test_ekf_full_record_bit_exact(golden, name):
     assert np.array_equal(rows, g["rows"])
 
 
+@pytest.mark.parametrize("name", ["ekf_default", "ekf_offset"])
+def test_ekf_resume_options_at_their_defaults_are_bit_exact(golden, name):
+    """k0 = 0 and init_cov = None (or the same diagonal given as a full matrix) leave the filter the reference's."""
+    g = golden(name)
+    kw = ekf_kwargs(g)
+    rows = orc.ekf_track(g["x"], 200e3, 1000.0, 20, k0=0, init_cov=None, **kw)
+    assert np.array_equal(rows, g["rows"])
+    cov = np.diag(kw.get("p0_diag", orc.EKF_P0_DIAG))
+    rows = orc.ekf_track(g["x"], 200e3, 1000.0, 20, init_cov=cov, **kw)
+    assert np.array_equal(rows, g["rows"])
+
+
 def test_crlb_helper_is_finite():
     s = orc.crlb_sigma_m(6.0, 10, 40.0, 4000)
     assert 1e-5 < s < 1e-2
