@@ -1,5 +1,5 @@
 #!/usr/bin/env python
-"""A/B of the cfg-5 pipeline pieces (development tool): generator shapes, single-period demod, cold LM variants."""
+"""Timings of the cfg-5 pipeline pieces (development tool): generator shapes, single-period demod, the cold LM kernel."""
 import json
 import os
 import sys
@@ -25,7 +25,6 @@ def timed(fn, reps=5):
 def main():
     ctx = _lib.Context(0)
     ctx.use_torch_stream()
-    lib = _lib.load_library()
     what = sys.argv[1:] or ["synth", "lm"]
     if "synth" in what:
         x = torch.empty(1_600_000_000, dtype=torch.float64, device="cuda")
@@ -48,15 +47,8 @@ def main():
         guess = torch.from_numpy(g).cuda()
         rows = torch.zeros((C, 8), dtype=torch.float64, device="cuda")
         opts = _lib.default_lm_opts()
-        ref = None
-        for mode in (4, 5, 6):
-            lib.dfk_dev_clear(); lib.dfk_dev_set(b"DFK_LM_FLAT_MINB", mode)
-            t = timed(lambda: ctx.lm_fit(qi.data_ptr(), C, nd, guess.data_ptr(), 4, dc.data_ptr(), opts, rows.data_ptr()))
-            r = rows.clone()
-            same = True if ref is None else bool(torch.equal(r[:, :7], ref[:, :7]))
-            ref = r if ref is None else ref
-            print(json.dumps({"what": f"lm_flat minb={mode}", "ms": t, "Mfits_per_s": C / t / 1e3, "same_rows": same}), flush=True)
-        lib.dfk_dev_clear()
+        t = timed(lambda: ctx.lm_fit(qi.data_ptr(), C, nd, guess.data_ptr(), 4, dc.data_ptr(), opts, rows.data_ptr()))
+        print(json.dumps({"what": "lm_flat", "ms": t, "Mfits_per_s": C / t / 1e3}), flush=True)
     ctx.close()
 
 

@@ -1,5 +1,5 @@
 #!/usr/bin/env python
-"""Consumer warps x ring depth of the single-period lock-in kernel (development tool)."""
+"""Ring depth of the single-period lock-in kernel (development tool)."""
 import json, os, sys
 import numpy as np
 import torch
@@ -14,17 +14,16 @@ def main():
     ctx.synth_snr_dev(x.data_ptr(), R, C, 200e3, 1000.0, 6.0, seed=5)
     qi = torch.empty((C, 2 * N), dtype=torch.float64, device="cuda"); dc = torch.empty(C, dtype=torch.float64, device="cuda")
     ref = None
-    for warps in (8, 6, 10):
-        for nst in (12, 8, 6, 5):
-            lib.dfk_dev_clear(); lib.dfk_dev_set(b"DFK_PERIOD_WARPS", warps); lib.dfk_dev_set(b"DFK_PERIOD_NSTAGES", nst)
-            best = 1e30
-            for _ in range(4):
-                a, b = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
-                a.record(); ctx.demod(x.data_ptr(), C, R, N, 2 * np.pi / 200, qi.data_ptr(), dc.data_ptr()); b.record(); b.synchronize()
-                best = min(best, a.elapsed_time(b))
-            same = True if ref is None else bool(torch.equal(qi, ref))
-            ref = qi.clone() if ref is None else ref
-            print(json.dumps({"warps": warps, "nstages_max": nst, "ms": best, "GBps": C * (R * 8 + 8 * (2 * N + 1)) / best / 1e6, "same": same}), flush=True)
+    for nst in (12, 8, 6, 5):
+        lib.dfk_dev_clear(); lib.dfk_dev_set(b"DFK_PERIOD_NSTAGES", nst)
+        best = 1e30
+        for _ in range(4):
+            a, b = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
+            a.record(); ctx.demod(x.data_ptr(), C, R, N, 2 * np.pi / 200, qi.data_ptr(), dc.data_ptr()); b.record(); b.synchronize()
+            best = min(best, a.elapsed_time(b))
+        same = True if ref is None else bool(torch.equal(qi, ref))
+        ref = qi.clone() if ref is None else ref
+        print(json.dumps({"nstages_max": nst, "ms": best, "GBps": C * (R * 8 + 8 * (2 * N + 1)) / best / 1e6, "same": same}), flush=True)
     lib.dfk_dev_clear()
 
 if __name__ == "__main__":

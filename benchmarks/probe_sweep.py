@@ -19,8 +19,6 @@ def main():
     lib = _lib.load_library()
     if len(sys.argv) > 2:
         lib.dfk_dev_set(b"DFK_NO_SWEEP_FUSE", int(sys.argv[2]))
-    if len(sys.argv) > 3:  # consumer warps x 100 + generator warps: 88, 79, 610, 511
-        lib.dfk_dev_set(b"DFK_SWEEP_SHAPE", int(sys.argv[3]))
     for rep in range(3):
         ctx.profile_enable(True)
         ctx.profile_read(reset=True)

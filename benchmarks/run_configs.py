@@ -163,11 +163,6 @@ def main():
                 _lib.load_library().dfk_dev_set(b"DFK_EKF_CPW", cpw)
                 ekf_case(ctx, f"cfg4 cpw={cpw}", 4096, 0.25, 2, False)
             _lib.load_library().dfk_dev_clear()
-        elif c == "cfg4unroll":
-            for u in (1, 2, 4):
-                _lib.load_library().dfk_dev_set(b"DFK_EKF_UNROLL", u)
-                ekf_case(ctx, f"cfg4 unroll={u}", 4096, 0.25, 2, False)
-            _lib.load_library().dfk_dev_clear()
         elif c == "cfg4small":
             ekf_case(ctx, "cfg4small", 4096, 0.1, 1, False)
             ekf_case(ctx, "cfg4small", 4096, 0.1, 1, True)

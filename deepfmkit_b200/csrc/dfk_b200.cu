@@ -64,6 +64,29 @@ dfk::LmOpts to_opts(const dfk_lm_opts* o) {
     return r;
 }
 
+// Every kernel launch of this file but the FP64 probe's: raise the kernel's dynamic shared-memory limit to what this
+// launch uses, launch it on st, count it (dfk_launch_count) and report a launch error.
+template <class... Params, class... Args>
+int launch_kernel(dfk_ctx* ctx, void (*kernel)(Params...), dim3 grid, dim3 block, size_t smem, cudaStream_t st,
+                  const Args&... args) {
+    if (smem) DFK_CUDA(cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, static_cast<int>(smem)));
+    kernel<<<grid, block, smem, st>>>(args...);
+    ctx->launches++;
+    DFK_CUDA(cudaGetLastError());
+    return DFK_OK;
+}
+
+// The deepest ring of 2..deepest stages whose shared memory, smem_of(stages), fits one CTA less `reserve` bytes:
+// its depth, or 0 when not even two stages fit; its size goes to *smem.
+template <class SmemOf>
+int ring_depth(const dfk_ctx* ctx, int deepest, size_t reserve, SmemOf smem_of, size_t* smem) {
+    for (int nst = deepest; nst >= 2; --nst) {
+        *smem = smem_of(nst);
+        if (*smem <= static_cast<size_t>(ctx->max_smem_optin) - reserve) return nst;
+    }
+    return 0;
+}
+
 // ---- demodulation -------------------------------------------------------------------------------
 // Shared memory left free on every SM next to a persistent demod CTA so that one block of the cold seed fits
 // (Bessel columns: (N+2) x 128 doubles) can co-reside and overlap with it; given up when it would cost the
@@ -73,13 +96,40 @@ size_t seed_fit_reserve(int N) {
     return need <= 24 * 1024 ? need : 0;
 }
 
+// The lock-in plan of R-sample buffers; the development override DFK_FOLD_DRIFT forces the drift term on or off.
+dfk::DemodPlan demod_plan(int64_t R, double w0, int N) {
+    dfk::DemodPlan pl = dfk::make_demod_plan(R, w0, N);
+    const int forced = dev_int("DFK_FOLD_DRIFT", -1);
+    if (forced >= 0) pl.drift = forced != 0;
+    return pl;
+}
+
+// The fields of the fold kernels' parameters that do not depend on the launch geometry (pps, nstages).
+dfk::FoldParams fold_params(const dfk::DemodPlan& pl, const double* x, int64_t nbuf, int64_t bpc, int64_t ld_c, int64_t R,
+                            int64_t P, int N, double* qi, double* dc) {
+    dfk::FoldParams p;
+    p.x = x;
+    p.qi = qi;
+    p.dc = dc;
+    p.nbuf = nbuf;
+    p.bpc = bpc;
+    p.ld_c = ld_c;
+    p.R = static_cast<int>(R);
+    p.P = static_cast<int>(P);
+    p.periods = static_cast<int>(pl.periods);
+    p.N = N;
+    p.kmul = pl.kmul;
+    for (int k = 0; k < dfk::kMaxHarmonics; ++k) p.delta[k] = pl.delta[k];
+    return p;
+}
+
 struct FoldGeometry {
     int pps, nstages;
     size_t smem;
     int ctas_per_sm;
 };
 
-bool fold_geometry(const dfk_ctx* ctx, const dfk::DemodPlan& pl, int N, bool leave_room, FoldGeometry* g) {
+bool fold_geometry(const dfk_ctx* ctx, const dfk::DemodPlan& pl, int N, size_t reserve, FoldGeometry* g) {
     const int P = static_cast<int>(pl.P);
     // development overrides (tuning runs only): DFK_FOLD_STAGE_BYTES, DFK_FOLD_NSTAGES, DFK_FOLD_CTAS
     const int env_stage = dev_int("DFK_FOLD_STAGE_BYTES", 0), env_nst = dev_int("DFK_FOLD_NSTAGES", 0),
@@ -109,9 +159,8 @@ bool fold_geometry(const dfk_ctx* ctx, const dfk::DemodPlan& pl, int N, bool lea
     int best_stage = 0;
     bool found = false;
     for (int ctas = 2; ctas >= 1; --ctas) {
-        const size_t room = leave_room ? seed_fit_reserve(N) : 0;
-        const size_t budget = ctas == 2 ? (static_cast<size_t>(ctx->smem_per_sm) - room) / 2 - 1024
-                                        : static_cast<size_t>(ctx->max_smem_optin) - room;
+        const size_t budget = ctas == 2 ? (static_cast<size_t>(ctx->smem_per_sm) - reserve) / 2 - 1024
+                                        : static_cast<size_t>(ctx->max_smem_optin) - reserve;
         for (int target : stage_targets) {
             int q = target / (P * 8);
             if (q < 1) q = 1;
@@ -137,84 +186,41 @@ bool fold_geometry(const dfk_ctx* ctx, const dfk::DemodPlan& pl, int N, bool lea
     return found;
 }
 
-template <bool DRIFT, int SLOTS>
-int launch_fold_t(const dfk::FoldParams& p, size_t smem, int grid, cudaStream_t st) {
-    DFK_CUDA(cudaFuncSetAttribute(dfk::demod_fold_kernel<DRIFT, SLOTS>, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                  static_cast<int>(smem)));
-    dfk::demod_fold_kernel<DRIFT, SLOTS><<<grid, dfk::kFoldThreads, smem, st>>>(p);
-    return DFK_OK;
-}
-
-template <bool DRIFT, int NBW>
-int launch_tile_t(dfk_ctx* ctx, const dfk::TileParams& p, size_t smem, int grid, cudaStream_t st) {
-    DFK_CUDA(cudaFuncSetAttribute(dfk::demod_tile_kernel<DRIFT, NBW>, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                  static_cast<int>(smem)));
-    dfk::demod_tile_kernel<DRIFT, NBW><<<grid, dfk::kFoldThreads, smem, st>>>(p);
-    (void)ctx;
-    return DFK_OK;
-}
-
-// One period per buffer (R == P <= 256, P % 4 == 0, no drift term): the quarter-wave kernel.  1 = launched, 0 = does not fit.
-template <int WARPS>
-int launch_period_t(dfk_ctx* ctx, dfk::PeriodParams p, bool leave_room, int64_t ngroups, cudaStream_t st) {
-    int nst = dev_int("DFK_PERIOD_NSTAGES", WARPS);  // a stage per consumer warp: measured flat from 6 stages up
-    size_t smem = 0;
-    for (; nst >= 2; --nst) {
-        smem = dfk::period_smem_layout(p.P, p.N, nst, WARPS).total;
-        if (smem <= static_cast<size_t>(ctx->max_smem_optin) - (leave_room ? seed_fit_reserve(p.N) : 0)) break;
-    }
-    if (nst < 2) return 0;
-    p.nstages = nst;
-    const int grid = static_cast<int>(std::min<int64_t>(ngroups, ctx->sm_count));
-    DFK_CUDA(cudaFuncSetAttribute(dfk::demod_period_kernel<WARPS>, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                  static_cast<int>(smem)));
-    dfk::demod_period_kernel<WARPS><<<grid, (WARPS + 1) * 32, smem, st>>>(p);
-    return 1;
-}
-
+// One period per buffer (R == P <= 256, P % 4 == 0, no drift term): the quarter-wave kernel.  Returns 1 if it
+// launched, 0 if the geometry does not fit it, < 0 on error.
 int try_launch_period(dfk_ctx* ctx, const dfk::DemodPlan& pl, const double* x, int64_t nbuf, int32_t N, double* qi,
-                      double* dc, bool leave_room, cudaStream_t st) {
-    if (pl.periods != 1 || pl.kmul != 1 || pl.drift || pl.P > dfk::kTileMaxPeriod || (pl.P % 4) != 0 || dev_int("DFK_NO_PERIOD", 0))
-        return 0;
+                      double* dc, size_t reserve, cudaStream_t st) {
+    if (pl.periods != 1 || pl.kmul != 1 || pl.drift || pl.P > dfk::kTileMaxPeriod || (pl.P % 4) != 0) return 0;
     if (reinterpret_cast<uintptr_t>(qi) & 15u) return 0;  // the kernel stores harmonic vectors 128 bits at a time
-    dfk::PeriodParams p;
-    p.x = x;
-    p.qi = qi;
-    p.dc = dc;
-    p.nbuf = nbuf;
-    p.P = static_cast<int>(pl.P);
-    p.N = N;
-    p.nstages = 0;
+    const int P = static_cast<int>(pl.P);
+    size_t smem = 0;
+    // a stage per consumer warp: measured flat from 6 stages up
+    const int nst = ring_depth(ctx, dev_int("DFK_PERIOD_NSTAGES", dfk::kPeriodWarps), reserve,
+                               [&](int n) { return dfk::period_smem_layout(P, N, n).total; }, &smem);
+    if (nst == 0) return 0;
+    const dfk::PeriodParams p = {x, qi, dc, nbuf, P, N, nst};
     const int64_t ngroups = (nbuf + dfk::kPeriodNbw - 1) / dfk::kPeriodNbw;
-    // consumer warps against ring depth: each warp's scratch costs one stage's worth of shared memory
-    switch (dev_int("DFK_PERIOD_WARPS", dfk::kPeriodWarps)) {
-        case 6: return launch_period_t<6>(ctx, p, leave_room, ngroups, st);
-        case 10: return launch_period_t<10>(ctx, p, leave_room, ngroups, st);
-        case 12: return launch_period_t<12>(ctx, p, leave_room, ngroups, st);
-        default: return launch_period_t<8>(ctx, p, leave_room, ngroups, st);
-    }
+    const int grid = static_cast<int>(std::min<int64_t>(ngroups, ctx->sm_count));
+    const int rc =
+        launch_kernel(ctx, dfk::demod_period_kernel<dfk::kPeriodWarps>, grid, (dfk::kPeriodWarps + 1) * 32, smem, st, p);
+    return rc ? rc : 1;
 }
 
 // Short periods (P <= 256) with contiguous buffers: the barrier-free tile kernel.  Returns 1 if it launched,
 // 0 if the geometry does not fit it, < 0 on error.
 int try_launch_tile(dfk_ctx* ctx, const dfk::DemodPlan& pl, const double* x, int64_t nbuf, int64_t R, int32_t N,
-                    double* qi, double* dc, bool leave_room, cudaStream_t st) {
+                    double* qi, double* dc, size_t reserve, cudaStream_t st) {
     if (pl.P > dfk::kTileMaxPeriod || dev_int("DFK_NO_TILE", 0)) return 0;
     const int P = static_cast<int>(pl.P), n = static_cast<int>(pl.periods);
     int nbw = 8;
     while (nbw > 1 && static_cast<int64_t>(nbw) * R * 8 > dfk::kTileStageBytes) nbw >>= 1;
-    const int env_nbw = dev_int("DFK_TILE_NBW", 0);  // development override
-    if (env_nbw == 1 || env_nbw == 2 || env_nbw == 4 || env_nbw == 8) nbw = env_nbw;
     int pps = dfk::kTileStageBytes / (P * 8);
     if (pps < 1) pps = 1;
     if (pps > nbw * n) pps = nbw * n;
-    int nst = dev_int("DFK_TILE_NSTAGES", 12);
     size_t smem = 0;
-    for (; nst >= 2; --nst) {
-        smem = dfk::tile_smem_layout(P, N, nbw, pps, nst, pl.drift).total;
-        if (smem <= static_cast<size_t>(ctx->max_smem_optin) - (leave_room ? seed_fit_reserve(N) : 0)) break;
-    }
-    if (nst < 2) return 0;
+    const int nst = ring_depth(ctx, dev_int("DFK_TILE_NSTAGES", 12), reserve,
+                               [&](int s) { return dfk::tile_smem_layout(P, N, nbw, pps, s, pl.drift).total; }, &smem);
+    if (nst == 0) return 0;
     dfk::TileParams p;
     p.x = x;
     p.qi = qi;
@@ -231,23 +237,38 @@ int try_launch_tile(dfk_ctx* ctx, const dfk::DemodPlan& pl, const double* x, int
     for (int k = 0; k < dfk::kMaxHarmonics; ++k) p.delta[k] = pl.delta[k];
     const int64_t ngroups = (nbuf + nbw - 1) / nbw;
     const int grid = static_cast<int>(std::min<int64_t>(ngroups, ctx->sm_count));
+    auto tile = [&](auto kernel) { return launch_kernel(ctx, kernel, grid, dfk::kFoldThreads, smem, st, p); };
     int rc;
     if (pl.drift) {
         switch (nbw) {
-            case 8: rc = launch_tile_t<true, 8>(ctx, p, smem, grid, st); break;
-            case 4: rc = launch_tile_t<true, 4>(ctx, p, smem, grid, st); break;
-            case 2: rc = launch_tile_t<true, 2>(ctx, p, smem, grid, st); break;
-            default: rc = launch_tile_t<true, 1>(ctx, p, smem, grid, st); break;
+            case 8: rc = tile(dfk::demod_tile_kernel<true, 8>); break;
+            case 4: rc = tile(dfk::demod_tile_kernel<true, 4>); break;
+            case 2: rc = tile(dfk::demod_tile_kernel<true, 2>); break;
+            default: rc = tile(dfk::demod_tile_kernel<true, 1>); break;
         }
     } else {
         switch (nbw) {
-            case 8: rc = launch_tile_t<false, 8>(ctx, p, smem, grid, st); break;
-            case 4: rc = launch_tile_t<false, 4>(ctx, p, smem, grid, st); break;
-            case 2: rc = launch_tile_t<false, 2>(ctx, p, smem, grid, st); break;
-            default: rc = launch_tile_t<false, 1>(ctx, p, smem, grid, st); break;
+            case 8: rc = tile(dfk::demod_tile_kernel<false, 8>); break;
+            case 4: rc = tile(dfk::demod_tile_kernel<false, 4>); break;
+            case 2: rc = tile(dfk::demod_tile_kernel<false, 2>); break;
+            default: rc = tile(dfk::demod_tile_kernel<false, 1>); break;
         }
     }
     return rc ? rc : 1;
+}
+
+// Fold lengths beyond the register kernel: column chunks of 2048, 32 kB stages (two period slices), as deep a ring as
+// one CTA per SM holds.  STORE: the folded arrays go to p.qi and p.dc instead of the harmonics (time-major records).
+template <bool STORE>
+int launch_fold_long(dfk_ctx* ctx, dfk::FoldParams p, bool drift, size_t reserve, cudaStream_t st) {
+    p.pps = std::min(2, p.periods);
+    size_t smem = 0;
+    p.nstages = ring_depth(ctx, 6, reserve, [&](int n) { return dfk::fold_long_smem_layout(p.pps, n, p.N, drift).total; },
+                           &smem);
+    if (p.nstages == 0) return fail(DFK_ERR_ARG, "no shared memory for the long-period fold");
+    const int grid = static_cast<int>(std::min<int64_t>(p.nbuf, ctx->sm_count));
+    return drift ? launch_kernel(ctx, dfk::demod_fold_long_kernel<true, STORE>, grid, dfk::kFoldThreads, smem, st, p)
+                 : launch_kernel(ctx, dfk::demod_fold_long_kernel<false, STORE>, grid, dfk::kFoldThreads, smem, st, p);
 }
 
 // nbuf buffers in channel records of bpc buffers each, records ld_c samples apart
@@ -256,24 +277,18 @@ int try_launch_tile(dfk_ctx* ctx, const dfk::DemodPlan& pl, const double* x, int
 // harmonics per pass; a piece is the buffer when a CTA's table can hold its steps, else a 16 384-sample chunk of it.
 template <int KB, int THREADS>
 int launch_direct_one(dfk_ctx* ctx, const dfk::DirectParams& q, size_t smem, int per_sm, cudaStream_t st) {
-    auto kernel = dfk::demod_direct_kernel<KB, THREADS>;
-    DFK_CUDA(cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, static_cast<int>(smem)));
     const int64_t warps_per_cta = THREADS / 32, npieces = q.nbuf * q.cpb;
     const int grid = static_cast<int>(std::max<int64_t>(1, std::min<int64_t>((npieces + warps_per_cta - 1) / warps_per_cta,
                                                                             static_cast<int64_t>(ctx->sm_count) * per_sm)));
-    kernel<<<grid, THREADS, smem, st>>>(q);
-    return DFK_OK;
+    return launch_kernel(ctx, dfk::demod_direct_kernel<KB, THREADS>, grid, THREADS, smem, st, q);
 }
 
 template <int KB, int THREADS>
 int launch_direct_pair(dfk_ctx* ctx, const dfk::DirectParams& q, size_t smem, cudaStream_t st) {
-    auto kernel = dfk::demod_direct_pair_kernel<KB, THREADS>;
-    DFK_CUDA(cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, static_cast<int>(smem)));
     const int64_t warps_per_cta = THREADS / 32, npairs = (q.nbuf * q.cpb + 1) / 2;
     const int grid = static_cast<int>(std::max<int64_t>(1, std::min<int64_t>((npairs + warps_per_cta - 1) / warps_per_cta,
                                                                             static_cast<int64_t>(ctx->sm_count))));
-    kernel<<<grid, THREADS, smem, st>>>(q);
-    return DFK_OK;
+    return launch_kernel(ctx, dfk::demod_direct_pair_kernel<KB, THREADS>, grid, THREADS, smem, st, q);
 }
 
 template <int KB>
@@ -287,7 +302,7 @@ int launch_direct_t(dfk_ctx* ctx, const dfk::DirectParams& q, cudaStream_t st) {
     const int per_sm = static_cast<int>(std::max<size_t>(1, std::min<size_t>(4, static_cast<size_t>(ctx->smem_per_sm) / (smem + 1024))));
     // one CTA per SM (a long table): 512 threads, which the 128 registers of the narrower builds allow
     if constexpr (KB <= 12) {
-        if (per_sm == 1 && dev_int("DFK_DIRECT_THREADS", 512) == 512) return launch_direct_one<KB, 512>(ctx, q, smem, per_sm, st);
+        if (per_sm == 1) return launch_direct_one<KB, 512>(ctx, q, smem, per_sm, st);
     }
     return launch_direct_one<KB, dfk::kDirectThreads>(ctx, q, smem, per_sm, st);
 }
@@ -318,111 +333,48 @@ int launch_direct(dfk_ctx* ctx, const double* x, int64_t nbuf, int64_t bpc, int6
         case 12: rc = launch_direct_t<12>(ctx, p, st); break;
         default: rc = launch_direct_t<16>(ctx, p, st); break;
     }
-    if (rc) return rc;
-    if (p.cpb > 1) {
-        const int64_t n = nbuf * (N + 1);
-        dfk::direct_combine_kernel<<<static_cast<unsigned>((n + 127) / 128), 128, 0, st>>>(p);
-        ctx->launches++;
-    }
-    return DFK_OK;
+    if (rc || p.cpb == 1) return rc;
+    const int64_t n = nbuf * (N + 1);
+    return launch_kernel(ctx, dfk::direct_combine_kernel, static_cast<unsigned>((n + 127) / 128), 128, 0, st, p);
 }
 
 int launch_demod(dfk_ctx* ctx, const double* x, int64_t nbuf, int64_t bpc, int64_t ld_c, int64_t R, int32_t N, double w0,
                  double* qi, double* dc, cudaStream_t st, bool leave_room = false) {
     if (nbuf == 0) return DFK_OK;
-    dfk::DemodPlan pl = dfk::make_demod_plan(R, w0, N);
-    const int env_drift = dev_int("DFK_FOLD_DRIFT", -1);  // development override
-    if (env_drift >= 0) pl.drift = env_drift != 0;
+    const dfk::DemodPlan pl = demod_plan(R, w0, N);
+    const size_t reserve = leave_room ? seed_fit_reserve(N) : 0;
+    const bool fold = pl.folded && (reinterpret_cast<uintptr_t>(x) & 15u) == 0 && (ld_c % 2) == 0;
+    if (fold && ld_c == bpc * R) {
+        int tiled = try_launch_period(ctx, pl, x, nbuf, N, qi, dc, reserve, st);
+        if (tiled == 0) tiled = try_launch_tile(ctx, pl, x, nbuf, R, N, qi, dc, reserve, st);
+        if (tiled) return tiled < 0 ? tiled : DFK_OK;
+    }
+    const bool fold_int = fold && R <= std::numeric_limits<int>::max();
+    if (fold_int && pl.P > dfk::kFoldRegisterPeriod && !dev_int("DFK_NO_FOLD_LONG", 0))
+        return launch_fold_long<false>(ctx, fold_params(pl, x, nbuf, bpc, ld_c, R, pl.P, N, qi, dc), pl.drift, reserve, st);
     FoldGeometry g;
-    const bool aligned = (reinterpret_cast<uintptr_t>(x) & 15u) == 0 && (ld_c % 2) == 0;
-    int tiled = 0;
-    if (pl.folded && aligned && ld_c == bpc * R) {
-        tiled = try_launch_period(ctx, pl, x, nbuf, N, qi, dc, leave_room, st);
-        if (tiled == 0) tiled = try_launch_tile(ctx, pl, x, nbuf, R, N, qi, dc, leave_room, st);
-        if (tiled < 0) return tiled;
+    if (!(fold_int && pl.P <= dfk::kFoldRegisterPeriod && fold_geometry(ctx, pl, N, reserve, &g)))
+        return launch_direct(ctx, x, nbuf, bpc, ld_c, R, N, w0, qi, dc, st);
+    dfk::FoldParams p = fold_params(pl, x, nbuf, bpc, ld_c, R, pl.P, N, qi, dc);
+    p.pps = g.pps;
+    p.nstages = g.nstages;
+    const int grid = static_cast<int>(std::min<int64_t>(nbuf, static_cast<int64_t>(ctx->sm_count) * g.ctas_per_sm));
+    const int slots = (p.P / 2 + dfk::kFoldConsumers - 1) / dfk::kFoldConsumers;
+    auto fold_t = [&](auto kernel) { return launch_kernel(ctx, kernel, grid, dfk::kFoldThreads, g.smem, st, p); };
+    if (pl.drift) {
+        switch (slots) {
+            case 1: return fold_t(dfk::demod_fold_kernel<true, 1>);
+            case 2: return fold_t(dfk::demod_fold_kernel<true, 2>);
+            case 3: return fold_t(dfk::demod_fold_kernel<true, 3>);
+            default: return fold_t(dfk::demod_fold_kernel<true, 4>);
+        }
     }
-    if (tiled) {
-        // launched above
-    } else if (pl.folded && aligned && R <= std::numeric_limits<int>::max() && pl.P > dfk::kFoldRegisterPeriod &&
-               !dev_int("DFK_NO_FOLD_LONG", 0)) {
-        // fold lengths beyond the register kernel: column chunks of 2048, 32 kB stages (two period slices), as deep
-        // a ring as one CTA per SM holds
-        dfk::FoldParams p;
-        p.x = x;
-        p.qi = qi;
-        p.dc = dc;
-        p.nbuf = nbuf;
-        p.bpc = bpc;
-        p.ld_c = ld_c;
-        p.R = static_cast<int>(R);
-        p.P = static_cast<int>(pl.P);
-        p.periods = static_cast<int>(pl.periods);
-        p.N = N;
-        p.kmul = pl.kmul;
-        p.pps = static_cast<int>(std::min<int64_t>(2, pl.periods));
-        for (int k = 0; k < dfk::kMaxHarmonics; ++k) p.delta[k] = pl.delta[k];
-        const size_t room = leave_room ? seed_fit_reserve(N) : 0;
-        int nst = 6;
-        size_t smem = 0;
-        for (; nst >= 2; --nst) {
-            smem = dfk::fold_long_smem_layout(p.pps, nst, N, pl.drift).total;
-            if (smem <= static_cast<size_t>(ctx->max_smem_optin) - room) break;
-        }
-        if (nst < 2) return fail(DFK_ERR_ARG, "no shared memory for the long-period demodulation");
-        p.nstages = nst;
-        const int grid = static_cast<int>(std::min<int64_t>(nbuf, ctx->sm_count));
-        if (pl.drift) {
-            DFK_CUDA(cudaFuncSetAttribute(dfk::demod_fold_long_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                          static_cast<int>(smem)));
-            dfk::demod_fold_long_kernel<true><<<grid, dfk::kFoldThreads, smem, st>>>(p);
-        } else {
-            DFK_CUDA(cudaFuncSetAttribute(dfk::demod_fold_long_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                          static_cast<int>(smem)));
-            dfk::demod_fold_long_kernel<false><<<grid, dfk::kFoldThreads, smem, st>>>(p);
-        }
-    } else if (pl.folded && aligned && R <= std::numeric_limits<int>::max() && pl.P <= dfk::kFoldRegisterPeriod &&
-               fold_geometry(ctx, pl, N, leave_room, &g)) {
-        dfk::FoldParams p;
-        p.x = x;
-        p.qi = qi;
-        p.dc = dc;
-        p.nbuf = nbuf;
-        p.bpc = bpc;
-        p.ld_c = ld_c;
-        p.R = static_cast<int>(R);
-        p.P = static_cast<int>(pl.P);
-        p.periods = static_cast<int>(pl.periods);
-        p.N = N;
-        p.kmul = pl.kmul;
-        p.pps = g.pps;
-        p.nstages = g.nstages;
-        for (int k = 0; k < dfk::kMaxHarmonics; ++k) p.delta[k] = pl.delta[k];
-        const int grid = static_cast<int>(std::min<int64_t>(nbuf, static_cast<int64_t>(ctx->sm_count) * g.ctas_per_sm));
-        const int slots = (p.P / 2 + dfk::kFoldConsumers - 1) / dfk::kFoldConsumers;
-        int rc;
-        if (pl.drift) {
-            switch (slots) {
-                case 1: rc = launch_fold_t<true, 1>(p, g.smem, grid, st); break;
-                case 2: rc = launch_fold_t<true, 2>(p, g.smem, grid, st); break;
-                case 3: rc = launch_fold_t<true, 3>(p, g.smem, grid, st); break;
-                default: rc = launch_fold_t<true, 4>(p, g.smem, grid, st); break;
-            }
-        } else {
-            switch (slots) {
-                case 1: rc = launch_fold_t<false, 1>(p, g.smem, grid, st); break;
-                case 2: rc = launch_fold_t<false, 2>(p, g.smem, grid, st); break;
-                case 3: rc = launch_fold_t<false, 3>(p, g.smem, grid, st); break;
-                default: rc = launch_fold_t<false, 4>(p, g.smem, grid, st); break;
-            }
-        }
-        if (rc) return rc;
-    } else {
-        const int rc_direct = launch_direct(ctx, x, nbuf, bpc, ld_c, R, N, w0, qi, dc, st);
-        if (rc_direct) return rc_direct;
+    switch (slots) {
+        case 1: return fold_t(dfk::demod_fold_kernel<false, 1>);
+        case 2: return fold_t(dfk::demod_fold_kernel<false, 2>);
+        case 3: return fold_t(dfk::demod_fold_kernel<false, 3>);
+        default: return fold_t(dfk::demod_fold_kernel<false, 4>);
     }
-    ctx->launches++;
-    DFK_CUDA(cudaGetLastError());
-    return DFK_OK;
 }
 
 // ---- LM -------------------------------------------------------------------------------------------
@@ -433,9 +385,7 @@ int launch_demod(dfk_ctx* ctx, const double* x, int64_t nbuf, int64_t bpc, int64
 int launch_demod_tm(dfk_ctx* ctx, const double* x, int64_t nbuf_t, int64_t C, int64_t R, int32_t N, double w0, double* qi,
                     double* dc, cudaStream_t st) {
     if (nbuf_t == 0 || C == 0) return DFK_OK;
-    dfk::DemodPlan pl = dfk::make_demod_plan(R, w0, N);
-    const int env_drift = dev_int("DFK_FOLD_DRIFT", -1);  // development override, as in launch_demod
-    if (env_drift >= 0) pl.drift = env_drift != 0;
+    const dfk::DemodPlan pl = demod_plan(R, w0, N);
     const int64_t Pc = pl.P * C, Rc = R * C;
     if (!pl.folded || (Pc & 1) || Pc > dfk::kMaxFoldPeriod || Rc > std::numeric_limits<int>::max() ||
         (reinterpret_cast<uintptr_t>(x) & 15u) != 0)
@@ -448,47 +398,12 @@ int launch_demod_tm(dfk_ctx* ctx, const double* x, int64_t nbuf_t, int64_t C, in
     double* ft = pl.drift ? fs + fold_doubles : fs;
     double* delta_dev = static_cast<double*>(ctx->post[7].ptr);
     DFK_CUDA(cudaMemcpyAsync(delta_dev, pl.delta, sizeof(double) * dfk::kMaxHarmonics, cudaMemcpyHostToDevice, st));
-    dfk::FoldParams p;
-    p.x = x;
-    p.qi = fs;
-    p.dc = ft;
-    p.nbuf = nbuf_t;
-    p.bpc = nbuf_t;
-    p.ld_c = 0;
-    p.R = static_cast<int>(Rc);
-    p.P = static_cast<int>(Pc);
-    p.periods = static_cast<int>(pl.periods);
-    p.N = N;
-    p.kmul = pl.kmul;
-    p.pps = static_cast<int>(std::min<int64_t>(2, pl.periods));
-    for (int k = 0; k < dfk::kMaxHarmonics; ++k) p.delta[k] = pl.delta[k];
-    int nst = 6;
-    size_t smem = 0;
-    for (; nst >= 2; --nst) {
-        smem = dfk::fold_long_smem_layout(p.pps, nst, N, pl.drift).total;
-        if (smem <= static_cast<size_t>(ctx->max_smem_optin)) break;
-    }
-    if (nst < 2) return fail(DFK_ERR_ARG, "no shared memory for the time-major fold");
-    p.nstages = nst;
-    const int grid = static_cast<int>(std::min<int64_t>(nbuf_t, ctx->sm_count));
-    const int64_t units = nbuf_t * C;
-    const unsigned pgrid = static_cast<unsigned>((units + 127) / 128);
-    if (pl.drift) {
-        DFK_CUDA(cudaFuncSetAttribute(dfk::demod_fold_long_kernel<true, true>, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                      static_cast<int>(smem)));
-        dfk::demod_fold_long_kernel<true, true><<<grid, dfk::kFoldThreads, smem, st>>>(p);
-        dfk::project_interleaved_kernel<true><<<pgrid, 128, 0, st>>>(fs, ft, nbuf_t, static_cast<int>(C), static_cast<int>(pl.P),
-                                                                      static_cast<int>(R), N, pl.kmul, delta_dev, qi, dc);
-    } else {
-        DFK_CUDA(cudaFuncSetAttribute(dfk::demod_fold_long_kernel<false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                      static_cast<int>(smem)));
-        dfk::demod_fold_long_kernel<false, true><<<grid, dfk::kFoldThreads, smem, st>>>(p);
-        dfk::project_interleaved_kernel<false><<<pgrid, 128, 0, st>>>(fs, ft, nbuf_t, static_cast<int>(C), static_cast<int>(pl.P),
-                                                                       static_cast<int>(R), N, pl.kmul, delta_dev, qi, dc);
-    }
-    ctx->launches += 2;
-    DFK_CUDA(cudaGetLastError());
-    return DFK_OK;
+    rc = launch_fold_long<true>(ctx, fold_params(pl, x, nbuf_t, nbuf_t, 0, Rc, Pc, N, fs, ft), pl.drift, 0, st);
+    if (rc) return rc;
+    const unsigned pgrid = static_cast<unsigned>((nbuf_t * C + 127) / 128);
+    return launch_kernel(ctx, pl.drift ? dfk::project_interleaved_kernel<true> : dfk::project_interleaved_kernel<false>, pgrid,
+                         128, 0, st, fs, ft, nbuf_t, static_cast<int>(C), static_cast<int>(pl.P), static_cast<int>(R), N,
+                         pl.kmul, delta_dev, qi, dc);
 }
 
 int pick_lanes(const dfk_ctx* ctx, int64_t nfit, int N, int requested) {
@@ -508,8 +423,6 @@ int launch_first_b(dfk_ctx* ctx, const double* qi, int64_t nfit, dfk::FitMap map
                    const dfk::LmOpts& o, double* rows, int* list, int* count, dfk::LmCounts* counters, cudaStream_t st,
                    int* flags) {
     const size_t smem = static_cast<size_t>(N + 2) * TPB * sizeof(double);
-    DFK_CUDA(cudaFuncSetAttribute(dfk::lm_first_kernel<G, MINB, TPB>, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                  static_cast<int>(smem)));
     // keep the SM's L1/shared split at "all shared": a block of this kernel may share an SM with a demod CTA that
     // needs > 200 kB, and an SM only changes its carve-out when it is idle
     // (only the one-warp-block variant, which is the one that overlaps a demod launch: the bulk variant wants its L1)
@@ -519,35 +432,18 @@ int launch_first_b(dfk_ctx* ctx, const double* qi, int64_t nfit, dfk::FitMap map
     const int64_t fits_per_block = TPB / G;
     const int64_t blocks = (nfit + fits_per_block - 1) / fits_per_block;
     const int grid = static_cast<int>(std::min<int64_t>(blocks, static_cast<int64_t>(ctx->sm_count) * 16));
-    dfk::lm_first_kernel<G, MINB, TPB><<<grid, TPB, smem, st>>>(qi, nfit, map, N, gs, dc, o, rows, list, count, counters, flags);
-    ctx->launches++;
-    DFK_CUDA(cudaGetLastError());
-    return DFK_OK;
+    return launch_kernel(ctx, dfk::lm_first_kernel<G, MINB, TPB>, grid, TPB, smem, st, qi, nfit, map, N, gs, dc, o, rows, list,
+                         count, counters, flags);
 }
 
-template <int MINB>
-int launch_flat_b(dfk_ctx* ctx, const double* qi, int64_t nfit, dfk::FitMap map, int N, const dfk::GuessSrc& gs, const double* dc,
-                  const dfk::LmOpts& o, double* rows, int* list, int* count, dfk::LmCounts* counters, cudaStream_t st) {
-    const size_t smem = static_cast<size_t>(N + 2 + dfk::kNeDoubles) * dfk::kLmThreads * sizeof(double);
-    DFK_CUDA(cudaFuncSetAttribute(dfk::lm_flat_kernel<MINB>, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                  static_cast<int>(smem)));
-    const int64_t blocks = (nfit + dfk::kLmThreads - 1) / dfk::kLmThreads;
-    const int per_sm = dev_int("DFK_LM_FLAT_BLOCKS", MINB);
-    const int grid = static_cast<int>(std::min<int64_t>(blocks, static_cast<int64_t>(ctx->sm_count) * per_sm));
-    dfk::lm_flat_kernel<MINB><<<grid, dfk::kLmThreads, smem, st>>>(qi, nfit, map, N, gs, dc, o, rows, list, count, counters);
-    ctx->launches++;
-    DFK_CUDA(cudaGetLastError());
-    return DFK_OK;
-}
-
+// The per-lane state machine: its one build, four 128-thread blocks per SM
 int launch_flat(dfk_ctx* ctx, const double* qi, int64_t nfit, dfk::FitMap map, int N, const dfk::GuessSrc& gs, const double* dc,
                 const dfk::LmOpts& o, double* rows, int* list, int* count, dfk::LmCounts* counters, cudaStream_t st) {
-    switch (dev_int("DFK_LM_FLAT_MINB", 4)) {
-        case 5: return launch_flat_b<5>(ctx, qi, nfit, map, N, gs, dc, o, rows, list, count, counters, st);
-        case 6: return launch_flat_b<6>(ctx, qi, nfit, map, N, gs, dc, o, rows, list, count, counters, st);
-        case 8: return launch_flat_b<8>(ctx, qi, nfit, map, N, gs, dc, o, rows, list, count, counters, st);
-        default: return launch_flat_b<4>(ctx, qi, nfit, map, N, gs, dc, o, rows, list, count, counters, st);
-    }
+    const size_t smem = static_cast<size_t>(N + 2 + dfk::kNeDoubles) * dfk::kLmThreads * sizeof(double);
+    const int64_t blocks = (nfit + dfk::kLmThreads - 1) / dfk::kLmThreads;
+    const int grid = static_cast<int>(std::min<int64_t>(blocks, static_cast<int64_t>(ctx->sm_count) * 4));
+    return launch_kernel(ctx, dfk::lm_flat_kernel<4>, grid, dfk::kLmThreads, smem, st, qi, nfit, map, N, gs, dc, o, rows, list,
+                         count, counters);
 }
 
 template <int G>
@@ -578,7 +474,8 @@ int ensure_counters(dfk_ctx* ctx) {
 // max_unit: largest unit index + 1 the launch can touch (sizes the retry list).
 // cold: the guesses are not expected to be near the solutions, so the fits of a warp will need very different
 // numbers of steps -- measured, the per-lane state machine (lm_flat_kernel) is 1.56x faster than the lock-step
-// kernel on 4e6 cold N = 15 fits, but 0.84x on warm ones, hence the switch.
+// kernel on 4e6 cold N = 15 fits, but 0.84x on warm ones, hence the switch.  (DFK_LM_FLAT = 0 puts cold fits on the
+// lock-step kernel, for tests.)
 int launch_lm(dfk_ctx* ctx, const double* qi, int64_t nfit, dfk::FitMap map, int N, const dfk::GuessSrc& gs,
               const double* dc, const dfk_lm_opts* opts, double* rows, cudaStream_t st, bool cold = false,
               const dfk::ChainPlan* chain = nullptr) {
@@ -604,7 +501,7 @@ int launch_lm(dfk_ctx* ctx, const double* qi, int64_t nfit, dfk::FitMap map, int
     if (requested == 0 && nfit <= 2 * static_cast<int64_t>(ctx->sm_count)) {
         // a handful of fits: one warp per fit in one-warp blocks, spread over all SMs
         rc = launch_first_b<32, 4, 32>(ctx, qi, nfit, map, N, gs, dc, o, rows, list, count, counters, st, flags);
-    } else if (G == 1 && !chain && (cold ? dev_int("DFK_LM_FLAT", 1) != 0 : dev_int("DFK_LM_FLAT", 0) == 2)) {
+    } else if (G == 1 && !chain && cold && dev_int("DFK_LM_FLAT", 1) != 0) {
         rc = launch_flat(ctx, qi, nfit, map, N, gs, dc, o, rows, list, count, counters, st);
     } else
     switch (G) {
@@ -620,36 +517,25 @@ int launch_lm(dfk_ctx* ctx, const double* qi, int64_t nfit, dfk::FitMap map, int
     const int64_t warps = dfk::kLmThreads / 32;
     if (chain) {
         if (map.step != 1 || map.offset != 0 || map.row_mul != 1) return fail(DFK_ERR_ARG, "chain schedule needs contiguous units");
-        DFK_CUDA(cudaFuncSetAttribute(dfk::lm_chain_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                      static_cast<int>(smem)));
         DFK_CUDA(cudaFuncSetAttribute(dfk::lm_chain_kernel, cudaFuncAttributePreferredSharedMemoryCarveout,
                                       cudaSharedmemCarveoutMaxShared));
         const int64_t spans = (nfit + 31) / 32;  // a warp scans 32 units at a time
         const int grid = static_cast<int>(std::min<int64_t>((spans + warps - 1) / warps, static_cast<int64_t>(ctx->sm_count) * 8));
-        dfk::lm_chain_kernel<<<grid, dfk::kLmThreads, smem, st>>>(qi, nfit, N, o, *chain, rows, flags, counters);
-        ctx->launches++;
-        DFK_CUDA(cudaGetLastError());
-        return DFK_OK;
+        return launch_kernel(ctx, dfk::lm_chain_kernel, grid, dfk::kLmThreads, smem, st, qi, nfit, N, o, *chain, rows, flags,
+                             counters);
     }
-    DFK_CUDA(cudaFuncSetAttribute(dfk::lm_retry_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                  static_cast<int>(smem)));
     DFK_CUDA(cudaFuncSetAttribute(dfk::lm_retry_kernel, cudaFuncAttributePreferredSharedMemoryCarveout,
                                   cudaSharedmemCarveoutMaxShared));
     const int grid = static_cast<int>(std::min<int64_t>((nfit + warps - 1) / warps, static_cast<int64_t>(ctx->sm_count) * 8));
-    dfk::lm_retry_kernel<<<grid, dfk::kLmThreads, smem, st>>>(qi, N, o, map.row_mul, rows, list, count, counters);
-    ctx->launches++;
-    DFK_CUDA(cudaGetLastError());
-    if (nfit >= dfk::kFlatRetryMin) {  // enough fits that many may be parked: the thread-per-fit retry kernel stands by
-        const size_t fsmem = static_cast<size_t>(N + 2 + dfk::kNeDoubles) * dfk::kLmThreads * sizeof(double);
-        DFK_CUDA(cudaFuncSetAttribute(dfk::lm_retry_flat_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                      static_cast<int>(fsmem)));
-        const int fgrid = static_cast<int>(std::min<int64_t>((nfit + dfk::kLmThreads - 1) / dfk::kLmThreads,
-                                                             static_cast<int64_t>(ctx->sm_count) * 3));
-        dfk::lm_retry_flat_kernel<<<fgrid, dfk::kLmThreads, fsmem, st>>>(qi, N, o, map.row_mul, rows, list, count, counters);
-        ctx->launches++;
-        DFK_CUDA(cudaGetLastError());
-    }
-    return DFK_OK;
+    rc = launch_kernel(ctx, dfk::lm_retry_kernel, grid, dfk::kLmThreads, smem, st, qi, N, o, map.row_mul, rows, list, count,
+                       counters);
+    if (rc || nfit < dfk::kFlatRetryMin) return rc;
+    // enough fits that many may be parked: the thread-per-fit retry kernel stands by
+    const size_t fsmem = static_cast<size_t>(N + 2 + dfk::kNeDoubles) * dfk::kLmThreads * sizeof(double);
+    const int fgrid = static_cast<int>(std::min<int64_t>((nfit + dfk::kLmThreads - 1) / dfk::kLmThreads,
+                                                         static_cast<int64_t>(ctx->sm_count) * 3));
+    return launch_kernel(ctx, dfk::lm_retry_flat_kernel, fgrid, dfk::kLmThreads, fsmem, st, qi, N, o, map.row_mul, rows, list,
+                         count, counters);
 }
 
 int check_nls_args(int64_t nbuf, int64_t R, int32_t N, double w0) {
@@ -787,17 +673,14 @@ int launch_channel_stats(dfk_ctx* ctx, const double* z, int64_t T, int64_t C, in
         double* sums = static_cast<double*>(ctx->stats_part.ptr);
         double* sq = sums + static_cast<size_t>(nsplit) * C;
         const dim3 grid(static_cast<unsigned>(groups), static_cast<unsigned>(nsplit));
-        dfk::stats_tm_kernel<<<grid, dfk::kStatsThreads, 0, st>>>(z, T, C, ld_t, 0, nullptr, 0, sums);
-        dfk::stats_tm_kernel<<<grid, dfk::kStatsThreads, 0, st>>>(z, T, C, ld_t, 1, sums, nsplit, sq);
-        dfk::stats_tm_finish_kernel<<<static_cast<int>((C + 127) / 128), 128, 0, st>>>(sums, sq, nsplit, T, C, stats, acc);
-        ctx->launches += 3;
-    } else {
-        const int sgrid = static_cast<int>(std::min<int64_t>(C, static_cast<int64_t>(ctx->sm_count) * 8));
-        dfk::channel_stats_kernel<<<sgrid, dfk::kStatsThreads, 0, st>>>(z, T, C, ld_t, ld_c, stats, acc);
-        ctx->launches++;
+        rc = launch_kernel(ctx, dfk::stats_tm_kernel, grid, dfk::kStatsThreads, 0, st, z, T, C, ld_t, 0, nullptr, 0, sums);
+        if (!rc) rc = launch_kernel(ctx, dfk::stats_tm_kernel, grid, dfk::kStatsThreads, 0, st, z, T, C, ld_t, 1, sums, nsplit, sq);
+        if (rc) return rc;
+        return launch_kernel(ctx, dfk::stats_tm_finish_kernel, static_cast<int>((C + 127) / 128), 128, 0, st, sums, sq, nsplit,
+                             T, C, stats, acc);
     }
-    DFK_CUDA(cudaGetLastError());
-    return DFK_OK;
+    const int sgrid = static_cast<int>(std::min<int64_t>(C, static_cast<int64_t>(ctx->sm_count) * 8));
+    return launch_kernel(ctx, dfk::channel_stats_kernel, sgrid, dfk::kStatsThreads, 0, st, z, T, C, ld_t, ld_c, stats, acc);
 }
 
 }  // namespace
@@ -1171,14 +1054,7 @@ int dfk_ekf_stream_dev(dfk_ctx* ctx, const double* z_dev, int64_t T, int64_t C, 
     const int64_t grid = (C + cpw - 1) / cpw;
     if (grid > std::numeric_limits<int>::max()) return fail(DFK_ERR_ARG, "too many channels");
     ProfScope ps(ctx, 3, st);
-    switch (dev_int("DFK_EKF_UNROLL", 1)) {
-        case 2: dfk::ekf_kernel<2><<<static_cast<int>(grid), 32, 0, st>>>(z_dev, T, C, ld_t, ld_c, R, a, stats, rows_dev); break;
-        case 4: dfk::ekf_kernel<4><<<static_cast<int>(grid), 32, 0, st>>>(z_dev, T, C, ld_t, ld_c, R, a, stats, rows_dev); break;
-        default: dfk::ekf_kernel<1><<<static_cast<int>(grid), 32, 0, st>>>(z_dev, T, C, ld_t, ld_c, R, a, stats, rows_dev); break;
-    }
-    ctx->launches++;
-    DFK_CUDA(cudaGetLastError());
-    return DFK_OK;
+    return launch_kernel(ctx, dfk::ekf_kernel, static_cast<int>(grid), 32, 0, st, z_dev, T, C, ld_t, ld_c, R, a, stats, rows_dev);
 }
 
 // EKFFitter.fit on host records [C][T].  A record that fits the device goes up whole.  A longer one (cfg 4 is 655 GB)
@@ -1271,10 +1147,9 @@ int dfk_ekf_host(dfk_ctx* ctx, const double* z_host, int64_t T, int64_t C, int64
                 DFK_CUDA(cudaEventRecord(ctx->consumed[sl], st));
             }
             if (pass == 0) {
-                dfk::stats_finish_kernel<<<static_cast<int>((C + 127) / 128), 128, 0, st>>>(
-                    acc, C, static_cast<double*>(ctx->stats.ptr));
-                ctx->launches++;
-                DFK_CUDA(cudaGetLastError());
+                rc = launch_kernel(ctx, dfk::stats_finish_kernel, static_cast<int>((C + 127) / 128), 128, 0, st, acc, C,
+                                   static_cast<double*>(ctx->stats.ptr));
+                if (rc) return rc;
             }
         }
     }
@@ -1337,10 +1212,7 @@ int dfk_synth_snr_slab_dev(dfk_ctx* ctx, double* x_dev, int64_t T, int64_t C, in
     }
     const dim3 grid(static_cast<unsigned>(gx), static_cast<unsigned>((C + ch_per_block - 1) / ch_per_block));
     const size_t smem = table ? static_cast<size_t>(p.P) * sizeof(double) : 0;
-    dfk::synth_snr_kernel<<<grid, dfk::kSynthThreads, smem, ctx->stream()>>>(p, table, ch_per_block);
-    ctx->launches++;
-    DFK_CUDA(cudaGetLastError());
-    return DFK_OK;
+    return launch_kernel(ctx, dfk::synth_snr_kernel, grid, dfk::kSynthThreads, smem, ctx->stream(), p, table, ch_per_block);
 }
 
 int dfk_sweep_demod_dev(dfk_ctx* ctx, int64_t nbuf, int64_t c0, int64_t R, int32_t N, double f_samp, double f_mod, double m,
@@ -1379,29 +1251,17 @@ int dfk_sweep_demod_dev(dfk_ctx* ctx, int64_t nbuf, int64_t c0, int64_t R, int32
         sp.N = N;
         const int64_t ngroups = (nbuf + dfk::kPeriodNbw - 1) / dfk::kPeriodNbw;
         const int grid = static_cast<int>(std::min<int64_t>(ngroups, ctx->sm_count));
-        int launched = 0;
-        auto launch = [&](auto kernel, int wc, int wg, int ns) -> int {
-            const dfk::SweepSmem S = dfk::sweep_smem_layout(static_cast<int>(P), N, wc, ns);
-            if (S.total > static_cast<size_t>(ctx->max_smem_optin)) return DFK_OK;  // does not fit: try the next shape
-            DFK_CUDA(cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, static_cast<int>(S.total)));
+        // 6 consumer and 10 generator warps around a ring of 10 stages; many harmonics: 5 and 11 around a ring of 6
+        size_t smem = dfk::sweep_smem_layout(static_cast<int>(P), N, 6, 10).total;
+        if (smem <= static_cast<size_t>(ctx->max_smem_optin)) {
             ProfScope ps(ctx, 0, st);
-            kernel<<<grid, (wc + wg) * 32, S.total, st>>>(sp);
-            ctx->launches++;
-            DFK_CUDA(cudaGetLastError());
-            launched = 1;
-            return DFK_OK;
-        };
-        int rc = DFK_OK;
-        switch (dev_int("DFK_SWEEP_SHAPE", 610)) {  // consumer warps x 100 + generator warps
-            case 88: rc = launch(dfk::sweep_period_kernel<8, 8, 8>, 8, 8, 8); break;
-            case 79: rc = launch(dfk::sweep_period_kernel<7, 9, 9>, 7, 9, 9); break;
-            case 511: rc = launch(dfk::sweep_period_kernel<5, 11, 11>, 5, 11, 11); break;
-            default: rc = launch(dfk::sweep_period_kernel<6, 10, 10>, 6, 10, 10); break;
+            return launch_kernel(ctx, dfk::sweep_period_kernel<6, 10, 10>, grid, (6 + 10) * 32, smem, st, sp);
         }
-        if (rc) return rc;
-        if (!launched) rc = launch(dfk::sweep_period_kernel<5, 11, 6>, 5, 11, 6);  // many harmonics: a shallower ring
-        if (rc) return rc;
-        if (launched) return DFK_OK;
+        smem = dfk::sweep_smem_layout(static_cast<int>(P), N, 5, 6).total;
+        if (smem <= static_cast<size_t>(ctx->max_smem_optin)) {
+            ProfScope ps(ctx, 0, st);
+            return launch_kernel(ctx, dfk::sweep_period_kernel<5, 11, 6>, grid, (5 + 11) * 32, smem, st, sp);
+        }
     }
     // any other geometry: records generated into scratch in waves, then the ordinary lock-in
     const double w0 = 2.0 * dfk::kPi * f_mod / f_samp;
@@ -1575,10 +1435,8 @@ int dfk_bessel_dev(dfk_ctx* ctx, const double* x_dev, int64_t n, int32_t nmax, d
     if (n < 0 || nmax < 0 || nmax > DFK_MAX_HARMONICS + 1) return fail(DFK_ERR_ARG, "bad arguments");
     if (n == 0) return DFK_OK;
     if (!x_dev || !out_dev) return fail(DFK_ERR_ARG, "null device pointer");
-    dfk::bessel_kernel<<<static_cast<int>((n + 127) / 128), 128, 0, ctx->stream()>>>(x_dev, n, nmax, out_dev);
-    ctx->launches++;
-    DFK_CUDA(cudaGetLastError());
-    return DFK_OK;
+    return launch_kernel(ctx, dfk::bessel_kernel, static_cast<int>((n + 127) / 128), 128, 0, ctx->stream(), x_dev, n, nmax,
+                         out_dev);
 }
 
 }  // extern "C"

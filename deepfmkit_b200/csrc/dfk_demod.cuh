@@ -981,7 +981,10 @@ __global__ void __launch_bounds__(kFoldThreads, 1) demod_tile_kernel(const TileP
 //   * every lane produces 2 output rows x 4 buffers (instead of 1 x 8), which loads 6 operands per 8 FMAs
 //     instead of 9: shared-memory loads are charged per lane-byte, broadcast or not.
 constexpr int kPeriodNbw = 8;
-constexpr int kPeriodWarps = 8;  // default consumer warps of demod_period_kernel<WARPS> (+ one producer warp)
+// Consumer warps of the one build of demod_period_kernel<WARPS> (+ one producer warp).  It stays a template: as a
+// plain kernel its 128-byte-aligned smem_raw would be the module's first dynamic shared array, which moves the dynamic
+// shared memory of synth_snr_kernel from byte 16 to byte 128.
+constexpr int kPeriodWarps = 8;
 
 struct PeriodParams {
     const double* x;

@@ -166,7 +166,6 @@ DFK_D void cp_async_wait() {
 // warp, 512 warps on 592 sub-partitions).  Samples arrive through each thread's private shared-memory column by
 // cp.async, kEkfStages tiles ahead: no registers, no barrier (a thread only ever reads what it copied itself),
 // and either record layout ([C][T] or [T][C]) costs one 8-byte copy per sample.
-template <int UNROLL>
 __global__ void __launch_bounds__(32) ekf_kernel(const double* __restrict__ z, long long T, long long C,
                                                  long long ld_t, long long ld_c, long long R, EkfLaunch a,
                                                  const double* __restrict__ stats, double* __restrict__ rows) {
@@ -235,7 +234,7 @@ __global__ void __launch_bounds__(32) ekf_kernel(const double* __restrict__ z, l
         while (pos < lim) {
             const int run = (us < lim - pos) ? static_cast<int>(us) : lim - pos;
             double A = carrier_angle(kdl, k);
-#pragma unroll UNROLL
+#pragma unroll 1
             for (int i = 0; i < run; ++i) {
                 kdl += 1.0;
                 const double A_next = carrier_angle(kdl, k);  // off the chain: ready before the next step needs it

@@ -55,8 +55,7 @@ def test_random_geometries(monkeypatch):
         lib.dfk_dev_clear()
         if rng.rand() < 0.3:
             lib.dfk_dev_set(b"DFK_TILE_NSTAGES", int(rng.randint(2, 6)))
-        if kind == 0 and rng.rand() < 0.6:  # consumer warps and ring depth of the single-period kernel
-            lib.dfk_dev_set(b"DFK_PERIOD_WARPS", int(rng.choice([6, 8, 10, 12])))
+        if kind == 0 and rng.rand() < 0.6:  # ring depth of the single-period kernel
             lib.dfk_dev_set(b"DFK_PERIOD_NSTAGES", int(rng.randint(2, 13)))
         t = np.arange(nbuf * R)
         x = 1.0 + np.cos(0.3 + 4.0 * np.cos(2 * np.pi * t / P + 0.1)) + 0.05 * rng.randn(nbuf * R)

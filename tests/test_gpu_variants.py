@@ -64,7 +64,7 @@ def assert_ran(names, kernel):
 # DFK_LM_FLAT = 0; MINB 4 / 5 are the 128- and 96-register builds of one PTX.
 LM_COLD = ([(g, dict(DFK_LM_MINB=mb), f"lm_first_kernel<{g}, {mb}, 128>") for g in (2, 4, 8, 16, 32) for mb in (4, 5)]
            + [(1, dict(DFK_LM_FLAT=0, DFK_LM_MINB=mb), f"lm_first_kernel<1, {mb}, 128>") for mb in (4, 5)]
-           + [(1, dict(DFK_LM_FLAT_MINB=fm), f"lm_flat_kernel<{fm}>") for fm in (4, 5, 6, 8)])
+           + [(1, {}, "lm_flat_kernel<4>")])
 LM_COLD_IDS = [k.replace(", ", "_").replace("<", "-").replace(">", "") for _, _, k in LM_COLD]
 W0_BANK = 2.0 * np.pi * F_MOD / F_SAMP
 FLAT_RETRY_MIN = 4096  # kFlatRetryMin: from this many parked fits the retry stage is a thread per fit
@@ -155,8 +155,7 @@ def test_lm_cold_build_vs_oracle(torch_mod, ctx, lm_bank, retry, i):
     assert (parked >= FLAT_RETRY_MIN) == (retry == "flat")
 
 
-MINB_PAIRS = [(f"lm_first_kernel<{g}, 4, 128>", f"lm_first_kernel<{g}, 5, 128>") for g in (1, 2, 4, 8, 16, 32)] + \
-    [("lm_flat_kernel<4>", f"lm_flat_kernel<{fm}>") for fm in (5, 6, 8)]
+MINB_PAIRS = [(f"lm_first_kernel<{g}, 4, 128>", f"lm_first_kernel<{g}, 5, 128>") for g in (1, 2, 4, 8, 16, 32)]
 
 
 @pytest.mark.parametrize("pair", MINB_PAIRS, ids=[f"{a}-vs-{b}" for a, b in MINB_PAIRS])
@@ -186,16 +185,14 @@ def test_lm_cold_builds_pairwise_equality(torch_mod, ctx, lm_bank):
             print(f"LM pair {retry:4s} {a} vs {b}: {'bit-equal' if same else 'differs'}")
 
 
-LM_WARM = [(g, dict(DFK_LM_MINB=mb), f"lm_first_kernel<{g}, {mb}, 128>") for g in (2, 8, 16) for mb in (4, 5)] + \
-    [(1, dict(DFK_LM_FLAT=2), "lm_flat_kernel<4>")]
+LM_WARM = [(g, dict(DFK_LM_MINB=mb), f"lm_first_kernel<{g}, {mb}, 128>") for g in (2, 8, 16) for mb in (4, 5)]
 GOLDEN_NLS = ["cfg1_quickstart", "cfg2_1mhz", "cfg3_channel", "deep_mod_n62", "fallback_m16", "pathological_m3", "low_snr"]
 
 
 @pytest.mark.parametrize("name", GOLDEN_NLS)
 def test_lm_warm_builds_vs_reference(torch_mod, ctx, golden, name):
     """Warm-started readouts (every buffer from buffer 0's result) of the golden records through the builds that
-    bigger batches select -- G = 2, 8, 16 at both register budgets -- and through the per-lane state machine on
-    warm fits (DFK_LM_FLAT = 2), against the reference's own rows."""
+    bigger batches select -- G = 2, 8, 16 at both register budgets -- against the reference's own rows."""
     from deepfmkit_b200 import _lib
     g, x, f_samp, f_mod, n, nh, R, w0 = _case(golden, name)
     meta = g["meta"]
@@ -215,7 +212,7 @@ def test_lm_warm_builds_vs_reference(torch_mod, ctx, golden, name):
         assert np.array_equal(got[f"lm_first_kernel<{gl}, 4, 128>"], got[f"lm_first_kernel<{gl}, 5, 128>"], equal_nan=True)
 
 
-# ---- 2. EKF channels per warp and unrolling ---------------------------------------------------------------
+# ---- 2. EKF channels per warp -----------------------------------------------------------------------------
 EKF_C, EKF_T, EKF_R = 67, 12_123, 4000
 EKF_CHECK = (0, 1, 7, 8, 31, 32, 33, 63, 64, 66)  # both sides of every warp boundary for cpw 1..32, and the last
 EKF_EXPLICIT = dict(init_a=1.1, init_m=6.0, init_phi=0.15, init_psi=0.02, p0_diag=np.array([0.5, 0.8, 1.2, 0.3, 0.6]),
@@ -260,7 +257,7 @@ def ekf_bank():
             "ref_explicit": dict(zip(EKF_CHECK, refs[len(EKF_CHECK):]))}
 
 
-def _ekf_run(torch, ctx, z, layout, cpw, unroll, kw=None):
+def _ekf_run(torch, ctx, z, layout, cpw, kw=None):
     from deepfmkit_b200 import _lib
     C, T = z.shape
     if layout == "channel_major":
@@ -269,9 +266,7 @@ def _ekf_run(torch, ctx, z, layout, cpw, unroll, kw=None):
         zd, ld_t, ld_c = torch.from_numpy(np.ascontiguousarray(z.T)).cuda(), C, 1
     rows = torch.full((C, T // EKF_R, 8), float("nan"), dtype=torch.float64, device="cuda")
     opts = _ekf_opts(kw)
-    over = dict(DFK_EKF_UNROLL=unroll)
-    if cpw:
-        over["DFK_EKF_CPW"] = cpw
+    over = dict(DFK_EKF_CPW=cpw) if cpw else {}
 
     def call():
         ctx.ekf_dev(zd.data_ptr(), T, C, ld_t, ld_c, EKF_R, F_SAMP, F_MOD, opts, rows.data_ptr())
@@ -279,7 +274,7 @@ def _ekf_run(torch, ctx, z, layout, cpw, unroll, kw=None):
 
     with _lib.dev_overrides(**over):
         _, names = launched_kernels(call)
-    assert_ran(names, f"ekf_kernel<{unroll}>")
+    assert_ran(names, "ekf_kernel")
     return rows.cpu().numpy()
 
 
@@ -289,29 +284,27 @@ def assert_ekf_rows(rows, ref):
 
 
 @pytest.mark.parametrize("layout", ["channel_major", "time_major"])
-def test_ekf_channels_per_warp_and_unroll(torch_mod, ctx, ekf_bank, layout):
-    """DFK_EKF_CPW in {1, ..., 32} x DFK_EKF_UNROLL in {1, 2, 4}: a lane's arithmetic depends on neither, so every
-    combination gives cpw 1 / unroll 1's rows bit for bit, and those match the oracle on both sides of every warp
-    boundary (initial dc and R from each channel's own statistics)."""
+def test_ekf_channels_per_warp(torch_mod, ctx, ekf_bank, layout):
+    """DFK_EKF_CPW in {1, ..., 32}: a lane's arithmetic does not depend on it, so every value gives cpw 1's rows bit
+    for bit, and those match the oracle on both sides of every warp boundary (initial dc and R from each channel's
+    own statistics)."""
     z = ekf_bank["z"]
-    base = _ekf_run(torch_mod, ctx, z, layout, 1, 1)
+    base = _ekf_run(torch_mod, ctx, z, layout, 1)
     for c in EKF_CHECK:
         assert_ekf_rows(base[c], ekf_bank["ref"][c])
-    for cpw in (1, 2, 4, 8, 16, 32):
-        for unroll in (1, 2, 4):
-            if (cpw, unroll) != (1, 1):
-                rows = _ekf_run(torch_mod, ctx, z, layout, cpw, unroll)
-                assert np.array_equal(rows, base), (cpw, unroll)
+    for cpw in (2, 4, 8, 16, 32):
+        rows = _ekf_run(torch_mod, ctx, z, layout, cpw)
+        assert np.array_equal(rows, base), cpw
 
 
 def test_ekf_channels_per_warp_explicit_options(torch_mod, ctx, ekf_bank):
     """Options given in full (initial state, P0, Q, R, dc): the same bit-equality over cpw, the oracle's rows."""
     z = ekf_bank["z_explicit"]
-    base = _ekf_run(torch_mod, ctx, z, "channel_major", 1, 1, EKF_EXPLICIT)
+    base = _ekf_run(torch_mod, ctx, z, "channel_major", 1, EKF_EXPLICIT)
     for c in EKF_CHECK:
         assert_ekf_rows(base[c], ekf_bank["ref_explicit"][c])
     for cpw in (2, 4, 8, 16, 32):
-        assert np.array_equal(_ekf_run(torch_mod, ctx, z, "channel_major", cpw, 4, EKF_EXPLICIT), base), cpw
+        assert np.array_equal(_ekf_run(torch_mod, ctx, z, "channel_major", cpw, EKF_EXPLICIT), base), cpw
 
 
 def test_ekf_heuristic_channels_per_warp(torch_mod, ctx):
@@ -330,8 +323,8 @@ def test_ekf_heuristic_channels_per_warp(torch_mod, ctx):
         cpw *= 2
     if sm == 148:
         assert cpw == 4
-    auto = _ekf_run(torch, ctx, z, "channel_major", 0, 1)
-    one = _ekf_run(torch, ctx, z, "channel_major", 1, 1)
+    auto = _ekf_run(torch, ctx, z, "channel_major", 0)
+    one = _ekf_run(torch, ctx, z, "channel_major", 1)
     assert np.array_equal(auto, one)
     sample = (0, 3, 4, 599, 1196, 1199)
     with Pool(len(sample)) as pool:
@@ -388,7 +381,7 @@ def replay_refs():
     return {k: (inp, ref) for (k, inp), ref in zip(inputs.items(), refs)}
 
 
-def _stream(torch, ctx, z, state, k0, unroll=1):
+def _stream(torch, ctx, z, state, k0):
     from deepfmkit_b200 import _lib
     T = len(z)
     zd = torch.from_numpy(z[None, :].copy()).cuda()
@@ -400,9 +393,8 @@ def _stream(torch, ctx, z, state, k0, unroll=1):
         ctx.ekf_stream_dev(zd.data_ptr(), T, 1, 1, T, REPLAY_R, F_SAMP, F_MOD, opts, k0, sd.data_ptr(), rows.data_ptr())
         ctx.synchronize()
 
-    with _lib.dev_overrides(DFK_EKF_UNROLL=unroll):
-        _, names = launched_kernels(call)
-    assert_ran(names, f"ekf_kernel<{unroll}>")
+    _, names = launched_kernels(call)
+    assert_ran(names, "ekf_kernel")
     return rows.cpu().numpy()[0], sd.cpu().numpy()[0]
 
 
@@ -461,7 +453,7 @@ def test_ekf_checked_replay_vs_oracle(torch_mod, ctx, replay_refs, case):
                           init_phi=state_a[2], init_psi=state_a[3], init_dc=state_a[4], r_val=state_a[30], init_cov=P,
                           k0=k0 + CROSS_SPLIT)
     assert np.max(np.abs(b[:, :5] - ref_b[:, :5])) < EKF_TOL
-    assert np.array_equal(_stream(torch_mod, ctx, z, state, k0, unroll=4)[0], rows)
+    assert np.array_equal(_stream(torch_mod, ctx, z, state, k0)[0], rows)
 
 # ---- 4. forced drift term --------------------------------------------------------------------------------
 EXTREME_SHAPES = [(2048, 3, 10), (1536, 2, 7), (1000, 1, 64), (6, 50, 2), (2, 40, 1), (256, 5, 31), (258, 4, 16),
