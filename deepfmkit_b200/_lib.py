@@ -15,8 +15,9 @@ import numpy as np
 from ._build import LIB_PATH
 
 ROW_STRIDE = 8
+COV_STRIDE = 8          # [C_aa, C_am, C_aphi, C_mm, C_mphi, C_phiphi, C_psipsi, s^2] per result row
 MAX_HARMONICS = 64
-ABI_VERSION = 4
+ABI_VERSION = 5
 PROFILE_KINDS = 4
 ASD_TRIAL_DOUBLES = 37
 TRIAL_STATS_DOUBLES = 6
@@ -77,13 +78,20 @@ SYMBOLS = {
     "dfk_default_ekf_opts": (None, [ctypes.POINTER(EkfOpts)]),
     "dfk_demod": (ctypes.c_int, [_vp, _vp, _i64, _i64, _i32, _d, _vp, _vp]),
     "dfk_lm_fit": (ctypes.c_int, [_vp, _vp, _i64, _i32, _vp, _i64, _vp, ctypes.POINTER(LmOpts), _vp]),
+    "dfk_lm_cov": (ctypes.c_int, [_vp, _vp, _i64, _i32, _vp, _vp]),
     "dfk_nls_fit_dev": (ctypes.c_int, [_vp, _vp, _i64, _i64, _i32, _d, c_double_p, _i32, ctypes.POINTER(LmOpts), _vp]),
+    "dfk_nls_fit_cov_dev": (ctypes.c_int, [_vp, _vp, _i64, _i64, _i32, _d, c_double_p, _i32, ctypes.POINTER(LmOpts), _vp,
+                                           _vp]),
     "dfk_nls_fit_seeded_dev": (ctypes.c_int, [_vp, _vp, _i64, _i64, _i32, _d, c_double_p, _i32, ctypes.POINTER(LmOpts), _vp]),
     "dfk_nls_fit_batch_dev": (ctypes.c_int, [_vp, _vp, _i64, _i64, _i64, _i64, _i32, _d, c_double_p, _vp, _i64, _i32,
                                              ctypes.POINTER(LmOpts), _vp]),
+    "dfk_nls_fit_batch_cov_dev": (ctypes.c_int, [_vp, _vp, _i64, _i64, _i64, _i64, _i32, _d, c_double_p, _vp, _i64, _i32,
+                                                 ctypes.POINTER(LmOpts), _vp, _vp]),
     "dfk_demod_tm_dev": (ctypes.c_int, [_vp, _vp, _i64, _i64, _i64, _i32, _d, _vp, _vp]),
     "dfk_nls_fit_batch_tm_dev": (ctypes.c_int, [_vp, _vp, _i64, _i64, _i64, _i32, _d, c_double_p, _vp, _i64, _i32,
                                                 ctypes.POINTER(LmOpts), _vp]),
+    "dfk_nls_fit_batch_tm_cov_dev": (ctypes.c_int, [_vp, _vp, _i64, _i64, _i64, _i32, _d, c_double_p, _vp, _i64, _i32,
+                                                    ctypes.POINTER(LmOpts), _vp, _vp]),
     "dfk_ekf_dev": (ctypes.c_int, [_vp, _vp, _i64, _i64, _i64, _i64, _i64, _d, _d, ctypes.POINTER(EkfOpts), _vp]),
     "dfk_ekf_stream_dev": (ctypes.c_int, [_vp, _vp, _i64, _i64, _i64, _i64, _i64, _d, _d, ctypes.POINTER(EkfOpts), _i64,
                                           _vp, _vp]),
@@ -93,7 +101,11 @@ SYMBOLS = {
     "dfk_sweep_demod_dev": (ctypes.c_int, [_vp, _i64, _i64, _i64, _i32, _d, _d, _d, _d, _d, _d, _d, _d, ctypes.c_uint64, _vp, _vp]),
     "dfk_nls_sweep_dev": (ctypes.c_int, [_vp, c_double_p, _i32, _i64, _i64, _i64, _i64, _i32, _d, _d, _d, _d, _d, _d, _d,
                                          ctypes.c_uint64, _d, _d, ctypes.POINTER(LmOpts), _vp]),
+    "dfk_nls_sweep_cov_dev": (ctypes.c_int, [_vp, c_double_p, _i32, _i64, _i64, _i64, _i64, _i32, _d, _d, _d, _d, _d, _d,
+                                             _d, ctypes.c_uint64, _d, _d, ctypes.POINTER(LmOpts), _vp, _vp]),
     "dfk_nls_fit_host": (ctypes.c_int, [_vp, _vp, _i64, _i64, _i32, _d, c_double_p, _i32, ctypes.POINTER(LmOpts), _vp]),
+    "dfk_nls_fit_cov_host": (ctypes.c_int, [_vp, _vp, _i64, _i64, _i32, _d, c_double_p, _i32, ctypes.POINTER(LmOpts), _vp,
+                                            _vp]),
     "dfk_nls_fit_seeded_host": (ctypes.c_int, [_vp, _vp, _i64, _i64, _i32, _d, c_double_p, _i32, ctypes.POINTER(LmOpts), _vp]),
     "dfk_ekf_host": (ctypes.c_int, [_vp, _vp, _i64, _i64, _i64, _d, _d, ctypes.POINTER(EkfOpts), _vp]),
     "dfk_set_host_slab_bytes": (ctypes.c_int, [_vp, _i64]),
@@ -279,10 +291,20 @@ class Context:
         _check(self.lib, self.lib.dfk_lm_fit(self._h, qi_ptr, nbuf, N, guess_ptr, guess_stride, dc_ptr,
                                              ctypes.byref(opts) if opts is not None else None, rows_ptr))
 
-    def nls_fit_dev(self, x_ptr, nbuf, R, N, w0, init, seeded, opts, rows_ptr):
+    def lm_cov(self, qi_ptr, nbuf, N, rows_ptr, cov_ptr):
+        """Covariance rows [nbuf, COV_STRIDE] of fitted rows on their harmonic vectors (dfk_lm_cov)."""
+        _check(self.lib, self.lib.dfk_lm_cov(self._h, qi_ptr, int(nbuf), int(N), rows_ptr, cov_ptr))
+
+    # The record calls take an optional cov_ptr (device, [units, COV_STRIDE]): given, they route to the _cov entry,
+    # which also writes every buffer's parameter covariance there.
+    def nls_fit_dev(self, x_ptr, nbuf, R, N, w0, init, seeded, opts, rows_ptr, cov_ptr=None):
         init_arr = (ctypes.c_double * 4)(*[float(v) for v in init])
-        _check(self.lib, self.lib.dfk_nls_fit_dev(self._h, x_ptr, nbuf, R, N, w0, init_arr, schedule_code(seeded),
-                                                  ctypes.byref(opts) if opts is not None else None, rows_ptr))
+        args = (self._h, x_ptr, nbuf, R, N, w0, init_arr, schedule_code(seeded),
+                ctypes.byref(opts) if opts is not None else None, rows_ptr)
+        if cov_ptr is None:
+            _check(self.lib, self.lib.dfk_nls_fit_dev(*args))
+        else:
+            _check(self.lib, self.lib.dfk_nls_fit_cov_dev(*args, cov_ptr))
 
     def nls_fit_seeded_dev(self, x_ptr, nbuf, R, N, w0, seed, opts, rows_ptr, chunks=1):
         seed_arr = (ctypes.c_double * 4)(*[float(v) for v in seed])
@@ -290,22 +312,28 @@ class Context:
                                                          ctypes.byref(opts) if opts is not None else None, rows_ptr))
 
     def nls_fit_batch_dev(self, x_ptr, C, bufs_per_channel, ld_c, R, N, w0, init, init_dev_ptr, init_stride, seeded,
-                          opts, rows_ptr):
+                          opts, rows_ptr, cov_ptr=None):
         init_arr = (ctypes.c_double * 4)(*[float(v) for v in init]) if init is not None else None
-        _check(self.lib, self.lib.dfk_nls_fit_batch_dev(self._h, x_ptr, C, bufs_per_channel, ld_c, R, N, w0, init_arr,
-                                                        init_dev_ptr, init_stride, schedule_code(seeded),
-                                                        ctypes.byref(opts) if opts is not None else None, rows_ptr))
+        args = (self._h, x_ptr, C, bufs_per_channel, ld_c, R, N, w0, init_arr, init_dev_ptr, init_stride,
+                schedule_code(seeded), ctypes.byref(opts) if opts is not None else None, rows_ptr)
+        if cov_ptr is None:
+            _check(self.lib, self.lib.dfk_nls_fit_batch_dev(*args))
+        else:
+            _check(self.lib, self.lib.dfk_nls_fit_batch_cov_dev(*args, cov_ptr))
 
     def demod_tm(self, x_ptr, bufs_per_channel, C, R, N, w0, qi_ptr, dc_ptr):
         _check(self.lib, self.lib.dfk_demod_tm_dev(self._h, x_ptr, int(bufs_per_channel), int(C), int(R), int(N), float(w0),
                                                    qi_ptr, dc_ptr))
 
-    def nls_fit_batch_tm_dev(self, x_ptr, C, bufs_per_channel, R, N, w0, init, init_dev_ptr, init_stride, seeded, opts, rows_ptr):
+    def nls_fit_batch_tm_dev(self, x_ptr, C, bufs_per_channel, R, N, w0, init, init_dev_ptr, init_stride, seeded, opts, rows_ptr,
+                             cov_ptr=None):
         init_arr = (ctypes.c_double * 4)(*[float(v) for v in init]) if init is not None else None
-        _check(self.lib, self.lib.dfk_nls_fit_batch_tm_dev(self._h, x_ptr, int(C), int(bufs_per_channel), int(R), int(N),
-                                                           float(w0), init_arr, init_dev_ptr, int(init_stride),
-                                                           schedule_code(seeded),
-                                                           ctypes.byref(opts) if opts is not None else None, rows_ptr))
+        args = (self._h, x_ptr, int(C), int(bufs_per_channel), int(R), int(N), float(w0), init_arr, init_dev_ptr,
+                int(init_stride), schedule_code(seeded), ctypes.byref(opts) if opts is not None else None, rows_ptr)
+        if cov_ptr is None:
+            _check(self.lib, self.lib.dfk_nls_fit_batch_tm_dev(*args))
+        else:
+            _check(self.lib, self.lib.dfk_nls_fit_batch_tm_cov_dev(*args, cov_ptr))
 
     def ekf_dev(self, z_ptr, T, C, ld_t, ld_c, R, f_samp, f_mod, opts, rows_ptr):
         _check(self.lib, self.lib.dfk_ekf_dev(self._h, z_ptr, T, C, ld_t, ld_c, R, f_samp, f_mod,
@@ -333,28 +361,37 @@ class Context:
                                                       int(seed), qi_ptr, dc_ptr))
 
     def nls_sweep_dev(self, m_values, ntrials, trial0, seed_stride, R, N, f_samp, f_mod, rows_ptr, amp=1.0, visibility=1.0,
-                      phi0=0.0, psi0=0.0, snr_db=40.0, seed=0, init_a=1.6, init_m=None, opts=None):
+                      phi0=0.0, psi0=0.0, snr_db=40.0, seed=0, init_a=1.6, init_m=None, opts=None, cov_ptr=None):
         ms = np.ascontiguousarray(m_values, dtype=np.float64)
-        _check(self.lib, self.lib.dfk_nls_sweep_dev(self._h, ms.ctypes.data_as(c_double_p), len(ms), int(ntrials), int(trial0),
-                                                    int(seed_stride), int(R), int(N), float(f_samp), float(f_mod), amp,
-                                                    visibility, phi0, psi0, snr_db, int(seed), float(init_a),
-                                                    float("nan") if init_m is None else float(init_m),
-                                                    ctypes.byref(opts) if opts is not None else None, rows_ptr))
+        args = (self._h, ms.ctypes.data_as(c_double_p), len(ms), int(ntrials), int(trial0), int(seed_stride), int(R), int(N),
+                float(f_samp), float(f_mod), amp, visibility, phi0, psi0, snr_db, int(seed), float(init_a),
+                float("nan") if init_m is None else float(init_m), ctypes.byref(opts) if opts is not None else None, rows_ptr)
+        if cov_ptr is None:
+            _check(self.lib, self.lib.dfk_nls_sweep_dev(*args))
+        else:
+            _check(self.lib, self.lib.dfk_nls_sweep_cov_dev(*args, cov_ptr))
 
     def bessel_dev(self, x_ptr, n, nmax, out_ptr):
         _check(self.lib, self.lib.dfk_bessel_dev(self._h, x_ptr, n, nmax, out_ptr))
 
     # ---- host-pointer calls ----------------------------------------------------------------------------
-    def nls_fit_host(self, x, R, N, w0, init, seeded=True, opts=None, rows_out=None):
+    def nls_fit_host(self, x, R, N, w0, init, seeded=True, opts=None, rows_out=None, cov_out=None):
         """x: 1-D float64 host array (numpy or a pinned torch tensor's numpy view). Returns rows[nbuf, 8].
-        seeded: see schedule_code (True: every buffer from buffer 0's result; k: the reference's k-chunk chain)."""
+        seeded: see schedule_code (True: every buffer from buffer 0's result; k: the reference's k-chunk chain).
+        cov_out: a C-contiguous float64 array [nbuf, COV_STRIDE] that receives every buffer's parameter covariance."""
         x, xp = _host_array(x)
         nbuf = x.size // int(R)
         rows = rows_out if rows_out is not None else np.empty((nbuf, ROW_STRIDE), dtype=np.float64)
         init_arr = (ctypes.c_double * 4)(*[float(v) for v in init])
-        _check(self.lib, self.lib.dfk_nls_fit_host(self._h, xp, x.size, int(R), int(N), float(w0), init_arr,
-                                                   schedule_code(seeded), ctypes.byref(opts) if opts is not None else None,
-                                                   rows.ctypes.data))
+        args = (self._h, xp, x.size, int(R), int(N), float(w0), init_arr, schedule_code(seeded),
+                ctypes.byref(opts) if opts is not None else None, rows.ctypes.data)
+        if cov_out is None:
+            _check(self.lib, self.lib.dfk_nls_fit_host(*args))
+        else:
+            if not (isinstance(cov_out, np.ndarray) and cov_out.dtype == np.float64 and cov_out.flags.c_contiguous
+                    and cov_out.size >= nbuf * COV_STRIDE):
+                raise ValueError(f"cov_out must be a C-contiguous float64 array of [{nbuf}, {COV_STRIDE}]")
+            _check(self.lib, self.lib.dfk_nls_fit_cov_host(*args, cov_out.ctypes.data))
         return rows
 
     def nls_fit_seeded_host(self, x, R, N, w0, seed, chunks=1, opts=None, rows_out=None):

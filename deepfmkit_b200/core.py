@@ -121,6 +121,8 @@ class DeepFitObject:
         self.t0 = 0
         self.f_samp = self.f_mod = None
         self.ssq = self.amp = self.m = self.tau = self.phi = self.psi = self.dc = self.time = None
+        # one-sigma errors, filled by fit(..., uncertainties=True) (not part of the fit_data text format)
+        self.amp_err = self.m_err = self.phi_err = self.psi_err = self.tau_err = None
         # spectral-estimate settings and results (data.py:148-158)
         self.f = None
         self.Sxx = None
@@ -424,6 +426,9 @@ class DeepFitFramework:
             return None
         sim = getattr(main_raw, "sim", None)
         results_df["tau"] = results_df["m"] / (2 * np.pi * sim.laser.df) if sim else 0.0  # core.py:506-507
+        uncertainties = "m_err" in results_df.columns
+        if uncertainties:  # the error of tau follows from m's exactly as tau does
+            results_df["tau_err"] = results_df["m_err"] / (2 * np.pi * sim.laser.df) if sim else 0.0
         self.fits_df[fit_label] = results_df
 
         fit = DeepFitObject()
@@ -434,6 +439,10 @@ class DeepFitFramework:
         for col in ("ssq", "amp", "m", "tau", "phi", "psi", "dc"):
             setattr(fit, col, np.asarray(results_df[col], dtype=np.float64) if col != "tau" or sim
                     else np.zeros(len(results_df)))
+        if uncertainties:
+            for col in ("amp_err", "m_err", "tau_err", "phi_err", "psi_err"):
+                setattr(fit, col, np.asarray(results_df[col], dtype=np.float64) if col != "tau_err" or sim
+                        else np.zeros(len(results_df)))
         fit.time = np.arange(0, fit.ssq.shape[0] / fit.fs, 1.0 / fit.fs)
         fit.label = fit_label
         self.fits[fit_label] = fit

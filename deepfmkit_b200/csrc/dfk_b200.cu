@@ -538,6 +538,16 @@ int launch_lm(dfk_ctx* ctx, const double* qi, int64_t nfit, dfk::FitMap map, int
                          count, counters);
 }
 
+// Covariance rows (dfk::fit_covariance) of nfit final result rows on their harmonic vectors: a thread per fit.
+int launch_cov(dfk_ctx* ctx, const double* qi, int64_t nfit, int N, const double* rows, double* cov, cudaStream_t st) {
+    if (nfit == 0) return DFK_OK;
+    const size_t smem = static_cast<size_t>(N + 2) * dfk::kLmThreads * sizeof(double);
+    const int grid = static_cast<int>(std::min<int64_t>((nfit + dfk::kLmThreads - 1) / dfk::kLmThreads,
+                                                        static_cast<int64_t>(ctx->sm_count) * 8));
+    return launch_kernel(ctx, dfk::lm_cov_kernel, grid, dfk::kLmThreads, smem, st, qi, static_cast<long long>(nfit), N, rows,
+                         cov);
+}
+
 int check_nls_args(int64_t nbuf, int64_t R, int32_t N, double w0) {
     if (nbuf < 0 || R <= 0) return fail(DFK_ERR_ARG, "bad geometry: nbuf=%lld R=%lld", (long long)nbuf, (long long)R);
     if (N < 1 || N > DFK_MAX_HARMONICS) return fail(DFK_ERR_ARG, "harmonic count %d outside 1..%d", N, DFK_MAX_HARMONICS);
@@ -590,9 +600,11 @@ dfk::ChainPlan chain_plan(const Schedule& sc, int64_t bpc) {
 // demod + fits of C device-resident channel records of bpc buffers each (records ld_c samples apart).
 //   init_dev == nullptr: every cold start uses init[4]; else channel c starts from init_dev[c * init_stride ..+3].
 //   seed_row (single-channel continuation slabs only): the row that already holds buffer 0's result.
+//   cov (may be NULL): receives the covariance row of every buffer, from the whole record's harmonic vectors.
 int nls_on_device(dfk_ctx* ctx, const double* x, int64_t C, int64_t bpc, int64_t ld_c, int64_t R, int32_t N, double w0,
                   const double init[4], const double* init_dev, int64_t init_stride, const Schedule& sc,
-                  const double* seed_row, const dfk_lm_opts* opts, double* rows, cudaStream_t st, bool time_major = false) {
+                  const double* seed_row, const dfk_lm_opts* opts, double* rows, double* cov, cudaStream_t st,
+                  bool time_major = false) {
     const int64_t nbuf = C * bpc;
     if (nbuf == 0) return DFK_OK;
     int rc = ensure(ctx, ctx->qi, static_cast<size_t>(nbuf) * 2 * N * sizeof(double));
@@ -645,14 +657,22 @@ int nls_on_device(dfk_ctx* ctx, const double* x, int64_t C, int64_t bpc, int64_t
     if (rc) return rc;
     if (two_stage) DFK_CUDA(cudaStreamWaitEvent(st, ctx->join, 0));  // before the LM timing scope opens
     ProfScope ps(ctx, 1, st);
-    if (sc.external_seed)  // a slab of a record whose buffer 0 lives elsewhere: init is that buffer's result
-        return launch_lm(ctx, qi, nbuf, {1, 0, 1}, N, cold, dc, opts, rows, st, false, chain);
-    if (!seeded || (bpc == 1 && !seed_row)) return launch_lm(ctx, qi, nbuf, {1, 0, 1}, N, cold, dc, opts, rows, st, true);
-    if (seed_row)  // continuation slab of a single record: chunk seeds come from the stored row of buffer 0
-        return launch_lm(ctx, qi, nbuf, {1, 0, 1}, N, guess_rows(seed_row, 0, nbuf, false), dc, opts, rows, st, false, chain);
-    // fitters.py:407-417: every chunk starts from its channel's buffer-0 result
-    return launch_lm(ctx, qi, nbuf, {1, 0, 1}, N, guess_rows(rows, bpc * DFK_ROW_STRIDE, bpc, true), dc, opts, rows, st,
-                     false, chain);
+    auto fit = [&]() {
+        if (sc.external_seed)  // a slab of a record whose buffer 0 lives elsewhere: init is that buffer's result
+            return launch_lm(ctx, qi, nbuf, {1, 0, 1}, N, cold, dc, opts, rows, st, false, chain);
+        if (!seeded || (bpc == 1 && !seed_row)) return launch_lm(ctx, qi, nbuf, {1, 0, 1}, N, cold, dc, opts, rows, st, true);
+        if (seed_row)  // continuation slab of a single record: chunk seeds come from the stored row of buffer 0
+            return launch_lm(ctx, qi, nbuf, {1, 0, 1}, N, guess_rows(seed_row, 0, nbuf, false), dc, opts, rows, st, false,
+                             chain);
+        // fitters.py:407-417: every chunk starts from its channel's buffer-0 result
+        return launch_lm(ctx, qi, nbuf, {1, 0, 1}, N, guess_rows(rows, bpc * DFK_ROW_STRIDE, bpc, true), dc, opts, rows, st,
+                         false, chain);
+    };
+    rc = fit();
+    // after the last LM launch, so it sees the final rows; buffer 0 of a two-stage record was fitted on qi_seed, but its
+    // covariance, like every other buffer's, comes from the whole record's harmonic vectors
+    if (rc || !cov) return rc;
+    return launch_cov(ctx, qi, nbuf, N, rows, cov, st);
 }
 
 Schedule schedule_of(int32_t seeded) {
@@ -783,7 +803,7 @@ int dfk_destroy(dfk_ctx* ctx) {
     if (ctx->copy_stream) cudaStreamSynchronize(ctx->copy_stream);
     if (ctx->aux_stream) cudaStreamSynchronize(ctx->aux_stream);
     DevBuf* bufs[] = {&ctx->qi, &ctx->dc, &ctx->retry, &ctx->counters, &ctx->slab[0], &ctx->slab[1],
-                      &ctx->rows, &ctx->stats, &ctx->stats_part, &ctx->misc, &ctx->qi_seed, &ctx->dc_seed};
+                      &ctx->rows, &ctx->stats, &ctx->stats_part, &ctx->misc, &ctx->qi_seed, &ctx->dc_seed, &ctx->cov};
     for (DevBuf* b : bufs)
         if (b->ptr) cudaFree(b->ptr);
     for (DevBuf& b : ctx->post)
@@ -849,15 +869,41 @@ int dfk_lm_fit(dfk_ctx* ctx, const double* qi_dev, int64_t nbuf, int32_t N, cons
     return launch_lm(ctx, qi_dev, nbuf, {1, 0, 1}, N, gs, dc_dev, opts, rows_dev, ctx->stream(), guess_stride != 0);
 }
 
-int dfk_nls_fit_dev(dfk_ctx* ctx, const double* x_dev, int64_t nbuf, int64_t R, int32_t N, double w0,
-                    const double init[4], int32_t seeded, const dfk_lm_opts* opts, double* rows_dev) {
+// The record entries below and their _cov variants share one body; cov == NULL launches exactly what the plain
+// entry always launched.
+static int nls_fit_dev_impl(dfk_ctx* ctx, const double* x_dev, int64_t nbuf, int64_t R, int32_t N, double w0,
+                            const double init[4], int32_t seeded, const dfk_lm_opts* opts, double* rows_dev, double* cov_dev) {
     DFK_ENTER(ctx);
     const int rc = check_nls_args(nbuf, R, N, w0);
     if (rc) return rc;
     if (!init) return fail(DFK_ERR_ARG, "null init");
     if (nbuf > 0 && (!x_dev || !rows_dev)) return fail(DFK_ERR_ARG, "null device pointer");
     return nls_on_device(ctx, x_dev, 1, nbuf, nbuf * R, R, N, w0, init, nullptr, 0, schedule_of(seeded), nullptr, opts,
-                         rows_dev, ctx->stream());
+                         rows_dev, cov_dev, ctx->stream());
+}
+
+// The _cov entries need somewhere to put the covariance rows.
+static int check_cov(const double* cov, int64_t n) {
+    return (n > 0 && !cov) ? fail(DFK_ERR_ARG, "null covariance pointer") : DFK_OK;
+}
+
+int dfk_lm_cov(dfk_ctx* ctx, const double* qi_dev, int64_t nbuf, int32_t N, const double* rows_dev, double* cov_dev) {
+    DFK_ENTER(ctx);
+    if (nbuf < 0) return fail(DFK_ERR_ARG, "negative fit count");
+    if (N < 1 || N > DFK_MAX_HARMONICS) return fail(DFK_ERR_ARG, "harmonic count %d outside 1..%d", N, DFK_MAX_HARMONICS);
+    if (nbuf > 0 && (!qi_dev || !rows_dev || !cov_dev)) return fail(DFK_ERR_ARG, "null device pointer");
+    return launch_cov(ctx, qi_dev, nbuf, N, rows_dev, cov_dev, ctx->stream());
+}
+
+int dfk_nls_fit_dev(dfk_ctx* ctx, const double* x_dev, int64_t nbuf, int64_t R, int32_t N, double w0,
+                    const double init[4], int32_t seeded, const dfk_lm_opts* opts, double* rows_dev) {
+    return nls_fit_dev_impl(ctx, x_dev, nbuf, R, N, w0, init, seeded, opts, rows_dev, nullptr);
+}
+
+int dfk_nls_fit_cov_dev(dfk_ctx* ctx, const double* x_dev, int64_t nbuf, int64_t R, int32_t N, double w0,
+                        const double init[4], int32_t seeded, const dfk_lm_opts* opts, double* rows_dev, double* cov_dev) {
+    return check_cov(cov_dev, nbuf) ? DFK_ERR_ARG
+                                    : nls_fit_dev_impl(ctx, x_dev, nbuf, R, N, w0, init, seeded, opts, rows_dev, cov_dev);
 }
 
 int dfk_nls_fit_seeded_dev(dfk_ctx* ctx, const double* x_dev, int64_t nbuf, int64_t R, int32_t N, double w0,
@@ -871,13 +917,13 @@ int dfk_nls_fit_seeded_dev(dfk_ctx* ctx, const double* x_dev, int64_t nbuf, int6
     Schedule sc;
     sc.chunks = chunks;
     sc.external_seed = true;
-    return nls_on_device(ctx, x_dev, 1, nbuf, nbuf * R, R, N, w0, seed, nullptr, 0, sc, nullptr, opts, rows_dev,
+    return nls_on_device(ctx, x_dev, 1, nbuf, nbuf * R, R, N, w0, seed, nullptr, 0, sc, nullptr, opts, rows_dev, nullptr,
                          ctx->stream());
 }
 
-int dfk_nls_fit_batch_dev(dfk_ctx* ctx, const double* x_dev, int64_t C, int64_t bufs_per_channel, int64_t ld_c,
-                          int64_t R, int32_t N, double w0, const double init[4], const double* init_dev,
-                          int64_t init_stride, int32_t seeded, const dfk_lm_opts* opts, double* rows_dev) {
+static int nls_fit_batch_impl(dfk_ctx* ctx, const double* x_dev, int64_t C, int64_t bufs_per_channel, int64_t ld_c,
+                              int64_t R, int32_t N, double w0, const double init[4], const double* init_dev,
+                              int64_t init_stride, int32_t seeded, const dfk_lm_opts* opts, double* rows_dev, double* cov_dev) {
     DFK_ENTER(ctx);
     if (C < 0 || bufs_per_channel < 0) return fail(DFK_ERR_ARG, "negative channel or buffer count");
     const int rc = check_nls_args(C * bufs_per_channel, R, N, w0);
@@ -888,7 +934,22 @@ int dfk_nls_fit_batch_dev(dfk_ctx* ctx, const double* x_dev, int64_t C, int64_t 
     if (C * bufs_per_channel > 0 && (!x_dev || !rows_dev)) return fail(DFK_ERR_ARG, "null device pointer");
     const double zero[4] = {0, 0, 0, 0};
     return nls_on_device(ctx, x_dev, C, bufs_per_channel, ld_c, R, N, w0, init ? init : zero, init_dev, init_stride,
-                         schedule_of(seeded), nullptr, opts, rows_dev, ctx->stream());
+                         schedule_of(seeded), nullptr, opts, rows_dev, cov_dev, ctx->stream());
+}
+
+int dfk_nls_fit_batch_dev(dfk_ctx* ctx, const double* x_dev, int64_t C, int64_t bufs_per_channel, int64_t ld_c,
+                          int64_t R, int32_t N, double w0, const double init[4], const double* init_dev,
+                          int64_t init_stride, int32_t seeded, const dfk_lm_opts* opts, double* rows_dev) {
+    return nls_fit_batch_impl(ctx, x_dev, C, bufs_per_channel, ld_c, R, N, w0, init, init_dev, init_stride, seeded, opts,
+                              rows_dev, nullptr);
+}
+
+int dfk_nls_fit_batch_cov_dev(dfk_ctx* ctx, const double* x_dev, int64_t C, int64_t bufs_per_channel, int64_t ld_c,
+                              int64_t R, int32_t N, double w0, const double init[4], const double* init_dev,
+                              int64_t init_stride, int32_t seeded, const dfk_lm_opts* opts, double* rows_dev, double* cov_dev) {
+    return check_cov(cov_dev, C * bufs_per_channel) ? DFK_ERR_ARG
+                                                    : nls_fit_batch_impl(ctx, x_dev, C, bufs_per_channel, ld_c, R, N, w0, init,
+                                                                         init_dev, init_stride, seeded, opts, rows_dev, cov_dev);
 }
 
 int dfk_demod_tm_dev(dfk_ctx* ctx, const double* x_dev, int64_t bufs_per_channel, int64_t C, int64_t R, int32_t N, double w0,
@@ -902,9 +963,9 @@ int dfk_demod_tm_dev(dfk_ctx* ctx, const double* x_dev, int64_t bufs_per_channel
     return launch_demod_tm(ctx, x_dev, bufs_per_channel, C, R, N, w0, qi_dev, dc_dev, ctx->stream());
 }
 
-int dfk_nls_fit_batch_tm_dev(dfk_ctx* ctx, const double* x_dev, int64_t C, int64_t bufs_per_channel, int64_t R, int32_t N,
-                             double w0, const double init[4], const double* init_dev, int64_t init_stride, int32_t seeded,
-                             const dfk_lm_opts* opts, double* rows_dev) {
+static int nls_fit_batch_tm_impl(dfk_ctx* ctx, const double* x_dev, int64_t C, int64_t bufs_per_channel, int64_t R,
+                                 int32_t N, double w0, const double init[4], const double* init_dev, int64_t init_stride,
+                                 int32_t seeded, const dfk_lm_opts* opts, double* rows_dev, double* cov_dev) {
     DFK_ENTER(ctx);
     if (C < 0 || bufs_per_channel < 0) return fail(DFK_ERR_ARG, "negative channel or buffer count");
     const int rc = check_nls_args(C * bufs_per_channel, R, N, w0);
@@ -914,16 +975,38 @@ int dfk_nls_fit_batch_tm_dev(dfk_ctx* ctx, const double* x_dev, int64_t C, int64
     if (C * bufs_per_channel > 0 && (!x_dev || !rows_dev)) return fail(DFK_ERR_ARG, "null device pointer");
     const double zero[4] = {0, 0, 0, 0};
     return nls_on_device(ctx, x_dev, C, bufs_per_channel, 0, R, N, w0, init ? init : zero, init_dev, init_stride,
-                         schedule_of(seeded), nullptr, opts, rows_dev, ctx->stream(), true);
+                         schedule_of(seeded), nullptr, opts, rows_dev, cov_dev, ctx->stream(), true);
+}
+
+int dfk_nls_fit_batch_tm_dev(dfk_ctx* ctx, const double* x_dev, int64_t C, int64_t bufs_per_channel, int64_t R, int32_t N,
+                             double w0, const double init[4], const double* init_dev, int64_t init_stride, int32_t seeded,
+                             const dfk_lm_opts* opts, double* rows_dev) {
+    return nls_fit_batch_tm_impl(ctx, x_dev, C, bufs_per_channel, R, N, w0, init, init_dev, init_stride, seeded, opts, rows_dev,
+                                 nullptr);
+}
+
+int dfk_nls_fit_batch_tm_cov_dev(dfk_ctx* ctx, const double* x_dev, int64_t C, int64_t bufs_per_channel, int64_t R, int32_t N,
+                                 double w0, const double init[4], const double* init_dev, int64_t init_stride, int32_t seeded,
+                                 const dfk_lm_opts* opts, double* rows_dev, double* cov_dev) {
+    return check_cov(cov_dev, C * bufs_per_channel) ? DFK_ERR_ARG
+                                                    : nls_fit_batch_tm_impl(ctx, x_dev, C, bufs_per_channel, R, N, w0, init,
+                                                                            init_dev, init_stride, seeded, opts, rows_dev, cov_dev);
 }
 
 
 static int nls_host_impl(dfk_ctx* ctx, const double* x_host, int64_t nsamp, int64_t R, int32_t N, double w0,
-                         const double init[4], Schedule sc, const dfk_lm_opts* opts, double* rows_host);
+                         const double init[4], Schedule sc, const dfk_lm_opts* opts, double* rows_host, double* cov_host);
 
 int dfk_nls_fit_host(dfk_ctx* ctx, const double* x_host, int64_t nsamp, int64_t R, int32_t N, double w0,
                      const double init[4], int32_t seeded, const dfk_lm_opts* opts, double* rows_host) {
-    return nls_host_impl(ctx, x_host, nsamp, R, N, w0, init, schedule_of(seeded), opts, rows_host);
+    return nls_host_impl(ctx, x_host, nsamp, R, N, w0, init, schedule_of(seeded), opts, rows_host, nullptr);
+}
+
+int dfk_nls_fit_cov_host(dfk_ctx* ctx, const double* x_host, int64_t nsamp, int64_t R, int32_t N, double w0,
+                         const double init[4], int32_t seeded, const dfk_lm_opts* opts, double* rows_host, double* cov_host) {
+    return check_cov(cov_host, R > 0 ? nsamp / R : 0)
+               ? DFK_ERR_ARG
+               : nls_host_impl(ctx, x_host, nsamp, R, N, w0, init, schedule_of(seeded), opts, rows_host, cov_host);
 }
 
 int dfk_nls_fit_seeded_host(dfk_ctx* ctx, const double* x_host, int64_t nsamp, int64_t R, int32_t N, double w0,
@@ -932,11 +1015,11 @@ int dfk_nls_fit_seeded_host(dfk_ctx* ctx, const double* x_host, int64_t nsamp, i
     Schedule sc;
     sc.chunks = chunks;
     sc.external_seed = true;
-    return nls_host_impl(ctx, x_host, nsamp, R, N, w0, seed, sc, opts, rows_host);
+    return nls_host_impl(ctx, x_host, nsamp, R, N, w0, seed, sc, opts, rows_host, nullptr);
 }
 
 static int nls_host_impl(dfk_ctx* ctx, const double* x_host, int64_t nsamp, int64_t R, int32_t N, double w0,
-                         const double init[4], Schedule sc, const dfk_lm_opts* opts, double* rows_host) {
+                         const double init[4], Schedule sc, const dfk_lm_opts* opts, double* rows_host, double* cov_host) {
     DFK_ENTER(ctx);
     if (nsamp < 0) return fail(DFK_ERR_ARG, "negative sample count");
     const int64_t nbuf = R > 0 ? nsamp / R : 0;
@@ -957,6 +1040,10 @@ static int nls_host_impl(dfk_ctx* ctx, const double* x_host, int64_t nsamp, int6
     }
     rc = ensure(ctx, ctx->rows, static_cast<size_t>(nbuf) * DFK_ROW_STRIDE * sizeof(double));
     if (rc) return rc;
+    if (cov_host) {
+        rc = ensure(ctx, ctx->cov, static_cast<size_t>(nbuf) * DFK_COV_STRIDE * sizeof(double));
+        if (rc) return rc;
+    }
     // scratch for one slab, sized up front so that no reallocation happens mid-pipeline
     rc = ensure(ctx, ctx->qi, static_cast<size_t>(slab_buffers) * 2 * N * sizeof(double));
     if (rc) return rc;
@@ -965,6 +1052,7 @@ static int nls_host_impl(dfk_ctx* ctx, const double* x_host, int64_t nsamp, int6
     rc = ensure(ctx, ctx->retry, (static_cast<size_t>(slab_buffers) + 4) * sizeof(int));
     if (rc) return rc;
     double* rows = static_cast<double*>(ctx->rows.ptr);
+    double* cov = cov_host ? static_cast<double*>(ctx->cov.ptr) : nullptr;
     cudaStream_t st = ctx->stream();
     const bool pageable = is_pageable(x_host);
     HostCallGuard quiesce(ctx);
@@ -981,14 +1069,19 @@ static int nls_host_impl(dfk_ctx* ctx, const double* x_host, int64_t nsamp, int6
         DFK_CUDA(cudaEventRecord(ctx->copied[sl], ctx->copy_stream));
         DFK_CUDA(cudaStreamWaitEvent(st, ctx->copied[sl], 0));
         sc.b0 = done;
+        // the covariance of a slab comes from that slab's harmonic vectors, before the next slab overwrites them
         rc = nls_on_device(ctx, dst, 1, nb, nb * R, R, N, w0, init, nullptr, 0, sc,
-                           (seeded && done > 0) ? rows : nullptr, opts, rows + done * DFK_ROW_STRIDE, st);
+                           (seeded && done > 0) ? rows : nullptr, opts, rows + done * DFK_ROW_STRIDE,
+                           cov ? cov + done * DFK_COV_STRIDE : nullptr, st);
         if (rc) return rc;
         DFK_CUDA(cudaEventRecord(ctx->consumed[sl], st));
         done += nb;
     }
     DFK_CUDA(cudaMemcpyAsync(rows_host, rows, static_cast<size_t>(nbuf) * DFK_ROW_STRIDE * sizeof(double),
                              cudaMemcpyDeviceToHost, st));
+    if (cov)
+        DFK_CUDA(cudaMemcpyAsync(cov_host, cov, static_cast<size_t>(nbuf) * DFK_COV_STRIDE * sizeof(double),
+                                 cudaMemcpyDeviceToHost, st));
     DFK_CUDA(cudaStreamSynchronize(st));
     quiesce.done();
     return DFK_OK;
@@ -1281,10 +1374,10 @@ int dfk_sweep_demod_dev(dfk_ctx* ctx, int64_t nbuf, int64_t c0, int64_t R, int32
     return DFK_OK;
 }
 
-int dfk_nls_sweep_dev(dfk_ctx* ctx, const double* m_values, int32_t nm, int64_t ntrials, int64_t trial0, int64_t seed_stride,
-                      int64_t R, int32_t N, double f_samp, double f_mod, double amp, double visibility, double phi0,
-                      double psi0, double snr_db, uint64_t seed, double init_a, double init_m, const dfk_lm_opts* opts,
-                      double* rows_dev) {
+static int nls_sweep_impl(dfk_ctx* ctx, const double* m_values, int32_t nm, int64_t ntrials, int64_t trial0,
+                          int64_t seed_stride, int64_t R, int32_t N, double f_samp, double f_mod, double amp, double visibility,
+                          double phi0, double psi0, double snr_db, uint64_t seed, double init_a, double init_m,
+                          const dfk_lm_opts* opts, double* rows_dev, double* cov_dev) {
     DFK_ENTER(ctx);
     if (nm < 0 || ntrials < 0 || trial0 < 0) return fail(DFK_ERR_ARG, "bad sweep size");
     if (nm == 0 || ntrials == 0) return DFK_OK;
@@ -1312,8 +1405,28 @@ int dfk_nls_sweep_dev(dfk_ctx* ctx, const double* m_values, int32_t nm, int64_t 
         if (rc) return rc;
     }
     ProfScope ps(ctx, 1, st);
-    return launch_lm(ctx, qi, nfit, {1, 0, 1}, N, guess_rows(static_cast<const double*>(ctx->qi_seed.ptr), 4, ntrials, false), dc,
-                     opts, rows_dev, st, true);
+    rc = launch_lm(ctx, qi, nfit, {1, 0, 1}, N, guess_rows(static_cast<const double*>(ctx->qi_seed.ptr), 4, ntrials, false), dc,
+                   opts, rows_dev, st, true);
+    if (rc || !cov_dev) return rc;
+    return launch_cov(ctx, qi, nfit, N, rows_dev, cov_dev, st);
+}
+
+int dfk_nls_sweep_dev(dfk_ctx* ctx, const double* m_values, int32_t nm, int64_t ntrials, int64_t trial0, int64_t seed_stride,
+                      int64_t R, int32_t N, double f_samp, double f_mod, double amp, double visibility, double phi0,
+                      double psi0, double snr_db, uint64_t seed, double init_a, double init_m, const dfk_lm_opts* opts,
+                      double* rows_dev) {
+    return nls_sweep_impl(ctx, m_values, nm, ntrials, trial0, seed_stride, R, N, f_samp, f_mod, amp, visibility, phi0, psi0,
+                          snr_db, seed, init_a, init_m, opts, rows_dev, nullptr);
+}
+
+int dfk_nls_sweep_cov_dev(dfk_ctx* ctx, const double* m_values, int32_t nm, int64_t ntrials, int64_t trial0,
+                          int64_t seed_stride, int64_t R, int32_t N, double f_samp, double f_mod, double amp, double visibility,
+                          double phi0, double psi0, double snr_db, uint64_t seed, double init_a, double init_m,
+                          const dfk_lm_opts* opts, double* rows_dev, double* cov_dev) {
+    return check_cov(cov_dev, static_cast<int64_t>(nm) * ntrials)
+               ? DFK_ERR_ARG
+               : nls_sweep_impl(ctx, m_values, nm, ntrials, trial0, seed_stride, R, N, f_samp, f_mod, amp, visibility, phi0,
+                                psi0, snr_db, seed, init_a, init_m, opts, rows_dev, cov_dev);
 }
 
 int dfk_lm_counters_read(dfk_ctx* ctx, dfk_lm_counters* out, int32_t reset) {

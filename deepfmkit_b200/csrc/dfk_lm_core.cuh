@@ -440,6 +440,90 @@ DFK_HD void normalise_params(double* p) {
     p[2] = r - kPi;
 }
 
+// Covariance of a fit's reported parameters: the standard NLS estimate s^2 (J^T J)^-1 with s^2 = ssq / (2N - 4), J^T J
+// evaluated at the row's own (normalised, wrapped) parameters -- the model is invariant under that normalisation.
+// The reference computes the same inv(J^T J) sigma^2 only at the true parameters, for its Cramer-Rao bound
+// (helpers.py:16-45, 60-96).  J^T J is block diagonal (see NormalEq), so the result is one 3x3 inverse -- elimination
+// with partial pivoting on unit right-hand sides, as damped_solve at lambda = 0 -- and a division for psi; the psi
+// cross terms are identically zero and not stored.
+//   row: [a, m, phi, psi, dc, ssq, ...];  bes[k*bs]: scratch column of N + 2 doubles (J_0..J_{N+1}(m) on return)
+//   cov: [C_aa, C_am, C_aphi, C_mm, C_mphi, C_phiphi, C_psipsi, s^2]  (kCovStride doubles)
+// Degenerate cases:
+//   2N - 4 <= 0, or a non-finite a, m, phi or psi: all eight entries NaN;
+//   a zero pivot in the 3x3 block (e.g. a = 0: the amplitude column vanishes, fit.py:126): the six block entries NaN;
+//   a33 = 0: C_psipsi NaN;
+//   ssq = 0 (noise-free input): the finite entries are zeros.
+// Computed whatever the row's fitok; callers filter on fitok as they do for the parameters.
+constexpr int kCovStride = 8;
+
+DFK_HD void fit_covariance(int N, const double* qi, int qs, double* bes, int bs, const double* row, double* cov) {
+    const double nan = std::nan("");
+    const int dof = 2 * N - 4;
+    const double p[4] = {row[0], row[1], row[2], row[3]};
+    if (dof <= 0 || !std::isfinite(p[0]) || !std::isfinite(p[1]) || !std::isfinite(p[2]) || !std::isfinite(p[3])) {
+        for (int k = 0; k < kCovStride; ++k) cov[k] = nan;
+        return;
+    }
+    const double s2 = row[5] / static_cast<double>(dof);
+    bessel_j_upto(p[1], N + 1, bes, bs);
+    NormalEq ne;
+    eval_state<1>(N, qi, qs, bes, bs, p, ne);
+    // [A | I] -> [U | L^-1 P]
+    double A[3][6] = {{ne.a00, ne.a01, ne.a02, 1.0, 0.0, 0.0},
+                      {ne.a01, ne.a11, ne.a12, 0.0, 1.0, 0.0},
+                      {ne.a02, ne.a12, ne.a22, 0.0, 0.0, 1.0}};
+    bool ok = true;
+#pragma unroll
+    for (int c = 0; c < 3; ++c) {
+        int piv = c;
+        double best = fabs(A[c][c]);
+#pragma unroll
+        for (int r = c + 1; r < 3; ++r) {
+            const double v = fabs(A[r][c]);
+            if (v > best) {
+                best = v;
+                piv = r;
+            }
+        }
+        if (!(best > 0.0)) ok = false;
+#pragma unroll
+        for (int r = c + 1; r < 3; ++r) {
+            if (piv == r) {
+#pragma unroll
+                for (int k = 0; k < 6; ++k) {
+                    const double tmp = A[c][k];
+                    A[c][k] = A[r][k];
+                    A[r][k] = tmp;
+                }
+            }
+        }
+        const double inv = 1.0 / A[c][c];
+#pragma unroll
+        for (int r = c + 1; r < 3; ++r) {
+            const double f = A[r][c] * inv;
+#pragma unroll
+            for (int k = c + 1; k < 6; ++k) A[r][k] -= f * A[c][k];
+        }
+    }
+    // back substitution, one column of the inverse per right-hand side
+    double X[3][3];
+#pragma unroll
+    for (int k = 0; k < 3; ++k) {
+        X[2][k] = A[2][3 + k] / A[2][2];
+        X[1][k] = (A[1][3 + k] - A[1][2] * X[2][k]) / A[1][1];
+        X[0][k] = (A[0][3 + k] - A[0][1] * X[1][k] - A[0][2] * X[2][k]) / A[0][0];
+    }
+    auto scaled = [s2](double x) { return s2 == 0.0 ? 0.0 : s2 * x; };  // no -0 for a noise-free record
+    cov[0] = ok ? scaled(X[0][0]) : nan;
+    cov[1] = ok ? scaled(X[0][1]) : nan;
+    cov[2] = ok ? scaled(X[0][2]) : nan;
+    cov[3] = ok ? scaled(X[1][1]) : nan;
+    cov[4] = ok ? scaled(X[1][2]) : nan;
+    cov[5] = ok ? scaled(X[2][2]) : nan;
+    cov[6] = ne.a33 != 0.0 ? s2 / ne.a33 : nan;
+    cov[7] = s2;
+}
+
 // Retry stage of fit.py:336-349 for a fit whose first descent ended at (p, ssq) >= threshold.
 template <int G>
 DFK_HD int retry_fit(int N, const double* qi, int qs, double* bes, int bs, const LmOpts& o, double* p, double& ssq,

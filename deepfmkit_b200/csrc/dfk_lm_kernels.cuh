@@ -9,6 +9,7 @@
 //   descent (fit.py:336-349) for the parked fits -- a warp per fit for a handful of stragglers, a thread per fit when
 //   thousands are parked.  Splitting the stages keeps the 20-40x more expensive fallback from stalling warps whose
 //   other fits converged at once.
+// Optional (lm_cov_kernel): the covariance of every final row, for callers that ask for uncertainties.
 //
 // Bessel columns live in shared memory, one column per thread (index k * blockDim.x + threadIdx.x), so
 // the Miller recurrence -- evaluated redundantly by the lanes of a group -- never conflicts on banks.
@@ -412,6 +413,17 @@ __global__ void __launch_bounds__(kLmThreads) lm_retry_kernel(const double* __re
         __syncwarp();
     }
     flush_counts(cnt, counts, lane == 0);
+}
+
+// Covariance of every fit's reported parameters (fit_covariance): one thread per fit, its Bessel column in shared
+// memory ((N + 2) x kLmThreads doubles, as lm_retry_flat_kernel).  Reads the final rows; touches no LM counter.
+__global__ void __launch_bounds__(kLmThreads) lm_cov_kernel(const double* __restrict__ qi, long long nfit, int N,
+                                                            const double* __restrict__ rows, double* __restrict__ cov) {
+    extern __shared__ double bes_smem[];
+    double* bes = bes_smem + threadIdx.x;
+    for (long long f = static_cast<long long>(blockIdx.x) * kLmThreads + threadIdx.x; f < nfit;
+         f += static_cast<long long>(gridDim.x) * kLmThreads)
+        fit_covariance(N, qi + f * 2 * N, 1, bes, kLmThreads, rows + f * kRowStride, cov + f * kCovStride);
 }
 
 // J_0..J_nmax of n arguments, one thread each (testing hook behind dfk_bessel_dev).

@@ -32,6 +32,8 @@ from . import _lib
 from . import fit as fit_tunables
 
 RESULT_COLUMNS = ["amp", "m", "phi", "psi", "dc", "ssq", "fitok"]
+# uncertainties=True: one-sigma errors from the covariance row (_lib.COV_STRIDE): column -> its variance's index
+ERROR_COLUMNS = {"amp_err": 0, "m_err": 3, "phi_err": 5, "psi_err": 6}
 
 
 def _calculate_fit_params(main_raw, n):
@@ -75,10 +77,14 @@ def _record_values(main_raw, column=None) -> np.ndarray:
     return np.ascontiguousarray(vals, dtype=np.float64).reshape(-1)
 
 
-def rows_to_frame(rows: np.ndarray) -> pd.DataFrame:
-    """[nbuf, >=7] row table -> the reference's result frame (fitok int64, the rest float64)."""
+def rows_to_frame(rows: np.ndarray, cov: np.ndarray | None = None) -> pd.DataFrame:
+    """[nbuf, >=7] row table -> the reference's result frame (fitok int64, the rest float64).  With the covariance
+    rows [nbuf, COV_STRIDE] the frame gains the float64 columns amp_err, m_err, phi_err, psi_err after fitok."""
     df = pd.DataFrame({c: np.asarray(rows[:, i], dtype=np.float64) for i, c in enumerate(RESULT_COLUMNS[:6])})
     df["fitok"] = np.asarray(rows[:, 6]).astype(np.int64)
+    if cov is not None:
+        for c, i in ERROR_COLUMNS.items():
+            df[c] = np.sqrt(np.asarray(cov[:, i], dtype=np.float64))
     return df
 
 
@@ -96,10 +102,15 @@ class BaseFitter(ABC):
 
 
 class StandardNLSFitter(BaseFitter):
-    """Frequency-domain NLS readout: lock-in demodulation + 4-parameter LM fit per buffer (fitters.py:322-447)."""
+    """Frequency-domain NLS readout: lock-in demodulation + 4-parameter LM fit per buffer (fitters.py:322-447).
+
+    ``uncertainties=True`` adds the one-sigma errors ``amp_err, m_err, phi_err, psi_err`` of every buffer: square roots
+    of the diagonal of s^2 (J^T J)^-1 at the fitted parameters, s^2 = ssq / (2 ndata - 4) (``dfk_lm_cov``).  They are
+    reported whatever the buffer's ``fitok``; filter on it as for the parameters."""
 
     def fit(self, main_raw, **kwargs) -> pd.DataFrame:
         n = self.config["n"]
+        uncertainties = bool(kwargs.get("uncertainties", False))
         ndata = self.config.get("ndata", 10)
         if "ndata" in kwargs:
             ndata = kwargs.pop("ndata")
@@ -122,24 +133,30 @@ class StandardNLSFitter(BaseFitter):
             import torch
             ctx = _lib.get_context(xd.device.index)
             rows_d = torch.empty((nbuf, _lib.ROW_STRIDE), dtype=torch.float64, device=xd.device)
+            cov_d = torch.empty((nbuf, _lib.COV_STRIDE), dtype=torch.float64, device=xd.device) if uncertainties else None
             with torch.cuda.device(xd.device):
                 ctx.use_torch_stream()
                 try:
                     ctx.nls_fit_dev(xd.data_ptr(), nbuf, R, int(ndata), w0, [init_a, init_m, 0.0, init_psi], chunks, opts,
-                                    rows_d.data_ptr())
+                                    rows_d.data_ptr(), cov_ptr=cov_d.data_ptr() if uncertainties else None)
                 finally:
                     ctx.use_default_stream()
-            return rows_to_frame(rows_d.cpu().numpy())
+            return rows_to_frame(rows_d.cpu().numpy(), cov_d.cpu().numpy() if uncertainties else None)
         x = _record_values(main_raw)[: nbuf * R]  # the reference's reshape(-1, R) raises on a ragged tail (Q7)
         ctx = _lib.get_context(device)
-        rows = ctx.nls_fit_host(x, R, int(ndata), w0, [init_a, init_m, 0.0, init_psi], seeded=chunks, opts=opts)
-        return rows_to_frame(rows)
+        cov = np.empty((nbuf, _lib.COV_STRIDE), dtype=np.float64) if uncertainties else None
+        rows = ctx.nls_fit_host(x, R, int(ndata), w0, [init_a, init_m, 0.0, init_psi], seeded=chunks, opts=opts, cov_out=cov)
+        return rows_to_frame(rows, cov)
 
 
 class EKFFitter(BaseFitter):
     """Time-domain 5-state EKF (fitters.py:210-320): one thread per channel, sequential in time."""
 
     def fit(self, main_raw, **kwargs) -> pd.DataFrame:
+        if kwargs.get("uncertainties", False):
+            # the filter's covariance P is not a per-buffer parameter covariance (its update is deferred inside the
+            # hot loop); only the NLS readout reports uncertainties
+            raise ValueError("uncertainties=True is supported by the NLS fitter only, not by the EKF")
         n = self.config["n"]
         opts = _lib.default_ekf_opts()
         opts.init[0] = kwargs.get("init_a", 1.6)
@@ -182,7 +199,7 @@ class EKFFitter(BaseFitter):
 # additive batch API
 # ------------------------------------------------------------------------------------------------------
 def nls_fit_batch(x, f_samp, f_mod, n, ndata=10, init_a=1.6, init_m=6.0, init_psi=0.0, seeded=True, device=0,
-                  tunables_from=None, return_tensor=False, time_major=False):
+                  tunables_from=None, return_tensor=False, time_major=False, return_cov=False):
     """NLS readout of C channel records in one pass.
 
     x: ``[C, T]`` float64 -- a numpy array (copied to the GPU) or a CUDA torch tensor (used in place).
@@ -193,6 +210,8 @@ def nls_fit_batch(x, f_samp, f_mod, n, ndata=10, init_a=1.6, init_m=6.0, init_ps
     seeded: False -> independent cold starts; True -> every buffer from its channel's buffer 0; an int k ->
     the reference's k-chunk chain schedule per channel (1 = ``parallel=False``).
     Returns rows ``[C, nbuf, 8]`` = amp, m, phi, psi, dc, ssq, fitok, accepted LM steps.
+    return_cov: return ``(rows, cov)`` with the covariance rows ``[C, nbuf, 8]`` = C_aa, C_am, C_aphi, C_mm, C_mphi,
+    C_phiphi, C_psipsi, s^2 of every buffer (``dfk_lm_cov``), of the same kind as rows.
     """
     import torch
     ctx = _lib.get_context(device)
@@ -225,8 +244,15 @@ def nls_fit_batch(x, f_samp, f_mod, n, ndata=10, init_a=1.6, init_m=6.0, init_ps
     bpc = T // R
     w0 = 2.0 * np.pi * f_mod / f_samp
     rows = torch.empty((C, bpc, _lib.ROW_STRIDE), dtype=torch.float64, device=dev)
+    cov = torch.empty((C, bpc, _lib.COV_STRIDE), dtype=torch.float64, device=dev) if return_cov else None
+    cov_ptr = cov.data_ptr() if return_cov and C * bpc > 0 else None
+
+    def result():
+        out = [t if return_tensor else t.cpu().numpy() for t in ((rows, cov) if return_cov else (rows,))]
+        return tuple(out) if return_cov else out[0]
+
     if C * bpc == 0:
-        return rows if return_tensor else rows.cpu().numpy()
+        return result()
     per_channel = any(np.ndim(v) > 0 for v in (init_a, init_m, init_psi))
     init_dev_ptr, init_stride, init = None, 0, [float(np.ravel(init_a)[0]), float(np.ravel(init_m)[0]), 0.0,
                                                   float(np.ravel(init_psi)[0])]
@@ -244,19 +270,20 @@ def nls_fit_batch(x, f_samp, f_mod, n, ndata=10, init_a=1.6, init_m=6.0, init_ps
             if native_tm:
                 try:
                     ctx.nls_fit_batch_tm_dev(xt.data_ptr(), C, bpc, R, int(ndata), w0, init, init_dev_ptr, init_stride,
-                                             seeded, fit_tunables.current_lm_opts(tunables_from), rows.data_ptr())
+                                             seeded, fit_tunables.current_lm_opts(tunables_from), rows.data_ptr(),
+                                             cov_ptr=cov_ptr)
                 except RuntimeError:  # a geometry the fold cannot take after all: transpose and go channel-major
                     xc = torch.empty((C, T), dtype=torch.float64, device=dev)
                     ctx.widen_dev(xt.data_ptr(), "float64", T, C, True, xc.data_ptr(), max(T, 1))
                     xt, native_tm = xc, False
             if not native_tm:
                 ctx.nls_fit_batch_dev(xt.data_ptr(), C, bpc, T, R, int(ndata), w0, init, init_dev_ptr, init_stride, seeded,
-                                      fit_tunables.current_lm_opts(tunables_from), rows.data_ptr())
+                                      fit_tunables.current_lm_opts(tunables_from), rows.data_ptr(), cov_ptr=cov_ptr)
         finally:
             ctx.use_default_stream()
         torch.cuda.current_stream(dev).synchronize()
     del keep
-    return rows if return_tensor else rows.cpu().numpy()
+    return result()
 
 
 def ekf_fit_batch(z, f_samp, f_mod, n, time_major=False, device=0, return_tensor=False, **kwargs):

@@ -73,7 +73,7 @@ def crlb_sigma_m(m_true: float, ndata: int, snr_db: float, buffer_size: int) -> 
 
 def nls_sweep(m_values, n_trials, snr_db=40.0, f_samp=200e3, f_mod=1000.0, n=1, ndata=15, init_a=1.6, init_m=None,
               amp=1.0, visibility=1.0, phi0=0.0, psi0=0.0, seed=0, device=0, max_resident_bytes=8 << 30,
-              tunables_from=None, return_rows=False, _seed_stride=None, _raw_stats=False):
+              tunables_from=None, return_rows=False, uncertainties=False, _seed_stride=None, _raw_stats=False):
     """Fit ``n_trials`` independent single-buffer realisations at every m in ``m_values``.
 
     init_m: None -> each realisation starts from its true m (workers.py:167-173); a float -> the same cold start
@@ -81,6 +81,9 @@ def nls_sweep(m_values, n_trials, snr_db=40.0, f_samp=200e3, f_mod=1000.0, n=1, 
     Returns a dict of per-m arrays: ``m_mean, m_std, m_min, m_max, m_worst`` (largest |m_hat - m|), the same for
     ``amp, phi, psi``, ``ssq_mean``, ``fitok`` fractions ``[len(m), 3]``, ``crlb_sigma_m``, and with return_rows the
     raw ``[len(m), n_trials, 8]`` table.
+    uncertainties: also fit every realisation's parameter covariance (``dfk_nls_sweep_cov_dev``) and report per m
+    ``amp_err_rms, m_err_rms, phi_err_rms, psi_err_rms``, the square root of the mean predicted variance over all trials
+    -- to set beside ``*_std`` and ``crlb_sigma_m``; with return_rows also the ``[len(m), n_trials, 8]`` table ``cov``.
     """
     import torch
     ms = np.atleast_1d(np.asarray(m_values, dtype=np.float64))
@@ -93,10 +96,13 @@ def nls_sweep(m_values, n_trials, snr_db=40.0, f_samp=200e3, f_mod=1000.0, n=1, 
     per_fit = 8 * (2 * int(ndata) + 1) + 8 * _lib.ROW_STRIDE + 16
     per_wave = max(1, min(int(n_trials), int(max_resident_bytes // (len(ms) * per_fit))))
     seed_stride = int(n_trials) if _seed_stride is None else int(_seed_stride)
+    # (uncertainties add 64 bytes of covariance per fit on top; the waves, and so the rows, stay those without them)
     waves = []
     all_rows = [] if return_rows else None
+    all_cov = [] if return_rows and uncertainties else None
     with torch.cuda.device(dev):
         rows = torch.empty((len(ms), per_wave, _lib.ROW_STRIDE), dtype=torch.float64, device=dev)
+        cov = torch.empty((len(ms), per_wave, _lib.COV_STRIDE), dtype=torch.float64, device=dev) if uncertainties else None
         truth = torch.from_numpy(np.stack([np.full_like(ms, amp), ms, np.full_like(ms, phi0), np.full_like(ms, psi0)], 1)).to(dev)
         center = torch.zeros((len(ms), 7), dtype=torch.float64, device=dev)
         center[:, :4] = truth
@@ -107,18 +113,28 @@ def nls_sweep(m_values, n_trials, snr_db=40.0, f_samp=200e3, f_mod=1000.0, n=1, 
                 nw = min(per_wave, n_trials - done)
                 rv = rows[:, :nw] if nw == per_wave else torch.empty((len(ms), nw, _lib.ROW_STRIDE), dtype=torch.float64,
                                                                       device=dev)
+                cv = None
+                if uncertainties:
+                    cv = cov[:, :nw] if nw == per_wave else torch.empty((len(ms), nw, _lib.COV_STRIDE), dtype=torch.float64,
+                                                                         device=dev)
                 # realisation t of grid point i is noise stream seed + i * seed_stride + t, whatever the wave it falls
                 # in: generated inside the demodulation kernel (dfk_nls_sweep_dev), fitted cold in one launch
                 ctx.nls_sweep_dev(ms, nw, done, seed_stride, R, int(ndata), f_samp, f_mod, rv.data_ptr(), amp=amp,
                                   visibility=visibility, phi0=phi0, psi0=psi0, snr_db=snr_db, seed=seed, init_a=init_a,
-                                  init_m=init_m, opts=opts)
+                                  init_m=init_m, opts=opts, cov_ptr=cv.data_ptr() if uncertainties else None)
                 # per-m statistics of the wave in one pass of the reduction kernel: columns amp, m, phi, psi, (dc,) ssq,
                 # fitok; "worst" measured from the true parameters
                 st = torch.empty((len(ms), 7, _lib.TRIAL_STATS_DOUBLES), dtype=torch.float64, device=dev)
                 ctx.trial_stats_dev(rv.data_ptr(), len(ms), nw, 7, _lib.ROW_STRIDE, st.data_ptr(), center_ptr=center.data_ptr())
-                waves.append((nw, st))
+                cst = None
+                if uncertainties:  # mean predicted variance per m: covariance columns 0, 3, 5, 6 of the same reduction
+                    cst = torch.empty((len(ms), 7, _lib.TRIAL_STATS_DOUBLES), dtype=torch.float64, device=dev)
+                    ctx.trial_stats_dev(cv.data_ptr(), len(ms), nw, 7, _lib.COV_STRIDE, cst.data_ptr())
+                waves.append((nw, st, cst))
                 if return_rows:
                     all_rows.append(rv.cpu().numpy().copy())
+                    if uncertainties:
+                        all_cov.append(cv.cpu().numpy().copy())
                 done += nw
             torch.cuda.current_stream(dev).synchronize()
         finally:
@@ -126,7 +142,13 @@ def nls_sweep(m_values, n_trials, snr_db=40.0, f_samp=200e3, f_mod=1000.0, n=1, 
     tr = truth.cpu().numpy()
     part = {"n": int(n_trials), "truth": tr, "sum": 0.0, "sumsq": 0.0, "ok": 0.0, "ssq": 0.0,
             "min": np.full((len(ms), 4), np.inf), "max": np.full((len(ms), 4), -np.inf), "worst": np.zeros((len(ms), 4))}
-    for nw, st in waves:
+    if uncertainties:
+        part["var_sum"], part["var_n"] = 0.0, 0.0
+    for nw, st, cst in waves:
+        if cst is not None:  # nan-aware: weight each wave's mean by its number of finite trials
+            c_ = cst.cpu().numpy()[:, [0, 3, 5, 6]]
+            part["var_sum"] = part["var_sum"] + np.nan_to_num(c_[:, :, 0]) * c_[:, :, 5]
+            part["var_n"] = part["var_n"] + c_[:, :, 5]
         s_ = st.cpu().numpy()
         mean, std = s_[:, :4, 0], s_[:, :4, 1]
         part["sum"] = part["sum"] + mean * nw
@@ -144,8 +166,15 @@ def nls_sweep(m_values, n_trials, snr_db=40.0, f_samp=200e3, f_mod=1000.0, n=1, 
     if _raw_stats:
         return part
     out = _combine_partials(ms, [part], ndata, snr_db, R)
+    if uncertainties:
+        with np.errstate(invalid="ignore", divide="ignore"):
+            rms = np.sqrt(part["var_sum"] / part["var_n"])
+        for c, name in enumerate(("amp", "m", "phi", "psi")):
+            out[f"{name}_err_rms"] = rms[:, c]
     if return_rows:
         out["rows"] = np.concatenate(all_rows, axis=1)
+        if uncertainties:
+            out["cov"] = np.concatenate(all_cov, axis=1)
     return out
 
 
@@ -163,6 +192,8 @@ def nls_sweep_sharded(m_values, n_trials, group=None, device=None, seed=0, **kwa
 
     if kwargs.pop("return_rows", False):
         raise ValueError("return_rows is a single-GPU option")
+    if kwargs.pop("uncertainties", False):
+        raise ValueError("uncertainties is a single-GPU option")
     rank, world = dist.get_rank(group), dist.get_world_size(group)
     lo, hi = slab_bounds(int(n_trials), world, rank)
     if device is None:

@@ -15,6 +15,9 @@
  *   - result row       [amp, m, phi, psi, dc, ssq, fitok, aux] (8 doubles, DFK_ROW_STRIDE);
  *     columns 0..6 are the reference's result-frame columns (fitters.py:55-58), fitok stored
  *     as a double holding 0/1/2; aux = accepted LM steps (NLS) or 0 (EKF)
+ *   - covariance row [C_aa, C_am, C_aphi, C_mm, C_mphi, C_phiphi, C_psipsi, s^2] (8 doubles,
+ *     DFK_COV_STRIDE), one per result row and laid out like the rows: s^2 (J^T J)^-1 at the row's
+ *     parameters, s^2 = ssq / (2N - 4) (see dfk_lm_cov)
  *   - "dev" pointers are device pointers on the context's device; "host" pointers are host
  *     memory (pinned memory is detected and copied from directly, pageable memory is staged)
  *   - all calls return 0 on success or a negative DFK_ERR_* code; dfk_last_error() gives the
@@ -30,8 +33,9 @@
 extern "C" {
 #endif
 
-#define DFK_ABI_VERSION 4
+#define DFK_ABI_VERSION 5
 #define DFK_ROW_STRIDE 8
+#define DFK_COV_STRIDE 8
 #define DFK_MAX_HARMONICS 64
 
 #define DFK_PROFILE_KINDS 4
@@ -149,11 +153,26 @@ int dfk_demod(dfk_ctx* ctx, const double* x_dev, int64_t nbuf, int64_t R, int32_
 int dfk_lm_fit(dfk_ctx* ctx, const double* qi_dev, int64_t nbuf, int32_t N, const double* guess_dev,
                int64_t guess_stride, const double* dc_dev, const dfk_lm_opts* opts, double* rows_dev);
 
+/* Parameter covariance of nbuf fitted rows (rows_dev: nbuf x DFK_ROW_STRIDE, e.g. from dfk_lm_fit) on their harmonic
+ * vectors qi_dev (nbuf x 2N, from dfk_demod): the standard NLS estimate s^2 (J^T J)^-1, J^T J of the harmonic model at
+ * the row's own amp, m, phi, psi and s^2 = ssq / (2N - 4) from the row's ssq.  The reference forms the same
+ * inv(J^T J) sigma^2 only at the true parameters, for its Cramer-Rao bound (helpers.py:16-45, 60-96).
+ * cov_dev: nbuf x DFK_COV_STRIDE = [C_aa, C_am, C_aphi, C_mm, C_mphi, C_phiphi, C_psipsi, s^2]; the psi cross terms are
+ * identically zero.  The estimate takes the residual scatter as the noise level; a caller who knows the I/Q noise
+ * variance sigma^2 rescales by sigma^2 / s^2.  Every row is computed whatever its fitok; filter on fitok as for the
+ * parameters.  Degenerate rows: 2N - 4 <= 0 or a non-finite parameter -> all eight NaN; a singular amp/m/phi block
+ * (e.g. amp = 0) -> its six entries NaN; a vanishing psi column -> C_psipsi NaN; ssq = 0 -> zeros. */
+int dfk_lm_cov(dfk_ctx* ctx, const double* qi_dev, int64_t nbuf, int32_t N, const double* rows_dev, double* cov_dev);
+
 /* Whole NLS readout of one device-resident record: demod, fit buffer 0 from init, fit the other
  * buffers on the schedule `seeded` names (DFK_SCHED_* above).  Replaces StandardNLSFitter._fit_sequential
  * (fitters.py:370-393) and _fit_parallel with its multiprocessing.Pool (fitters.py:395-428). */
 int dfk_nls_fit_dev(dfk_ctx* ctx, const double* x_dev, int64_t nbuf, int64_t R, int32_t N, double w0,
                     const double init[4], int32_t seeded, const dfk_lm_opts* opts, double* rows_dev);
+/* The same, plus the covariance row of every buffer (dfk_lm_cov on the record's harmonic vectors and the final rows)
+ * in cov_dev: nbuf x DFK_COV_STRIDE.  Rows are those of dfk_nls_fit_dev.  (helpers.py:16-45, 60-96) */
+int dfk_nls_fit_cov_dev(dfk_ctx* ctx, const double* x_dev, int64_t nbuf, int64_t R, int32_t N, double w0,
+                        const double init[4], int32_t seeded, const dfk_lm_opts* opts, double* rows_dev, double* cov_dev);
 
 /* A slab of a record whose buffer 0 lives elsewhere (another GPU): the slab is `chunks` chunks (>= 1, or
  * DFK_SCHED_EACH) whose first buffers start from seed[4], the fitted [amp, m, phi, psi] of the record's
@@ -171,6 +190,10 @@ int dfk_nls_fit_seeded_dev(dfk_ctx* ctx, const double* x_dev, int64_t nbuf, int6
 int dfk_nls_fit_batch_dev(dfk_ctx* ctx, const double* x_dev, int64_t C, int64_t bufs_per_channel, int64_t ld_c,
                           int64_t R, int32_t N, double w0, const double init[4], const double* init_dev,
                           int64_t init_stride, int32_t seeded, const dfk_lm_opts* opts, double* rows_dev);
+/* The same with covariance rows, cov_dev: C x bufs_per_channel x DFK_COV_STRIDE (helpers.py:16-45, 60-96). */
+int dfk_nls_fit_batch_cov_dev(dfk_ctx* ctx, const double* x_dev, int64_t C, int64_t bufs_per_channel, int64_t ld_c,
+                              int64_t R, int32_t N, double w0, const double init[4], const double* init_dev,
+                              int64_t init_stride, int32_t seeded, const dfk_lm_opts* opts, double* rows_dev, double* cov_dev);
 
 /* The same for a TIME-MAJOR record, sample (t, c) at x_dev[t * C + c] (interleaved channels: the layout acquisition
  * hardware and the DFMSWPM text format produce), without a transposition pass: an interleaved buffer folds like one
@@ -183,6 +206,10 @@ int dfk_demod_tm_dev(dfk_ctx* ctx, const double* x_dev, int64_t bufs_per_channel
 int dfk_nls_fit_batch_tm_dev(dfk_ctx* ctx, const double* x_dev, int64_t C, int64_t bufs_per_channel, int64_t R, int32_t N,
                              double w0, const double init[4], const double* init_dev, int64_t init_stride, int32_t seeded,
                              const dfk_lm_opts* opts, double* rows_dev);
+/* The same with covariance rows, cov_dev: C x bufs_per_channel x DFK_COV_STRIDE (helpers.py:16-45, 60-96). */
+int dfk_nls_fit_batch_tm_cov_dev(dfk_ctx* ctx, const double* x_dev, int64_t C, int64_t bufs_per_channel, int64_t R, int32_t N,
+                                 double w0, const double init[4], const double* init_dev, int64_t init_stride, int32_t seeded,
+                                 const dfk_lm_opts* opts, double* rows_dev, double* cov_dev);
 
 /* 5-state EKF over C independent channels, one thread per channel.
  * Replaces EKFFitter.fit (fitters.py:214-320).  Sample (t, c) is z_dev[t*ld_t + c*ld_c]
@@ -234,6 +261,12 @@ int dfk_nls_sweep_dev(dfk_ctx* ctx, const double* m_values, int32_t nm, int64_t 
                       int64_t R, int32_t N, double f_samp, double f_mod, double amp, double visibility, double phi0,
                       double psi0, double snr_db, uint64_t seed, double init_a, double init_m, const dfk_lm_opts* opts,
                       double* rows_dev);
+/* The same with covariance rows, cov_dev: nm x ntrials x DFK_COV_STRIDE -- the notebook's inv(J^T J) sigma^2 of
+ * helpers.py:16-45, 60-96 at every fitted realisation instead of at the truth only. */
+int dfk_nls_sweep_cov_dev(dfk_ctx* ctx, const double* m_values, int32_t nm, int64_t ntrials, int64_t trial0,
+                          int64_t seed_stride, int64_t R, int32_t N, double f_samp, double f_mod, double amp, double visibility,
+                          double phi0, double psi0, double snr_db, uint64_t seed, double init_a, double init_m,
+                          const dfk_lm_opts* opts, double* rows_dev, double* cov_dev);
 
 /* ---- host-pointer entry points (what the reference-side shim binds) ---------------------- */
 /* StandardNLSFitter.fit on one host record (fitters.py:330-428): nsamp samples, buffers of R,
@@ -241,6 +274,10 @@ int dfk_nls_sweep_dev(dfk_ctx* ctx, const double* m_values, int32_t nm, int64_t 
  * fitted.  rows_host: (nsamp / R) x DFK_ROW_STRIDE. */
 int dfk_nls_fit_host(dfk_ctx* ctx, const double* x_host, int64_t nsamp, int64_t R, int32_t N, double w0,
                      const double init[4], int32_t seeded, const dfk_lm_opts* opts, double* rows_host);
+/* The same with covariance rows, cov_host: (nsamp / R) x DFK_COV_STRIDE.  Each slab's covariance comes from that slab's
+ * harmonic vectors after its last LM launch; one more copy back beside the rows' (helpers.py:16-45, 60-96). */
+int dfk_nls_fit_cov_host(dfk_ctx* ctx, const double* x_host, int64_t nsamp, int64_t R, int32_t N, double w0,
+                         const double init[4], int32_t seeded, const dfk_lm_opts* opts, double* rows_host, double* cov_host);
 
 /* dfk_nls_fit_seeded_dev for a host slab (same streaming as dfk_nls_fit_host): what each rank of a record sharded
  * over several GPUs calls on its own slab once buffer 0's result is known. */
