@@ -17,7 +17,7 @@ from ._build import LIB_PATH
 ROW_STRIDE = 8
 COV_STRIDE = 8          # [C_aa, C_am, C_aphi, C_mm, C_mphi, C_phiphi, C_psipsi, s^2] per result row
 MAX_HARMONICS = 64
-ABI_VERSION = 5
+ABI_VERSION = 6
 PROFILE_KINDS = 4
 ASD_TRIAL_DOUBLES = 37
 TRIAL_STATS_DOUBLES = 6
@@ -127,6 +127,8 @@ SYMBOLS = {
                                      _vp]),
     "dfk_lpsd_dev": (ctypes.c_int, [_vp, _vp, _i64, _i64, _i64, _i64, _d, ctypes.POINTER(LpsdOpts), _i32,
                                     ctypes.POINTER(_i32), _vp, _vp, _vp, _vp, _vp]),
+    "dfk_lcsd_dev": (ctypes.c_int, [_vp, _vp, _i64, _i64, _vp, _i64, _i64, _i64, _i64, _d, ctypes.POINTER(LpsdOpts),
+                                    _i32, ctypes.POINTER(_i32), _vp, _vp, _vp, _vp, _vp, _vp]),
     "dfk_lm_counters_read": (ctypes.c_int, [_vp, ctypes.POINTER(LmCounters), _i32]),
     "dfk_profile_enable": (ctypes.c_int, [_vp, _i32]),
     "dfk_profile_read": (ctypes.c_int, [_vp, c_double_p, ctypes.POINTER(_i64), _i32]),
@@ -498,6 +500,23 @@ class Context:
                                                ctypes.byref(opts), n, ctypes.byref(nf), f.ctypes.data, ps.ctypes.data,
                                                psd.ctypes.data, enbw.ctypes.data, navs.ctypes.data))
         return {"f": f, "ps": ps, "psd": psd, "enbw": enbw, "navs": navs}
+
+    def lcsd_dev(self, x_ptr, Cx, ldx, y_ptr, Cy, ldy, N, stride, fs, opts=None) -> dict:
+        """Cross-spectral densities of Cx device-resident series x against Cy series y on the LPSD plan; returns host
+        arrays f[nf], Sxx[Cx, nf], Syy[Cy, nf], Sxy[Cx, Cy, nf] (complex128), enbw[nf], navs[nf]."""
+        opts = opts if opts is not None else default_lpsd_opts()
+        nf = _i32()
+        _check(self.lib, self.lib.dfk_lpsd_plan(int(N), float(fs), ctypes.byref(opts), 0, ctypes.byref(nf), None, None,
+                                                None, None, None))
+        n = int(nf.value)
+        f, enbw, navs = np.empty(n), np.empty(n), np.empty(n, dtype=np.int64)
+        sxx, syy = np.empty((int(Cx), n)), np.empty((int(Cy), n))
+        sxy = np.empty((int(Cx), int(Cy), n), dtype=np.complex128)
+        _check(self.lib, self.lib.dfk_lcsd_dev(self._h, x_ptr, int(Cx), int(ldx), y_ptr, int(Cy), int(ldy), int(N),
+                                               int(stride), float(fs), ctypes.byref(opts), n, ctypes.byref(nf),
+                                               f.ctypes.data, sxx.ctypes.data, syy.ctypes.data, sxy.ctypes.data,
+                                               enbw.ctypes.data, navs.ctypes.data))
+        return {"f": f, "Sxx": sxx, "Syy": syy, "Sxy": sxy, "enbw": enbw, "navs": navs}
 
     def set_host_slab_bytes(self, nbytes=0):
         """Slab size of the host-pointer entries (0: defaults); small values make a short record stream."""

@@ -6,7 +6,8 @@ Everything either side of the readout path is here under the reference's names: 
 stay with the reference (``fit`` hands those method names to the reference's classes when it is importable;
 INTEGRATION.md shows the opposite direction too: the reference's own façade pointed at these fitters).  Call
 signatures, default labels, the ``tau`` column, the error behaviour (log + ``None``) and the fields of the returned
-objects are those of the reference.
+objects are those of the reference.  ``DeepFitObject.calc_csd`` is this package's addition: the cross-spectral estimate
+(CSD, coherence, transfer function) of one fit against another on the LPSD frequency plan.
 """
 from __future__ import annotations
 
@@ -173,6 +174,21 @@ class DeepFitObject:
         from .spectra import lpsd
         self.f, _, self.Sxx, _, _, _ = lpsd(self.phi, self.fs, self.olap, self.bmin, self.Lmin, self.Jdes, self.Kdes,
                                             self.order, self.win, self.psll, return_type="legacy")
+
+    def calc_csd(self, other, column="phi"):
+        """Cross-spectral estimate of this fit's ``column`` against ``other``'s on the device, with this object's
+        spectral settings: the ``lcsd`` dict (f, Sxx, Syy, Sxy, coh, tf, enbw, navs), this fit as x and ``other`` as y.
+        Stores nothing.  Both fits must have the same fit rate and the same number of buffers."""
+        from .spectra import lcsd
+        if self.fs != other.fs:
+            raise ValueError(f"fit rates differ: {self.fs} and {other.fs}")
+        x, y = getattr(self, column), getattr(other, column)
+        if x is None or y is None:
+            raise ValueError(f"both fits need a '{column}' series")
+        if len(x) != len(y):
+            raise ValueError(f"series lengths differ: {len(x)} and {len(y)}")
+        return lcsd(x, y, self.fs, self.olap, self.bmin, self.Lmin, self.Jdes, self.Kdes, self.order, self.win,
+                    self.psll)
 
 
 class DeepFitFramework:

@@ -83,6 +83,67 @@ int make_plan(int64_t N, double fs, const dfk_lpsd_opts& o, std::vector<PlanRow>
     return DFK_OK;
 }
 
+// The device plan of one LPSD / LCSD call, built in one place so that both estimates use the same segments.
+struct DevicePlan {
+    std::vector<PlanRow> rows;          // make_plan's rows, K trimmed as below
+    std::vector<dfk::LpsdFreq> freq;
+    long long tiles = 0, groups = 0;    // per series
+};
+
+int make_device_plan(int64_t N, double fs, const dfk_lpsd_opts& o, DevicePlan& dp) {
+    const int rc = make_plan(N, fs, o, dp.rows);
+    if (rc) return rc;
+    const int nf = static_cast<int>(dp.rows.size());
+    dp.freq.resize(nf);
+    dp.tiles = dp.groups = 0;
+    for (int j = 0; j < nf; ++j) {
+        dfk::LpsdFreq& F = dp.freq[j];
+        PlanRow& row = dp.rows[j];
+        F.L = row.L;
+        F.K = row.K;
+        F.p = 2.0 * dfk::kPi * row.m / static_cast<double>(row.L);
+        double shift = F.K == 1 ? 1.0 : static_cast<double>(N - F.L) / static_cast<double>(F.K - 1);
+        if (shift < 1.0) shift = 1.0;
+        F.shift = shift;
+        // the last segment must stay inside the record whatever the rounding of the plan
+        while (F.K > 1 && static_cast<long long>(std::floor((F.K - 1) * shift + 0.5)) + F.L > N) F.K--;
+        row.K = F.K;
+        const long long ng = (F.K + dfk::kLpsdGroup - 1) / dfk::kLpsdGroup;
+        F.tile0 = dp.tiles;
+        F.group0 = dp.groups;
+        dp.tiles += F.L >= dfk::kLpsdCtaMin ? ng : (ng + dfk::kLpsdThreads / 32 - 1) / (dfk::kLpsdThreads / 32);
+        dp.groups += ng;
+    }
+    return DFK_OK;
+}
+
+// Kernel parameters of a plan already copied to plan_dev; the caller sets the series and the scratch.
+dfk::LpsdParams lpsd_params(const DevicePlan& dp, const void* plan_dev, int64_t N, int64_t stride,
+                            const dfk_lpsd_opts& o) {
+    dfk::LpsdParams P;
+    P.x = nullptr;
+    P.N = N;
+    P.stride = stride;
+    P.ld_c = 0;
+    P.plan = static_cast<const dfk::LpsdFreq*>(plan_dev);
+    P.nf = static_cast<int>(dp.freq.size());
+    P.ntiles = dp.tiles;
+    P.ngroups = dp.groups;
+    P.order = o.order;
+    P.window = o.window;
+    P.beta = dfk::kPi * kaiser_alpha(o.psll);
+    P.inv_i0_beta = 1.0 / host_i0(P.beta);
+    P.group_sum = nullptr;
+    return P;
+}
+
+void copy_plan_out(const DevicePlan& dp, double* f_host, int64_t* navs_host) {
+    for (size_t j = 0; j < dp.rows.size(); ++j) {
+        if (f_host) f_host[j] = dp.rows[j].f;
+        if (navs_host) navs_host[j] = dp.rows[j].K;
+    }
+}
+
 }  // namespace
 
 extern "C" {
@@ -132,33 +193,14 @@ int dfk_lpsd_dev(dfk_ctx* ctx, const double* x_dev, int64_t N, int64_t stride, i
     }
     if (!x_dev || !nf_out) return fail(DFK_ERR_ARG, "null pointer");
     if (C < 1 || stride < 1) return fail(DFK_ERR_ARG, "bad geometry: C=%lld stride=%lld", (long long)C, (long long)stride);
-    std::vector<PlanRow> rows;
-    int rc = make_plan(N, fs, *opts, rows);
+    DevicePlan dp;
+    int rc = make_device_plan(N, fs, *opts, dp);
     if (rc) return rc;
-    const int nf = static_cast<int>(rows.size());
+    const int nf = static_cast<int>(dp.rows.size());
     *nf_out = nf;
     if (nf > cap) return fail(DFK_ERR_ARG, "plan has %d frequencies, outputs hold %d (call dfk_lpsd_plan first)", nf, cap);
     if (nf == 0) return DFK_OK;
-
-    std::vector<dfk::LpsdFreq> plan(nf);
-    long long tiles = 0, groups = 0;
-    for (int j = 0; j < nf; ++j) {
-        dfk::LpsdFreq& F = plan[j];
-        F.L = rows[j].L;
-        F.K = rows[j].K;
-        F.p = 2.0 * dfk::kPi * rows[j].m / static_cast<double>(rows[j].L);
-        double shift = F.K == 1 ? 1.0 : static_cast<double>(N - F.L) / static_cast<double>(F.K - 1);
-        if (shift < 1.0) shift = 1.0;
-        F.shift = shift;
-        // the last segment must stay inside the record whatever the rounding of the plan
-        while (F.K > 1 && static_cast<long long>(std::floor((F.K - 1) * shift + 0.5)) + F.L > N) F.K--;
-        rows[j].K = F.K;
-        const long long ng = (F.K + dfk::kLpsdGroup - 1) / dfk::kLpsdGroup;
-        F.tile0 = tiles;
-        F.group0 = groups;
-        tiles += F.L >= dfk::kLpsdCtaMin ? ng : (ng + dfk::kLpsdThreads / 32 - 1) / (dfk::kLpsdThreads / 32);
-        groups += ng;
-    }
+    const long long tiles = dp.tiles, groups = dp.groups;
     if (tiles > 0x7fffffffll || C > 65535) return fail(DFK_ERR_ARG, "LPSD problem too large for one launch");
     DevBuf& plan_dev = ctx->post[0];
     DevBuf& group_dev = ctx->post[1];
@@ -168,20 +210,10 @@ int dfk_lpsd_dev(dfk_ctx* ctx, const double* x_dev, int64_t N, int64_t stride, i
     if (!rc) rc = ensure(ctx, out_dev, sizeof(double) * (2 * C + 1) * nf);
     if (rc) return rc;
     cudaStream_t st = ctx->stream();
-    DFK_CUDA(cudaMemcpyAsync(plan_dev.ptr, plan.data(), sizeof(dfk::LpsdFreq) * nf, cudaMemcpyHostToDevice, st));
-    dfk::LpsdParams P;
+    DFK_CUDA(cudaMemcpyAsync(plan_dev.ptr, dp.freq.data(), sizeof(dfk::LpsdFreq) * nf, cudaMemcpyHostToDevice, st));
+    dfk::LpsdParams P = lpsd_params(dp, plan_dev.ptr, N, stride, *opts);
     P.x = x_dev;
-    P.N = N;
-    P.stride = stride;
     P.ld_c = ld_c;
-    P.plan = static_cast<const dfk::LpsdFreq*>(plan_dev.ptr);
-    P.nf = nf;
-    P.ntiles = tiles;
-    P.ngroups = groups;
-    P.order = opts->order;
-    P.window = opts->window;
-    P.beta = dfk::kPi * kaiser_alpha(opts->psll);
-    P.inv_i0_beta = 1.0 / host_i0(P.beta);
     P.group_sum = static_cast<double*>(group_dev.ptr);
     double* ps_dev = static_cast<double*>(out_dev.ptr);
     double* psd_dev = ps_dev + C * nf;
@@ -196,10 +228,71 @@ int dfk_lpsd_dev(dfk_ctx* ctx, const double* x_dev, int64_t N, int64_t stride, i
     if (psd_host) DFK_CUDA(cudaMemcpyAsync(psd_host, psd_dev, sizeof(double) * C * nf, cudaMemcpyDeviceToHost, st));
     if (enbw_host) DFK_CUDA(cudaMemcpyAsync(enbw_host, enbw_dev, sizeof(double) * nf, cudaMemcpyDeviceToHost, st));
     DFK_CUDA(cudaStreamSynchronize(st));
-    for (int j = 0; j < nf; ++j) {
-        if (f_host) f_host[j] = rows[j].f;
-        if (navs_host) navs_host[j] = rows[j].K;
+    copy_plan_out(dp, f_host, navs_host);
+    return DFK_OK;
+}
+
+int dfk_lcsd_dev(dfk_ctx* ctx, const double* x_dev, int64_t Cx, int64_t ldx, const double* y_dev, int64_t Cy,
+                 int64_t ldy, int64_t N, int64_t stride, double fs, const dfk_lpsd_opts* opts, int32_t cap,
+                 int32_t* nf_out, double* f_host, double* sxx_host, double* syy_host, double* sxy_host,
+                 double* enbw_host, int64_t* navs_host) {
+    DFK_ENTER(ctx);
+    dfk_lpsd_opts d;
+    if (!opts) {
+        dfk_default_lpsd_opts(&d);
+        opts = &d;
     }
+    if (!x_dev || !y_dev || !nf_out) return fail(DFK_ERR_ARG, "null pointer");
+    if (Cx < 1 || Cy < 1 || stride < 1)
+        return fail(DFK_ERR_ARG, "bad geometry: Cx=%lld Cy=%lld stride=%lld", (long long)Cx, (long long)Cy,
+                    (long long)stride);
+    if (Cx + Cy > 65535) return fail(DFK_ERR_ARG, "LCSD takes at most 65535 series in all (Cx + Cy)");
+    DevicePlan dp;
+    int rc = make_device_plan(N, fs, *opts, dp);
+    if (rc) return rc;
+    const int nf = static_cast<int>(dp.rows.size());
+    *nf_out = nf;
+    if (nf > cap) return fail(DFK_ERR_ARG, "plan has %d frequencies, outputs hold %d (call dfk_lpsd_plan first)", nf, cap);
+    if (nf == 0) return DFK_OK;
+    if (dp.tiles > 0x7fffffffll) return fail(DFK_ERR_ARG, "LCSD problem too large for one launch");
+    const long long ns = Cx + Cy, npair = Cx * Cy;
+    const long long nslots = dp.groups * dfk::kLpsdGroup;
+    DevBuf& plan_dev = ctx->post[0];
+    DevBuf& seg_dev = ctx->post[1];
+    DevBuf& out_dev = ctx->post[2];
+    // per-segment projections: 16 B per slot and series; outputs: auto densities, cross densities (re, im), ENBW
+    rc = ensure(ctx, plan_dev, sizeof(dfk::LpsdFreq) * nf);
+    if (!rc) rc = ensure(ctx, seg_dev, sizeof(double2) * static_cast<size_t>(nslots) * static_cast<size_t>(ns));
+    if (!rc) rc = ensure(ctx, out_dev, sizeof(double) * static_cast<size_t>(ns + 2 * npair + 1) * static_cast<size_t>(nf));
+    if (rc) return rc;
+    cudaStream_t st = ctx->stream();
+    DFK_CUDA(cudaMemcpyAsync(plan_dev.ptr, dp.freq.data(), sizeof(dfk::LpsdFreq) * nf, cudaMemcpyHostToDevice, st));
+    dfk::LcsdParams Q;
+    Q.P = lpsd_params(dp, plan_dev.ptr, N, stride, *opts);
+    Q.P.x = x_dev;
+    Q.P.ld_c = ldx;
+    Q.y = y_dev;
+    Q.ld_y = ldy;
+    Q.cx = Cx;
+    Q.cy = Cy;
+    Q.seg = static_cast<double2*>(seg_dev.ptr);
+    Q.nslots = nslots;
+    double* psd_dev = static_cast<double*>(out_dev.ptr);  // [Cx + Cy][nf]: x series, then y
+    double* sxy_dev = psd_dev + ns * nf;                    // [Cx][Cy][nf][2]
+    double* enbw_dev = sxy_dev + 2 * npair * nf;
+    const dim3 grid(static_cast<unsigned>(dp.tiles), static_cast<unsigned>(ns));
+    dfk::lcsd_segment_kernel<<<grid, dfk::kLpsdThreads, 0, st>>>(Q);
+    DFK_CUDA(cudaGetLastError());
+    dfk::lcsd_finish_kernel<<<nf, dfk::kLcsdFinishThreads, 0, st>>>(Q, fs, psd_dev, sxy_dev, enbw_dev);
+    DFK_CUDA(cudaGetLastError());
+    ctx->launches += 2;
+    if (sxx_host) DFK_CUDA(cudaMemcpyAsync(sxx_host, psd_dev, sizeof(double) * Cx * nf, cudaMemcpyDeviceToHost, st));
+    if (syy_host)
+        DFK_CUDA(cudaMemcpyAsync(syy_host, psd_dev + Cx * nf, sizeof(double) * Cy * nf, cudaMemcpyDeviceToHost, st));
+    if (sxy_host) DFK_CUDA(cudaMemcpyAsync(sxy_host, sxy_dev, sizeof(double) * 2 * npair * nf, cudaMemcpyDeviceToHost, st));
+    if (enbw_host) DFK_CUDA(cudaMemcpyAsync(enbw_host, enbw_dev, sizeof(double) * nf, cudaMemcpyDeviceToHost, st));
+    DFK_CUDA(cudaStreamSynchronize(st));
+    copy_plan_out(dp, f_host, navs_host);
     return DFK_OK;
 }
 

@@ -1,7 +1,7 @@
 // Post-fit step of the readout (SURVEY 8f-4): block means of a raw-rate series at the fit rate
 // (dsp.py:3-56 vectorized_downsample) and the log-frequency spectral density of a fitted series
 // (core.py:590-609 / data.py:239-244 -> spectools.lpsd, restated from Troebs & Heinzel 2006 and the LTPDA scheduler;
-// see oracle/post_oracle.py for the sources).
+// see oracle/post_oracle.py for the sources), and the cross-spectral density of two sets of series on the same plan.
 #pragma once
 #include "dfk_common.cuh"
 
@@ -130,11 +130,11 @@ DFK_D double lpsd_window(const LpsdParams& P, long long n, double half_len) {
 DFK_D long long lpsd_start(double shift, long long k) { return static_cast<long long>(floor(static_cast<double>(k) * shift + 0.5)); }
 
 // One group: segments k0 .. k0+ns-1 of frequency row F, by `width` lanes (lane = this thread's index among them).
-// Returns, on every lane, this lane's partial of sum_s |A_s|^2 -- only after the caller's reduction; here the
-// per-segment complex partial sums are reduced by the caller-supplied functor `reduce` (warp or CTA wide).
+// On return re[s], im[s] (s < ns) hold, on every lane, the segment's projection A_s = sum_n w_n v_n e^{+i p n}
+// (v detrended), its lane partials reduced by the caller-supplied functor `reduce` (warp or CTA wide).
 template <class Reduce>
-DFK_D double lpsd_group(const LpsdParams& P, const LpsdFreq& F, const double* __restrict__ xc, long long k0, int ns, int lane,
-                        int width, Reduce reduce) {
+DFK_D void lpsd_group_dft(const LpsdParams& P, const LpsdFreq& F, const double* __restrict__ xc, long long k0, int ns,
+                          int lane, int width, Reduce reduce, double (&re)[kLpsdGroup], double (&im)[kLpsdGroup]) {
     const long long L = F.L;
     long long start[kLpsdGroup];
 #pragma unroll
@@ -170,7 +170,6 @@ DFK_D double lpsd_group(const LpsdParams& P, const LpsdFreq& F, const double* __
             }
         }
     }
-    double re[kLpsdGroup], im[kLpsdGroup];
 #pragma unroll
     for (int s = 0; s < kLpsdGroup; ++s) re[s] = im[s] = 0.0;
     const double half_len = 0.5 * Ld;
@@ -191,21 +190,22 @@ DFK_D double lpsd_group(const LpsdParams& P, const LpsdFreq& F, const double* __
             }
         }
     }
-    double total = 0.0;
+    // the reduced values, in the order the lanes reach them: re[0], im[0], re[1], ...
 #pragma unroll
     for (int s = 0; s < kLpsdGroup; ++s) {
         if (s < ns) {
             const double r = reduce(re[s]), i = reduce(im[s]);
-            total += r * r + i * i;
+            re[s] = r;
+            im[s] = i;
         }
     }
-    return total;
 }
 
-__global__ void __launch_bounds__(kLpsdThreads) lpsd_segment_kernel(const LpsdParams P) {
-    __shared__ double red[kLpsdThreads / 32];
-    const long long tile = blockIdx.x;
-    const long long c = blockIdx.y;
+// The group(s) of segments that tile `tile` of one series covers (a CTA per group when L >= kLpsdCtaMin, else a warp
+// per group): emit(F, g, ns, re, im, lead) receives, on every lane of the group, frequency row F, the group's index g
+// within the row, its segment count and the reduced projections; `lead` is true on one lane per group.
+template <class Emit>
+DFK_D void lpsd_tile(const LpsdParams& P, const double* __restrict__ xc, long long tile, double* red, Emit emit) {
     // frequency row of this tile: last row with tile0 <= tile
     int lo = 0, hi = P.nf - 1;
     while (lo < hi) {
@@ -213,10 +213,9 @@ __global__ void __launch_bounds__(kLpsdThreads) lpsd_segment_kernel(const LpsdPa
         if (P.plan[mid].tile0 <= tile) lo = mid; else hi = mid - 1;
     }
     const LpsdFreq F = P.plan[lo];
-    const double* xc = P.x + c * P.ld_c;
     const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
     const long long t = tile - F.tile0;
-    double* out = P.group_sum + c * P.ngroups + F.group0;
+    double re[kLpsdGroup], im[kLpsdGroup];
     if (F.L >= kLpsdCtaMin) {
         // one group per tile, all lanes of the CTA
         const long long k0 = t * kLpsdGroup;
@@ -231,8 +230,8 @@ __global__ void __launch_bounds__(kLpsdThreads) lpsd_segment_kernel(const LpsdPa
             for (int w = 0; w < kLpsdThreads / 32; ++w) s += red[w];
             return s;
         };
-        const double total = lpsd_group(P, F, xc, k0, ns, threadIdx.x, kLpsdThreads, reduce);
-        if (threadIdx.x == 0) out[t] = total;
+        lpsd_group_dft(P, F, xc, k0, ns, threadIdx.x, kLpsdThreads, reduce, re, im);
+        emit(F, t, ns, re, im, threadIdx.x == 0);
     } else {
         // a group per warp
         const long long g = t * (kLpsdThreads / 32) + warp;
@@ -240,8 +239,51 @@ __global__ void __launch_bounds__(kLpsdThreads) lpsd_segment_kernel(const LpsdPa
         if (k0 >= F.K) return;
         const int ns = static_cast<int>(min(static_cast<long long>(kLpsdGroup), F.K - k0));
         auto reduce = [&](double v) { return warp_sum(v); };
-        const double total = lpsd_group(P, F, xc, k0, ns, lane, 32, reduce);
-        if (lane == 0) out[g] = total;
+        lpsd_group_dft(P, F, xc, k0, ns, lane, 32, reduce, re, im);
+        emit(F, g, ns, re, im, lane == 0);
+    }
+}
+
+__global__ void __launch_bounds__(kLpsdThreads) lpsd_segment_kernel(const LpsdParams P) {
+    __shared__ double red[kLpsdThreads / 32];
+    const long long c = blockIdx.y;
+    double* out = P.group_sum + c * P.ngroups;
+    lpsd_tile(P, P.x + c * P.ld_c, blockIdx.x, red,
+              [&](const LpsdFreq& F, long long g, int ns, const double (&re)[kLpsdGroup], const double (&im)[kLpsdGroup],
+                  bool lead) {
+                  double total = 0.0;
+#pragma unroll
+                  for (int s = 0; s < kLpsdGroup; ++s)
+                      if (s < ns) total += re[s] * re[s] + im[s] * im[s];
+                  if (lead) out[F.group0 + g] = total;
+              });
+}
+
+// Window sums S1 = sum w_n and S2 = sum w_n^2 of row F by a CTA of kThreads lanes (lane partials in n order, warp
+// sums, then a fixed pairwise tree over the warps); red1, red2 hold kThreads / 32 doubles each.
+template <int kThreads>
+DFK_D void lpsd_window_sums(const LpsdParams& P, const LpsdFreq& F, double* red1, double* red2, double& s1, double& s2) {
+    static_assert(kThreads == 128 || kThreads == 256, "fixed reduction tree for 4 or 8 warps");
+    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+    s1 = s2 = 0.0;
+    const double half_len = 0.5 * static_cast<double>(F.L);
+    for (long long n = threadIdx.x; n < F.L; n += kThreads) {
+        const double w = lpsd_window(P, n, half_len);
+        s1 += w;
+        s2 = fma(w, w, s2);
+    }
+    s1 = warp_sum(s1);
+    s2 = warp_sum(s2);
+    if (lane == 0) {
+        red1[warp] = s1;
+        red2[warp] = s2;
+    }
+    __syncthreads();
+    s1 = (red1[0] + red1[1]) + (red1[2] + red1[3]);
+    s2 = (red2[0] + red2[1]) + (red2[2] + red2[3]);
+    if constexpr (kThreads == 256) {
+        s1 += (red1[4] + red1[5]) + (red1[6] + red1[7]);
+        s2 += (red2[4] + red2[5]) + (red2[6] + red2[7]);
     }
 }
 
@@ -252,22 +294,8 @@ __global__ void __launch_bounds__(128) lpsd_finish_kernel(const LpsdParams P, lo
     const int j = blockIdx.x;
     const LpsdFreq F = P.plan[j];
     const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
-    double s1 = 0.0, s2 = 0.0;
-    const double half_len = 0.5 * static_cast<double>(F.L);
-    for (long long n = threadIdx.x; n < F.L; n += 128) {
-        const double w = lpsd_window(P, n, half_len);
-        s1 += w;
-        s2 = fma(w, w, s2);
-    }
-    s1 = warp_sum(s1);
-    s2 = warp_sum(s2);
-    if (lane == 0) {
-        r1[warp] = s1;
-        r2[warp] = s2;
-    }
-    __syncthreads();
-    s1 = (r1[0] + r1[1]) + (r1[2] + r1[3]);
-    s2 = (r2[0] + r2[1]) + (r2[2] + r2[3]);
+    double s1, s2;
+    lpsd_window_sums<128>(P, F, r1, r2, s1, s2);
     const long long ng = (F.K + kLpsdGroup - 1) / kLpsdGroup;
     for (long long c = 0; c < C; ++c) {
         const double* g = P.group_sum + c * P.ngroups + F.group0;
@@ -281,6 +309,97 @@ __global__ void __launch_bounds__(128) lpsd_finish_kernel(const LpsdParams P, lo
             const double avg = ((r1[0] + r1[1]) + (r1[2] + r1[3])) / static_cast<double>(F.K);
             ps[c * P.nf + j] = 2.0 * avg / (s1 * s1);
             psd[c * P.nf + j] = 2.0 * avg / (fs * s2);
+        }
+    }
+    if (threadIdx.x == 0) enbw[j] = fs * s2 / (s1 * s1);
+}
+
+// ---------------------------------------------------------------------------------------------------------------
+// Cross-spectral density on the LPSD plan (the LTPDA log-frequency CSD).  For frequency row j, segment s of series u
+// has the projection A_{u,s} = sum_n w_n v_n e^{+i p_j n} that lpsd_group_dft forms (v detrended): the complex
+// conjugate of the usual DFT X.  Then
+//   Sxy[a,b,j] = 2 / (fs S2_j) * (1 / K_j) * sum_s A_{x_a,s} conj(A_{y_b,s})
+// is the one-sided CSD in the E[conj(X) Y] convention, and Sxx, Syy are the same sum on one series: lpsd's psd.
+// Stage 1 stores every segment's A in a table [series][group0 * kLpsdGroup + k] (at most kLpsdGroup - 1 unused slots
+// per row); the finish kernel takes a frequency row per CTA and sums each auto and cross term over the K_j segments in
+// a fixed order (lane partials in segment order, warp sums, a fixed tree over the warps), so the result does not
+// depend on scheduling.  Each product is rounded on its own (no contraction), so a series against itself gives a
+// real Sxy bit-equal to its Sxx.
+// ---------------------------------------------------------------------------------------------------------------
+constexpr int kLcsdFinishThreads = 256;
+
+struct LcsdParams {
+    LpsdParams P;        // the plan and the series x (P.x, P.ld_c); P.group_sum is not used
+    const double* y;     // sample i of y series b at y[b * ld_y + i * P.stride]
+    long long ld_y;
+    long long cx, cy;
+    double2* seg;        // [cx + cy][nslots]: x series first, then y
+    long long nslots;    // P.ngroups * kLpsdGroup
+};
+
+__global__ void __launch_bounds__(kLpsdThreads) lcsd_segment_kernel(const LcsdParams Q) {
+    __shared__ double red[kLpsdThreads / 32];
+    const long long u = blockIdx.y;
+    const double* xc = u < Q.cx ? Q.P.x + u * Q.P.ld_c : Q.y + (u - Q.cx) * Q.ld_y;
+    double2* out = Q.seg + u * Q.nslots;
+    lpsd_tile(Q.P, xc, blockIdx.x, red,
+              [&](const LpsdFreq& F, long long g, int ns, const double (&re)[kLpsdGroup], const double (&im)[kLpsdGroup],
+                  bool lead) {
+                  if (!lead) return;
+                  double2* o = out + (F.group0 + g) * kLpsdGroup;
+#pragma unroll
+                  for (int s = 0; s < kLpsdGroup; ++s)
+                      if (s < ns) o[s] = make_double2(re[s], im[s]);
+              });
+}
+
+// Per frequency row: S1, S2, then every auto term (series 0 .. cx+cy-1: psd[u][j]) and every pair (a, b)
+// (sxy[(a * cy + b) * nf + j] as re, im), then ENBW.
+__global__ void __launch_bounds__(kLcsdFinishThreads) lcsd_finish_kernel(const LcsdParams Q, double fs,
+                                                                        double* __restrict__ psd,
+                                                                        double* __restrict__ sxy,
+                                                                        double* __restrict__ enbw) {
+    constexpr int kWarps = kLcsdFinishThreads / 32;
+    __shared__ double r1[kWarps], r2[kWarps];
+    const int j = blockIdx.x;
+    const int nf = Q.P.nf;
+    const LpsdFreq F = Q.P.plan[j];
+    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+    double s1, s2;
+    lpsd_window_sums<kLcsdFinishThreads>(Q.P, F, r1, r2, s1, s2);
+    const long long nauto = Q.cx + Q.cy, nterms = nauto + Q.cx * Q.cy;
+    const double2* row = Q.seg + F.group0 * kLpsdGroup;
+    for (long long term = 0; term < nterms; ++term) {
+        const bool cross = term >= nauto;
+        const long long pair = term - nauto;
+        const long long a = cross ? pair / Q.cy : term, b = cross ? Q.cx + pair % Q.cy : term;
+        const double2* A = row + a * Q.nslots;
+        const double2* B = row + b * Q.nslots;
+        double re = 0.0, im = 0.0;
+        for (long long s = threadIdx.x; s < F.K; s += kLcsdFinishThreads) {
+            const double2 p = A[s], q = B[s];
+            // A conj(B) = (p.x q.x + p.y q.y) + i (p.y q.x - p.x q.y)
+            re = __dadd_rn(re, __dadd_rn(__dmul_rn(p.x, q.x), __dmul_rn(p.y, q.y)));
+            im = __dadd_rn(im, __dsub_rn(__dmul_rn(p.y, q.x), __dmul_rn(p.x, q.y)));
+        }
+        re = warp_sum(re);
+        im = warp_sum(im);
+        __syncthreads();  // the previous term's (or the window sums') reads of r1, r2 are done
+        if (lane == 0) {
+            r1[warp] = re;
+            r2[warp] = im;
+        }
+        __syncthreads();
+        if (threadIdx.x == 0) {
+            re = ((r1[0] + r1[1]) + (r1[2] + r1[3])) + ((r1[4] + r1[5]) + (r1[6] + r1[7]));
+            im = ((r2[0] + r2[1]) + (r2[2] + r2[3])) + ((r2[4] + r2[5]) + (r2[6] + r2[7]));
+            const double K = static_cast<double>(F.K);
+            if (cross) {
+                sxy[2 * (pair * nf + j)] = 2.0 * (re / K) / (fs * s2);
+                sxy[2 * (pair * nf + j) + 1] = 2.0 * (im / K) / (fs * s2);
+            } else {
+                psd[term * nf + j] = 2.0 * (re / K) / (fs * s2);
+            }
         }
     }
     if (threadIdx.x == 0) enbw[j] = fs * s2 / (s1 * s1);

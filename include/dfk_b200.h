@@ -33,7 +33,7 @@
 extern "C" {
 #endif
 
-#define DFK_ABI_VERSION 5
+#define DFK_ABI_VERSION 6
 #define DFK_ROW_STRIDE 8
 #define DFK_COV_STRIDE 8
 #define DFK_MAX_HARMONICS 64
@@ -387,6 +387,23 @@ int dfk_lpsd_plan(int64_t N, double fs, const dfk_lpsd_opts* opts, int32_t cap, 
 int dfk_lpsd_dev(dfk_ctx* ctx, const double* x_dev, int64_t N, int64_t stride, int64_t C, int64_t ld_c, double fs,
                  const dfk_lpsd_opts* opts, int32_t cap, int32_t* nf_out, double* f_host, double* ps_host,
                  double* psd_host, double* enbw_host, int64_t* navs_host);
+/* Log-frequency cross-spectral density of Cx device-resident series x against Cy series y on the plan of
+ * dfk_lpsd_plan with the same options (the LTPDA log-frequency CSD, Troebs & Heinzel 2006): same frequencies, segments,
+ * detrending and window as dfk_lpsd_dev.  Sample i of series a of x is x_dev[a * ldx + i * stride], likewise for y;
+ * stride = DFK_ROW_STRIDE reads a column of a row table in place.  Every series has N samples; Cx, Cy >= 1 and
+ * Cx + Cy <= 65535.
+ * For frequency row j (K_j segments, window w, S2_j = sum w^2) and segment s of series u let
+ * A_{u,s} = sum_n w_n v_n e^{+i p_j n}, v the detrended segment: the complex conjugate of the usual DFT X.  Then
+ *     Sxy[a,b,j] = 2 / (fs S2_j) * (1 / K_j) * sum_s A_{x_a,s} conj(A_{y_b,s})
+ * is the one-sided CSD in scipy's convention, E[conj(X) Y]; Sxx, Syy are the same sum on one series, i.e. the psd of
+ * dfk_lpsd_dev (equal up to the order of the segment sum).  If y(t) = x(t - tau), arg Sxy = -2 pi f tau.
+ * Host outputs: f_host[nf], sxx_host [Cx x nf], syy_host [Cy x nf], sxy_host [Cx x Cy x nf x 2] (re, im interleaved),
+ * enbw_host[nf], navs_host[nf] (K_j); any may be NULL.  Coherence |Sxy|^2 / (Sxx Syy) is identically 1 where K_j = 1.
+ * Fails if the plan needs more than cap frequencies.  Two kernel launches; synchronises like dfk_lpsd_dev. */
+int dfk_lcsd_dev(dfk_ctx* ctx, const double* x_dev, int64_t Cx, int64_t ldx, const double* y_dev, int64_t Cy, int64_t ldy,
+                 int64_t N, int64_t stride, double fs, const dfk_lpsd_opts* opts, int32_t cap, int32_t* nf_out,
+                 double* f_host, double* sxx_host, double* syy_host, double* sxy_host, double* enbw_host,
+                 int64_t* navs_host);
 
 /* ---- introspection ------------------------------------------------------------------------ */
 /* Counters accumulated by the LM kernels since the last reset (device -> host copy, syncs). */
