@@ -129,6 +129,9 @@ SYMBOLS = {
                                     ctypes.POINTER(_i32), _vp, _vp, _vp, _vp, _vp]),
     "dfk_lcsd_dev": (ctypes.c_int, [_vp, _vp, _i64, _i64, _vp, _i64, _i64, _i64, _i64, _d, ctypes.POINTER(LpsdOpts),
                                     _i32, ctypes.POINTER(_i32), _vp, _vp, _vp, _vp, _vp, _vp]),
+    "dfk_lcsd_cond_dev": (ctypes.c_int, [_vp, _vp, _i64, _i64, _vp, _i64, _i64, _i64, _i64, _d,
+                                         ctypes.POINTER(LpsdOpts), _i32, ctypes.POINTER(_i32), _vp, _vp, _vp, _vp, _vp,
+                                         _vp, _vp, _vp, _vp]),
     "dfk_lm_counters_read": (ctypes.c_int, [_vp, ctypes.POINTER(LmCounters), _i32]),
     "dfk_profile_enable": (ctypes.c_int, [_vp, _i32]),
     "dfk_profile_read": (ctypes.c_int, [_vp, c_double_p, ctypes.POINTER(_i64), _i32]),
@@ -517,6 +520,27 @@ class Context:
                                                f.ctypes.data, sxx.ctypes.data, syy.ctypes.data, sxy.ctypes.data,
                                                enbw.ctypes.data, navs.ctypes.data))
         return {"f": f, "Sxx": sxx, "Syy": syy, "Sxy": sxy, "enbw": enbw, "navs": navs}
+
+    def lcsd_cond_dev(self, x_ptr, Cx, ldx, y_ptr, Cy, ldy, N, stride, fs, opts=None) -> dict:
+        """Conditioned spectra of Cy device-resident targets y given Cx witnesses x on the LPSD plan; returns host
+        arrays f[nf], Sxx[Cx, Cx, nf], Syy[Cy, nf], Sxy[Cx, Cy, nf], H[Cx, Cy, nf] (complex128), Sres[Cy, nf],
+        mcoh[Cy, nf], enbw[nf], navs[nf]."""
+        opts = opts if opts is not None else default_lpsd_opts()
+        nf = _i32()
+        _check(self.lib, self.lib.dfk_lpsd_plan(int(N), float(fs), ctypes.byref(opts), 0, ctypes.byref(nf), None, None,
+                                                None, None, None))
+        n, cx, cy = int(nf.value), int(Cx), int(Cy)
+        f, enbw, navs = np.empty(n), np.empty(n), np.empty(n, dtype=np.int64)
+        sxx = np.empty((cx, cx, n), dtype=np.complex128)
+        syy, sres, mcoh = np.empty((cy, n)), np.empty((cy, n)), np.empty((cy, n))
+        sxy, h = np.empty((cx, cy, n), dtype=np.complex128), np.empty((cx, cy, n), dtype=np.complex128)
+        _check(self.lib, self.lib.dfk_lcsd_cond_dev(self._h, x_ptr, cx, int(ldx), y_ptr, cy, int(ldy), int(N),
+                                                    int(stride), float(fs), ctypes.byref(opts), n, ctypes.byref(nf),
+                                                    f.ctypes.data, sxx.ctypes.data, syy.ctypes.data, sxy.ctypes.data,
+                                                    h.ctypes.data, sres.ctypes.data, mcoh.ctypes.data,
+                                                    enbw.ctypes.data, navs.ctypes.data))
+        return {"f": f, "enbw": enbw, "navs": navs, "Sxx": sxx, "Syy": syy, "Sxy": sxy, "H": h, "Sres": sres,
+                "mcoh": mcoh}
 
     def set_host_slab_bytes(self, nbytes=0):
         """Slab size of the host-pointer entries (0: defaults); small values make a short record stream."""

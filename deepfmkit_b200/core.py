@@ -7,7 +7,8 @@ stay with the reference (``fit`` hands those method names to the reference's cla
 INTEGRATION.md shows the opposite direction too: the reference's own façade pointed at these fitters).  Call
 signatures, default labels, the ``tau`` column, the error behaviour (log + ``None``) and the fields of the returned
 objects are those of the reference.  ``DeepFitObject.calc_csd`` is this package's addition: the cross-spectral estimate
-(CSD, coherence, transfer function) of one fit against another on the LPSD frequency plan.
+(CSD, coherence, transfer function) of one fit against another on the LPSD frequency plan; ``calc_conditioned`` is its
+multi-witness counterpart (joint transfer functions, residual PSD, multiple coherence).
 """
 from __future__ import annotations
 
@@ -189,6 +190,33 @@ class DeepFitObject:
             raise ValueError(f"series lengths differ: {len(x)} and {len(y)}")
         return lcsd(x, y, self.fs, self.olap, self.bmin, self.Lmin, self.Jdes, self.Kdes, self.order, self.win,
                     self.psll)
+
+    def calc_conditioned(self, witness_fits, column="phi"):
+        """Conditioned spectra of this fit's ``column`` given the same column of every fit in ``witness_fits`` (one fit
+        or a sequence of up to 64), on the device with this object's spectral settings: the ``lcsd_conditioned`` dict
+        (f, enbw, navs, Sxx, Syy, Sxy, H, Sres, mcoh) with this fit as the one target.  Stores nothing.  Every fit must
+        have this fit's rate and number of buffers."""
+        from .spectra import lcsd_conditioned
+        if isinstance(witness_fits, DeepFitObject):
+            witness_fits = [witness_fits]
+        witness_fits = list(witness_fits)
+        if not witness_fits:
+            raise ValueError("need at least one witness fit")
+        y = getattr(self, column)
+        if y is None:
+            raise ValueError(f"this fit has no '{column}' series")
+        xs = []
+        for w in witness_fits:
+            if w.fs != self.fs:
+                raise ValueError(f"fit rates differ: {self.fs} and {w.fs}")
+            x = getattr(w, column)
+            if x is None:
+                raise ValueError(f"every witness fit needs a '{column}' series")
+            if len(x) != len(y):
+                raise ValueError(f"series lengths differ: {len(y)} and {len(x)}")
+            xs.append(np.asarray(x, dtype=np.float64))
+        return lcsd_conditioned(np.stack(xs), y, self.fs, self.olap, self.bmin, self.Lmin, self.Jdes, self.Kdes,
+                                self.order, self.win, self.psll)
 
 
 class DeepFitFramework:

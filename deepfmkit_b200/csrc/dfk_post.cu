@@ -296,6 +296,116 @@ int dfk_lcsd_dev(dfk_ctx* ctx, const double* x_dev, int64_t Cx, int64_t ldx, con
     return DFK_OK;
 }
 
+int dfk_lcsd_cond_dev(dfk_ctx* ctx, const double* x_dev, int64_t Cx, int64_t ldx, const double* y_dev, int64_t Cy,
+                      int64_t ldy, int64_t N, int64_t stride, double fs, const dfk_lpsd_opts* opts, int32_t cap,
+                      int32_t* nf_out, double* f_host, double* sxx_host, double* syy_host, double* sxy_host,
+                      double* h_host, double* sres_host, double* mcoh_host, double* enbw_host, int64_t* navs_host) {
+    DFK_ENTER(ctx);
+    dfk_lpsd_opts d;
+    if (!opts) {
+        dfk_default_lpsd_opts(&d);
+        opts = &d;
+    }
+    if (!x_dev || !y_dev || !nf_out) return fail(DFK_ERR_ARG, "null pointer");
+    if (Cx < 1 || Cx > dfk::kCondMaxWitnesses || Cy < 1 || stride < 1)
+        return fail(DFK_ERR_ARG, "bad geometry: Cx=%lld (1..%d) Cy=%lld stride=%lld", (long long)Cx,
+                    dfk::kCondMaxWitnesses, (long long)Cy, (long long)stride);
+    if (Cx + Cy > 65535) return fail(DFK_ERR_ARG, "conditioned spectra take at most 65535 series in all (Cx + Cy)");
+    DevicePlan dp;
+    int rc = make_device_plan(N, fs, *opts, dp);
+    if (rc) return rc;
+    const int nf = static_cast<int>(dp.rows.size());
+    *nf_out = nf;
+    if (nf > cap) return fail(DFK_ERR_ARG, "plan has %d frequencies, outputs hold %d (call dfk_lpsd_plan first)", nf, cap);
+    if (nf == 0) return DFK_OK;
+    const long long ns = Cx + Cy, npair = Cx * Cy;
+    const long long row_tiles = (Cx + dfk::kGramRows - 1) / dfk::kGramRows;
+    const long long col_tiles = (ns + dfk::kGramCols - 1) / dfk::kGramCols;
+    const long long gram_tiles = row_tiles * col_tiles + (Cy + dfk::kGramCols - 1) / dfk::kGramCols;
+    if (dp.tiles > 0x7fffffffll || gram_tiles > 0x7fffffffll)
+        return fail(DFK_ERR_ARG, "conditioned-spectra problem too large for one launch");
+    const long long nslots = dp.groups * dfk::kLpsdGroup;
+    DevBuf& plan_dev = ctx->post[0];
+    DevBuf& seg_dev = ctx->post[1];
+    DevBuf& out_dev = ctx->post[2];
+    // outputs: Sxx (re, im), Syy, Sxy (re, im), H (re, im), Sres, mcoh, ENBW
+    const size_t out_doubles = static_cast<size_t>(2 * Cx * Cx + 3 * Cy + 4 * npair + 1) * static_cast<size_t>(nf);
+    rc = ensure(ctx, plan_dev, sizeof(dfk::LpsdFreq) * nf);
+    if (!rc) rc = ensure(ctx, seg_dev, sizeof(double2) * static_cast<size_t>(nslots) * static_cast<size_t>(ns));
+    if (!rc) rc = ensure(ctx, out_dev, sizeof(double) * out_doubles);
+    if (rc) return rc;
+    cudaStream_t st = ctx->stream();
+    DFK_CUDA(cudaMemcpyAsync(plan_dev.ptr, dp.freq.data(), sizeof(dfk::LpsdFreq) * nf, cudaMemcpyHostToDevice, st));
+    dfk::LcsdParams Q;
+    Q.P = lpsd_params(dp, plan_dev.ptr, N, stride, *opts);
+    Q.P.x = x_dev;
+    Q.P.ld_c = ldx;
+    Q.y = y_dev;
+    Q.ld_y = ldy;
+    Q.cx = Cx;
+    Q.cy = Cy;
+    Q.seg = static_cast<double2*>(seg_dev.ptr);
+    Q.nslots = nslots;
+    double* sxx_dev = static_cast<double*>(out_dev.ptr);  // [Cx][Cx][nf][2]
+    double* syy_dev = sxx_dev + 2 * Cx * Cx * nf;          // [Cy][nf]
+    double* sxy_dev = syy_dev + Cy * nf;                   // [Cx][Cy][nf][2]
+    double* h_dev = sxy_dev + 2 * npair * nf;              // [Cx][Cy][nf][2]
+    double* sres_dev = h_dev + 2 * npair * nf;             // [Cy][nf]
+    double* mcoh_dev = sres_dev + Cy * nf;                 // [Cy][nf]
+    double* enbw_dev = mcoh_dev + Cy * nf;
+    dfk::GramParams G;
+    G.seg = Q.seg;
+    G.nslots = nslots;
+    G.plan = Q.P.plan;
+    G.nf = nf;
+    G.cx = Cx;
+    G.cy = Cy;
+    G.row_tiles = row_tiles;
+    G.col_tiles = col_tiles;
+    G.sxx = sxx_dev;
+    G.syy = syy_dev;
+    G.sxy = sxy_dev;
+    dfk::CondParams C;
+    C.P = Q.P;
+    C.cx = Cx;
+    C.cy = Cy;
+    C.fs = fs;
+    C.sxx = sxx_dev;
+    C.syy = syy_dev;
+    C.sxy = sxy_dev;
+    C.h = h_dev;
+    C.sres = sres_dev;
+    C.mcoh = mcoh_dev;
+    C.enbw = enbw_dev;
+    const size_t cond_smem = sizeof(double2) * static_cast<size_t>(Cx) * static_cast<size_t>(Cx + 1);
+    DFK_CUDA(cudaFuncSetAttribute(dfk::lcsd_cond_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                                  static_cast<int>(cond_smem)));
+    const dim3 seg_grid(static_cast<unsigned>(dp.tiles), static_cast<unsigned>(ns));
+    dfk::lcsd_segment_kernel<<<seg_grid, dfk::kLpsdThreads, 0, st>>>(Q);
+    DFK_CUDA(cudaGetLastError());
+    const dim3 gram_grid(static_cast<unsigned>(gram_tiles), static_cast<unsigned>(std::min(nf, 65535)));
+    dfk::lcsd_gram_kernel<<<gram_grid, dfk::kGramThreads, 0, st>>>(G);
+    DFK_CUDA(cudaGetLastError());
+    dfk::lcsd_cond_kernel<<<nf, dfk::kCondThreads, cond_smem, st>>>(C);
+    DFK_CUDA(cudaGetLastError());
+    ctx->launches += 3;
+    auto out = [&](double* host, const double* dev, long long n) -> int {
+        if (host) DFK_CUDA(cudaMemcpyAsync(host, dev, sizeof(double) * n, cudaMemcpyDeviceToHost, st));
+        return DFK_OK;
+    };
+    rc = out(sxx_host, sxx_dev, 2 * Cx * Cx * nf);
+    if (!rc) rc = out(syy_host, syy_dev, Cy * nf);
+    if (!rc) rc = out(sxy_host, sxy_dev, 2 * npair * nf);
+    if (!rc) rc = out(h_host, h_dev, 2 * npair * nf);
+    if (!rc) rc = out(sres_host, sres_dev, Cy * nf);
+    if (!rc) rc = out(mcoh_host, mcoh_dev, Cy * nf);
+    if (!rc) rc = out(enbw_host, enbw_dev, nf);
+    if (rc) return rc;
+    DFK_CUDA(cudaStreamSynchronize(st));
+    copy_plan_out(dp, f_host, navs_host);
+    return DFK_OK;
+}
+
 int dfk_downsample_dev(dfk_ctx* ctx, const double* x_dev, int64_t n, int64_t R, double* out_dev) {
     DFK_ENTER(ctx);
     if (R <= 0 || n < 0) return fail(DFK_ERR_ARG, "bad geometry: n=%lld R=%lld", (long long)n, (long long)R);

@@ -405,4 +405,332 @@ __global__ void __launch_bounds__(kLcsdFinishThreads) lcsd_finish_kernel(const L
     if (threadIdx.x == 0) enbw[j] = fs * s2 / (s1 * s1);
 }
 
+// ---------------------------------------------------------------------------------------------------------------
+// Conditioned spectra on the LPSD plan (multiple-input / single-output analysis, Bendat & Piersol, Random Data, ch. 7).
+// Witnesses x_1..x_Cx, targets y_1..y_Cy; for frequency row j with c_j = 2 / (fs S2_j K_j) and the segment table of
+// lcsd_segment_kernel (x series first, then y):
+//   Sxx[a,b,j] = c_j sum_s A_{x_a,s} conj(A_{x_b,s})   the Cx x Cx Hermitian witness matrix (diagonal: lpsd's psd)
+//   Sxy[a,t,j] = c_j sum_s A_{x_a,s} conj(A_{y_t,s})   lcsd's convention, E[conj(X) Y]
+//   Syy[t,j]   = lpsd's psd of target t
+//   H[:,t,j]   = Sxx^-1 Sxy[:,t]                      joint (MISO) transfer functions; for Cx = 1, lcsd's tf
+//   Sres[t,j]  = Syy - Sxy[:,t]^H Sxx^-1 Sxy[:,t]     conditioned PSD: y_t after the best linear subtraction of all x
+//   mcoh[t,j]  = 1 - Sres / Syy                       multiple coherence (NaN where Syy = 0)
+// H, Sres and mcoh are NaN on a row where K_j < Cx (the estimated Sxx has rank <= K_j) or where the Cholesky
+// factorisation of Sxx meets a pivot that is not above kCondPivotTol times its diagonal entry (a witness that the
+// earlier ones explain to within that fraction: a duplicated or linearly dependent witness).
+//
+// lcsd_gram_kernel forms the raw sums (before c_j) as a complex product of the segment table per row: output pairs
+// (witness a, series b) in tiles of kGramRows x kGramCols, over the Sxx upper triangle and all of Sxy, plus tiles of
+// kGramCols target diagonals (Syy); the Cy x Cy target block is never formed.  A CTA stages kGramChunk segments of its
+// rows and columns in shared memory; warp w sums the segments w, w + 8, ... of each chunk in a register tile of 2 x 4
+// complex accumulators, and the eight warp partials of every output are combined in a fixed tree, so each output has a
+// fixed order of summation.  The products may be contracted (FMA).
+// lcsd_cond_kernel then takes a frequency row per CTA: it scales the sums, completes Sxx by conjugation, factors it
+// (complex Cholesky in shared memory) and solves for every target, a warp per target.
+// ---------------------------------------------------------------------------------------------------------------
+constexpr int kGramThreads = 256;
+constexpr int kGramRows = 8;        // witnesses per tile
+constexpr int kGramCols = 32;       // series per tile
+constexpr int kGramChunk = 64;      // segments staged per step
+constexpr int kCondThreads = 256;
+constexpr int kCondMaxWitnesses = 64;
+constexpr double kCondPivotTol = 1e-10;
+
+struct GramParams {
+    const double2* seg;        // lcsd_segment_kernel's table [cx + cy][nslots]
+    long long nslots;
+    const LpsdFreq* plan;
+    int nf;
+    long long cx, cy;
+    long long row_tiles, col_tiles;  // block tiles: row_tiles x col_tiles, then ceil(cy / kGramCols) diagonal tiles
+    double* sxx;               // [cx][cx][nf] (re, im): upper triangle written here
+    double* syy;               // [cy][nf]
+    double* sxy;               // [cx][cy][nf] (re, im)
+};
+
+__global__ void __launch_bounds__(kGramThreads, 3) lcsd_gram_kernel(const GramParams G) {
+    constexpr int kWarps = kGramThreads / 32;
+    // staging (rows [k][kGramRows + 1], columns [k][kGramCols + 1]: padded so neither the stores nor the reads of a
+    // warp meet bank conflicts) and, after the segment loop, the warp partials [kWarps][kGramRows * kGramCols]
+    constexpr int kRowBytes = kGramChunk * (kGramRows + 1) * 16, kColBytes = kGramChunk * (kGramCols + 1) * 16;
+    constexpr int kRedBytes = kWarps * kGramRows * kGramCols * 16;
+    constexpr int kSmem = kRowBytes + kColBytes > kRedBytes ? kRowBytes + kColBytes : kRedBytes;
+    __shared__ __align__(16) unsigned char smem[kSmem];
+    double2* srow = reinterpret_cast<double2*>(smem);
+    double2* scol = reinterpret_cast<double2*>(smem + kRowBytes);
+    double2* red = reinterpret_cast<double2*>(smem);
+
+    const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
+    const long long tile = blockIdx.x;
+    const long long nblock = G.row_tiles * G.col_tiles;
+    const bool diag = tile >= nblock;
+    long long a0 = 0, b0;
+    if (diag) {
+        b0 = G.cx + (tile - nblock) * kGramCols;  // target diagonals b0 .. b0 + 31
+    } else {
+        a0 = (tile / G.col_tiles) * kGramRows;
+        b0 = (tile % G.col_tiles) * kGramCols;
+        if (b0 + kGramCols <= a0) return;  // wholly below the diagonal of Sxx
+    }
+    const long long ns = G.cx + G.cy;
+    const int ri = lane >> 3, ci = lane & 7;  // block tiles: rows 2 ri, 2 ri + 1; columns ci + 8 m
+    for (int j = blockIdx.y; j < G.nf; j += gridDim.y) {
+        const LpsdFreq F = G.plan[j];
+        const double2* base = G.seg + F.group0 * kLpsdGroup;
+        double2 acc[2][4];
+#pragma unroll
+        for (int r = 0; r < 2; ++r)
+#pragma unroll
+            for (int m = 0; m < 4; ++m) acc[r][m] = make_double2(0.0, 0.0);
+        for (long long k0 = 0; k0 < F.K; k0 += kGramChunk) {
+            __syncthreads();  // the previous chunk's (or row's) reads of the staging area are done
+            for (int i = tid; i < kGramCols * kGramChunk; i += kGramThreads) {
+                const int c = i / kGramChunk, k = i % kGramChunk;
+                const long long b = b0 + c;
+                scol[k * (kGramCols + 1) + c] =
+                    (b < ns && k0 + k < F.K) ? base[b * G.nslots + k0 + k] : make_double2(0.0, 0.0);
+            }
+            if (!diag) {
+                for (int i = tid; i < kGramRows * kGramChunk; i += kGramThreads) {
+                    const int r = i / kGramChunk, k = i % kGramChunk;
+                    const long long a = a0 + r;
+                    srow[k * (kGramRows + 1) + r] =
+                        (a < G.cx && k0 + k < F.K) ? base[a * G.nslots + k0 + k] : make_double2(0.0, 0.0);
+                }
+            }
+            __syncthreads();
+            if (diag) {
+#pragma unroll 4
+                for (int k = warp; k < kGramChunk; k += kWarps) {
+                    const double2 q = scol[k * (kGramCols + 1) + lane];
+                    acc[0][0].x = fma(q.x, q.x, acc[0][0].x);
+                    acc[0][0].x = fma(q.y, q.y, acc[0][0].x);
+                }
+            } else {
+#pragma unroll 1
+                for (int k = warp; k < kGramChunk; k += kWarps) {
+                    double2 p[2], q[4];
+#pragma unroll
+                    for (int r = 0; r < 2; ++r) p[r] = srow[k * (kGramRows + 1) + 2 * ri + r];
+#pragma unroll
+                    for (int m = 0; m < 4; ++m) q[m] = scol[k * (kGramCols + 1) + ci + 8 * m];
+                    // A conj(B) = (p.x q.x + p.y q.y) + i (p.y q.x - p.x q.y)
+#pragma unroll
+                    for (int r = 0; r < 2; ++r)
+#pragma unroll
+                        for (int m = 0; m < 4; ++m) {
+                            acc[r][m].x = fma(p[r].x, q[m].x, acc[r][m].x);
+                            acc[r][m].x = fma(p[r].y, q[m].y, acc[r][m].x);
+                            acc[r][m].y = fma(p[r].y, q[m].x, acc[r][m].y);
+                            acc[r][m].y = fma(-p[r].x, q[m].y, acc[r][m].y);
+                        }
+                }
+            }
+        }
+        __syncthreads();  // staging reads done: the area now holds the warp partials
+        if (diag) {
+            red[warp * kGramCols + lane] = acc[0][0];
+        } else {
+#pragma unroll
+            for (int r = 0; r < 2; ++r)
+#pragma unroll
+                for (int m = 0; m < 4; ++m) red[warp * (kGramRows * kGramCols) + (2 * ri + r) * kGramCols + ci + 8 * m] = acc[r][m];
+        }
+        __syncthreads();
+        const int nout = diag ? kGramCols : kGramRows * kGramCols;
+        if (tid < nout) {
+            const int stride = diag ? kGramCols : kGramRows * kGramCols;
+            double2 w[kWarps];
+#pragma unroll
+            for (int v = 0; v < kWarps; ++v) w[v] = red[v * stride + tid];
+            const double re = ((w[0].x + w[1].x) + (w[2].x + w[3].x)) + ((w[4].x + w[5].x) + (w[6].x + w[7].x));
+            const double im = ((w[0].y + w[1].y) + (w[2].y + w[3].y)) + ((w[4].y + w[5].y) + (w[6].y + w[7].y));
+            if (diag) {
+                const long long b = b0 + tid;
+                if (b < ns) G.syy[(b - G.cx) * G.nf + j] = re;
+            } else {
+                const long long a = a0 + tid / kGramCols, b = b0 + tid % kGramCols;
+                if (a < G.cx && b < ns) {
+                    if (b >= G.cx) {
+                        double* o = G.sxy + 2 * ((a * G.cy + (b - G.cx)) * G.nf + j);
+                        o[0] = re;
+                        o[1] = im;
+                    } else if (b >= a) {
+                        double* o = G.sxx + 2 * ((a * G.cx + b) * G.nf + j);
+                        o[0] = re;
+                        o[1] = im;
+                    }
+                }
+            }
+        }
+    }
+}
+
+struct CondParams {
+    LpsdParams P;              // the plan and window (for S2_j); series pointers unused
+    long long cx, cy;
+    double fs;
+    double* sxx;               // [cx][cx][nf] (re, im): upper triangle in raw sums on entry, the full matrix on exit
+    double* syy;               // [cy][nf]: raw sums on entry, scaled on exit
+    double* sxy;               // [cx][cy][nf] (re, im): likewise
+    double* h;                 // [cx][cy][nf] (re, im)
+    double* sres;              // [cy][nf]
+    double* mcoh;              // [cy][nf]
+    double* enbw;              // [nf]
+};
+
+DFK_D double2 cmul(double2 a, double2 b) { return make_double2(a.x * b.x - a.y * b.y, a.x * b.y + a.y * b.x); }
+DFK_D double2 cmul_conj(double2 a, double2 b) { return make_double2(a.x * b.x + a.y * b.y, a.y * b.x - a.x * b.y); }  // a conj(b)
+
+// Per frequency row: window sums, scaling of every sum lcsd's way (2 (sum / K) / (fs S2)), Sxx completed by
+// conjugation; then the Cholesky factor L of Sxx (lower triangle of the shared matrix, leading dimension cx + 1) and,
+// for each target, L z = Sxy[:,t], L^H H = z, Sres = Syy - |z|^2.  Dynamic shared memory: cx (cx + 1) double2.
+__global__ void __launch_bounds__(kCondThreads) lcsd_cond_kernel(const CondParams C) {
+    constexpr int kWarps = kCondThreads / 32;
+    extern __shared__ double2 M[];
+    __shared__ double r1[kWarps], r2[kWarps];
+    __shared__ double diag0[kCondMaxWitnesses];
+    __shared__ int singular;
+    const int j = blockIdx.x;
+    const int nf = C.P.nf;
+    const LpsdFreq F = C.P.plan[j];
+    const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
+    const int cx = static_cast<int>(C.cx), ld = cx + 1;
+    const long long cy = C.cy;
+    double s1, s2;
+    lpsd_window_sums<kCondThreads>(C.P, F, r1, r2, s1, s2);
+    const double K = static_cast<double>(F.K), den = C.fs * s2;
+    for (int i = tid; i < cx * cx; i += kCondThreads) {
+        const int a = i / cx, b = i % cx;
+        if (b < a) continue;
+        double* o = C.sxx + 2 * ((static_cast<long long>(a) * cx + b) * nf + j);
+        const double re = 2.0 * (o[0] / K) / den, im = a == b ? 0.0 : 2.0 * (o[1] / K) / den;
+        o[0] = re;
+        o[1] = im;
+        M[a * ld + b] = make_double2(re, im);
+        if (a != b) {
+            double* t = C.sxx + 2 * ((static_cast<long long>(b) * cx + a) * nf + j);
+            t[0] = re;
+            t[1] = -im;
+            M[b * ld + a] = make_double2(re, -im);
+        } else {
+            diag0[a] = re;
+        }
+    }
+    for (long long i = tid; i < cx * cy; i += kCondThreads) {
+        double* o = C.sxy + 2 * (i * nf + j);
+        o[0] = 2.0 * (o[0] / K) / den;
+        o[1] = 2.0 * (o[1] / K) / den;
+    }
+    for (long long t = tid; t < cy; t += kCondThreads) C.syy[t * nf + j] = 2.0 * (C.syy[t * nf + j] / K) / den;
+    if (tid == 0) {
+        C.enbw[j] = C.fs * s2 / (s1 * s1);
+        singular = F.K < cx;
+    }
+    __syncthreads();
+    // Cholesky, right-looking: column k of L, then the trailing lower triangle
+    for (int k = 0; k < cx && !singular; ++k) {
+        const double d = M[k * ld + k].x;
+        if (!(d > kCondPivotTol * diag0[k])) {  // also NaN and a zero witness
+            __syncthreads();                    // every thread has read d before the flag changes
+            if (tid == 0) singular = 1;
+            __syncthreads();
+            break;
+        }
+        const double l = sqrt(d);
+        for (int i = k + 1 + tid; i < cx; i += kCondThreads) {
+            const double2 v = M[i * ld + k];
+            M[i * ld + k] = make_double2(v.x / l, v.y / l);
+        }
+        __syncthreads();
+        if (tid == 0) M[k * ld + k] = make_double2(l, 0.0);
+        const int m = cx - k - 1;
+        for (int i = tid; i < m * m; i += kCondThreads) {
+            const int r = k + 1 + i / m, c = k + 1 + i % m;
+            if (c > r) continue;
+            const double2 u = cmul_conj(M[r * ld + k], M[c * ld + k]);
+            M[r * ld + c].x -= u.x;
+            M[r * ld + c].y -= u.y;
+        }
+        __syncthreads();
+    }
+    const bool bad = singular;
+    const double nan = __longlong_as_double(0x7ff8000000000000ll);
+    // a warp per target; lane owns rows lane and lane + 32 of the solves
+    for (long long t = warp; t < cy; t += kWarps) {
+        const double syy = C.syy[t * nf + j];
+        double2 z0 = make_double2(0.0, 0.0), z1 = z0;
+        if (lane < cx) {
+            const double* o = C.sxy + 2 * ((lane * cy + t) * nf + j);
+            z0 = make_double2(o[0], o[1]);
+        }
+        if (lane + 32 < cx) {
+            const double* o = C.sxy + 2 * (((lane + 32) * cy + t) * nf + j);
+            z1 = make_double2(o[0], o[1]);
+        }
+        double zz = 0.0;
+        if (!bad) {
+            // forward: L z = b, column by column
+            for (int k = 0; k < cx; ++k) {
+                const double2 own = k < 32 ? z0 : z1;
+                const double l = M[k * ld + k].x;
+                double2 zk;
+                zk.x = __shfl_sync(0xffffffffu, own.x, k & 31) / l;
+                zk.y = __shfl_sync(0xffffffffu, own.y, k & 31) / l;
+                zz += zk.x * zk.x + zk.y * zk.y;
+                if (lane == (k & 31)) {
+                    if (k < 32) z0 = zk; else z1 = zk;
+                }
+                if (lane > k && lane < cx) {
+                    const double2 u = cmul(M[lane * ld + k], zk);
+                    z0.x -= u.x;
+                    z0.y -= u.y;
+                }
+                if (lane + 32 > k && lane + 32 < cx) {
+                    const double2 u = cmul(M[(lane + 32) * ld + k], zk);
+                    z1.x -= u.x;
+                    z1.y -= u.y;
+                }
+            }
+            // backward: L^H h = z, column by column from the last row
+            for (int k = cx - 1; k >= 0; --k) {
+                const double2 own = k < 32 ? z0 : z1;
+                const double l = M[k * ld + k].x;
+                double2 hk;
+                hk.x = __shfl_sync(0xffffffffu, own.x, k & 31) / l;
+                hk.y = __shfl_sync(0xffffffffu, own.y, k & 31) / l;
+                if (lane == (k & 31)) {
+                    if (k < 32) z0 = hk; else z1 = hk;
+                }
+                // row i < k of L^H holds conj(L[k][i]) in column k
+                if (lane < k) {
+                    const double2 u = cmul_conj(hk, M[k * ld + lane]);
+                    z0.x -= u.x;
+                    z0.y -= u.y;
+                }
+                if (lane + 32 < k) {
+                    const double2 u = cmul_conj(hk, M[k * ld + lane + 32]);
+                    z1.x -= u.x;
+                    z1.y -= u.y;
+                }
+            }
+        }
+        if (lane < cx) {
+            double* o = C.h + 2 * ((lane * cy + t) * nf + j);
+            o[0] = bad ? nan : z0.x;
+            o[1] = bad ? nan : z0.y;
+        }
+        if (lane + 32 < cx) {
+            double* o = C.h + 2 * (((lane + 32) * cy + t) * nf + j);
+            o[0] = bad ? nan : z1.x;
+            o[1] = bad ? nan : z1.y;
+        }
+        if (lane == 0) {
+            const double res = bad ? nan : syy - zz;
+            C.sres[t * nf + j] = res;
+            C.mcoh[t * nf + j] = (bad || syy == 0.0) ? nan : 1.0 - res / syy;
+        }
+    }
+}
+
 }  // namespace dfk

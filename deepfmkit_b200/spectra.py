@@ -5,7 +5,9 @@ is dropped; a bad ``R`` or a signal shorter than ``R`` gives an empty array).  `
 reference passes to ``spectools.lpsd.lpsd`` (core.py:590-609, data.py:239-244) and returns, like its ``'legacy'``
 form, a 6-tuple whose first element is the frequency vector and whose third is the one-sided power spectral density
 the reference stores as ``Sxx``.  ``lcsd`` is the cross-spectral counterpart on the same frequency plan: the CSD,
-coherence and transfer function between fitted channels.  All run on the device only.
+coherence and transfer function between fitted channels.  ``lcsd_conditioned`` extends it to several witnesses at
+once: the joint transfer functions, the conditioned (residual) PSD and the multiple coherence of each target given all
+witnesses.  All run on the device only.
 """
 from __future__ import annotations
 
@@ -165,4 +167,69 @@ def lcsd(x, y, fs, olap="default", bmin=1, Lmin=0, Jdes=500, Kdes=100, order=0, 
         out["Syy"] = syy[0]
         for k in ("Sxy", "coh", "tf"):
             out[k] = out[k][..., 0, :]
+    return out
+
+
+MAX_WITNESSES = 64  # the witness matrix of one frequency is factored in one CTA's shared memory
+
+
+def lcsd_conditioned(witnesses, targets, fs, olap="default", bmin=1, Lmin=0, Jdes=500, Kdes=100, order=0,
+                     win=np.kaiser, psll=200, device=0):
+    """Conditioned spectra of ``targets`` given ``witnesses`` on the plan ``lpsd`` uses with the same settings: the
+    multiple-input / single-output analysis (Bendat & Piersol, *Random Data*, ch. 7).  It answers how much of each
+    target the witnesses explain together and what is left after the best linear subtraction of all of them, without
+    counting noise that several witnesses share more than once (as pairwise coherence does).
+
+    ``witnesses`` is ``[N]`` or ``[Cx, N]`` with 1 <= Cx <= 64, ``targets`` is ``[N]`` or ``[Cy, N]``; numpy arrays or
+    CUDA tensors, handled as by ``lcsd``.  With the segment projections A of ``lcsd`` and c_j = 2 / (fs S2_j K_j),
+    sums over the K_j segments of frequency row j, the result is a dict of host arrays:
+
+    - ``f``, ``enbw``, ``navs`` [nf]: as ``lcsd``;
+    - ``Sxx`` [Cx, Cx, nf] complex: c_j sum A_{x_a} conj(A_{x_b}), the Hermitian witness matrix; its diagonal is
+      ``lpsd``'s psd and entry (a, b) is ``lcsd``'s Sxy of witness a against witness b;
+    - ``Syy`` [Cy, nf]: ``lpsd``'s psd of each target;
+    - ``Sxy`` [Cx, Cy, nf] complex: c_j sum A_{x_a} conj(A_{y_t}), ``lcsd``'s convention E[conj(X) Y];
+    - ``H`` [Cx, Cy, nf] complex: Sxx^-1 Sxy[:, t], the joint transfer functions.  If y = sum_a h_a * x_a + n with n
+      independent of the witnesses, H[a, t] estimates the response h_a(f).  For one witness it is ``lcsd``'s ``tf``;
+    - ``Sres`` [Cy, nf]: Syy - Sxy[:, t]^H Sxx^-1 Sxy[:, t], the conditioned PSD: what remains of the target after the
+      best linear subtraction of all witnesses (real, >= 0 up to rounding).  For one witness it is Syy (1 - coh);
+    - ``mcoh`` [Cy, nf]: the multiple coherence 1 - Sres / Syy, NaN where Syy is 0.
+
+    ``H``, ``Sres`` and ``mcoh`` are NaN on a row with fewer segments than witnesses (K_j < Cx: the estimated Sxx then
+    has rank <= K_j), and on a row where the Cholesky factorisation of Sxx meets a pivot not above 1e-10 times its
+    diagonal entry: a duplicated or linearly dependent witness.
+
+    Bias: with no true coherence the expected multiple coherence is about Cx / K (K = ``navs``, fewer effective
+    averages where segments overlap), and it is 1 on rows where K = Cx whatever the data.  Read it against that floor,
+    as ``lcsd``'s coherence is read against 1 / K.
+
+    The witness axis is always kept; a 1-D ``targets`` drops the Cy axis."""
+    import torch
+    nx, ny = (tuple(a.shape) if hasattr(a, "shape") else np.shape(a) for a in (witnesses, targets))
+    if not nx or not ny or nx[-1] != ny[-1]:
+        raise ValueError(f"witnesses and targets must be series of the same number of samples, got shapes {nx} and {ny}")
+    Cx, Cy = (1 if len(nx) == 1 else nx[0]), (1 if len(ny) == 1 else ny[0])
+    if not 1 <= Cx <= MAX_WITNESSES:
+        raise ValueError(f"{Cx} witnesses: between 1 and {MAX_WITNESSES} are supported")
+    if Cy < 1 or Cx + Cy > 65535:
+        raise ValueError(f"{Cy} targets: at least 1, and at most 65535 series in all")
+    tensors = [a for a in (witnesses, targets) if isinstance(a, torch.Tensor) and a.is_cuda]
+    if tensors:
+        device = tensors[0].device.index
+    xt, _ = _device_rows(witnesses, device)
+    yt, y1 = _device_rows(targets, device)
+    if xt.device != yt.device:
+        raise ValueError(f"witnesses and targets are on different devices ({xt.device}, {yt.device})")
+    N = xt.shape[1]
+    opts = lpsd_opts(olap, bmin, Lmin, Jdes, Kdes, order, win, psll)
+    ctx = _lib.get_context(device)
+    with torch.cuda.device(xt.device):
+        ctx.use_torch_stream()
+        try:
+            out = ctx.lcsd_cond_dev(xt.data_ptr(), Cx, N, yt.data_ptr(), Cy, N, N, 1, float(fs), opts)
+        finally:
+            ctx.use_default_stream()
+    if y1:
+        out["Syy"], out["Sres"], out["mcoh"] = out["Syy"][0], out["Sres"][0], out["mcoh"][0]
+        out["Sxy"], out["H"] = out["Sxy"][:, 0], out["H"][:, 0]
     return out

@@ -404,6 +404,27 @@ int dfk_lcsd_dev(dfk_ctx* ctx, const double* x_dev, int64_t Cx, int64_t ldx, con
                  int64_t N, int64_t stride, double fs, const dfk_lpsd_opts* opts, int32_t cap, int32_t* nf_out,
                  double* f_host, double* sxx_host, double* syy_host, double* sxy_host, double* enbw_host,
                  int64_t* navs_host);
+/* Conditioned spectra on the same plan (multiple-input / single-output analysis, Bendat & Piersol, Random Data, ch. 7):
+ * how much of each target y_t the witnesses x_1..x_Cx explain together, and what is left after the best linear
+ * subtraction of all of them.  Series are read as by dfk_lcsd_dev; 1 <= Cx <= 64, Cy >= 1, Cx + Cy <= 65535.
+ * With A_{u,s} and c_j = 2 / (fs S2_j K_j) as above (sums over the K_j segments of row j):
+ *     Sxx[a,b,j] = c_j sum_s A_{x_a,s} conj(A_{x_b,s})   Cx x Cx Hermitian; diagonal = psd, (a, b) = dfk_lcsd_dev's Sxy
+ *     Sxy[a,t,j] = c_j sum_s A_{x_a,s} conj(A_{y_t,s})   as dfk_lcsd_dev
+ *     Syy[t,j]   = psd of target t
+ *     H[:,t,j]   = Sxx^-1 Sxy[:,t]                      joint transfer functions: y = sum_a h_a * x_a + n gives H[a,t] ~ h_a(f)
+ *     Sres[t,j]  = Syy - Sxy[:,t]^H Sxx^-1 Sxy[:,t]     conditioned PSD (real, >= 0 up to rounding)
+ *     mcoh[t,j]  = 1 - Sres / Syy                       multiple coherence, NaN where Syy = 0
+ * For Cx = 1, H is dfk_lcsd_dev's Sxy / Sxx and Sres = Syy (1 - coherence).  H, Sres and mcoh are NaN on a row where
+ * K_j < Cx (Sxx then has rank <= K_j) or where the Cholesky factorisation of Sxx meets a pivot not above 1e-10 times
+ * its diagonal entry (a witness that the earlier ones explain to 1 part in 1e10: duplicated or linearly dependent).
+ * The sums are formed in a fixed order (bit-identical from run to run) but not in dfk_lcsd_dev's order.
+ * Host outputs: f_host[nf], sxx_host [Cx x Cx x nf x 2] (the full matrix, re, im interleaved), syy_host [Cy x nf],
+ * sxy_host and h_host [Cx x Cy x nf x 2], sres_host and mcoh_host [Cy x nf], enbw_host[nf], navs_host[nf]; any may be
+ * NULL.  Fails if the plan needs more than cap frequencies.  Three kernel launches; synchronises like dfk_lpsd_dev. */
+int dfk_lcsd_cond_dev(dfk_ctx* ctx, const double* x_dev, int64_t Cx, int64_t ldx, const double* y_dev, int64_t Cy,
+                      int64_t ldy, int64_t N, int64_t stride, double fs, const dfk_lpsd_opts* opts, int32_t cap,
+                      int32_t* nf_out, double* f_host, double* sxx_host, double* syy_host, double* sxy_host,
+                      double* h_host, double* sres_host, double* mcoh_host, double* enbw_host, int64_t* navs_host);
 
 /* ---- introspection ------------------------------------------------------------------------ */
 /* Counters accumulated by the LM kernels since the last reset (device -> host copy, syncs). */
