@@ -132,6 +132,8 @@ SYMBOLS = {
     "dfk_lcsd_cond_dev": (ctypes.c_int, [_vp, _vp, _i64, _i64, _vp, _i64, _i64, _i64, _i64, _d,
                                          ctypes.POINTER(LpsdOpts), _i32, ctypes.POINTER(_i32), _vp, _vp, _vp, _vp, _vp,
                                          _vp, _vp, _vp, _vp]),
+    "dfk_wiener_dev": (ctypes.c_int, [_vp, _vp, _i64, _i64, _vp, _i64, _i64, _i64, _i64, _i64, _i64, _d, _vp, _i64, _vp,
+                                      _vp, _vp, ctypes.POINTER(_i32)]),
     "dfk_lm_counters_read": (ctypes.c_int, [_vp, ctypes.POINTER(LmCounters), _i32]),
     "dfk_profile_enable": (ctypes.c_int, [_vp, _i32]),
     "dfk_profile_read": (ctypes.c_int, [_vp, c_double_p, ctypes.POINTER(_i64), _i32]),
@@ -541,6 +543,23 @@ class Context:
                                                     enbw.ctypes.data, navs.ctypes.data))
         return {"f": f, "enbw": enbw, "navs": navs, "Sxx": sxx, "Syy": syy, "Sxy": sxy, "H": h, "Sres": sres,
                 "mcoh": mcoh}
+
+    def wiener_dev(self, x_ptr, Cx, ldx, y_ptr, Cy, ldy, N, stride, L, lead, ridge=0.0, res_ptr=None, ld_res=0,
+                   filters=True, variances=True) -> dict:
+        """Least-squares multi-input FIR filters of Cy device-resident targets y on Cx witnesses x (L taps, lead k0)
+        and, when ``res_ptr`` is given, the residual written there ([Cy][ld_res], M = N - L + 1 samples per target).
+        Returns host arrays h[Cy, Cx, L] (if ``filters``), var_y[Cy] and var_res[Cy] (if ``variances``) and the
+        ``singular`` flag; an output not asked for is passed to the library as NULL."""
+        cx, cy, taps = int(Cx), int(Cy), int(L)
+        h = np.empty((cy, cx, taps)) if filters else None
+        var_y = np.empty(cy) if variances else None
+        var_res = np.empty(cy) if variances else None
+        singular = _i32()
+        ptr = lambda a: a.ctypes.data if a is not None else None  # noqa: E731
+        _check(self.lib, self.lib.dfk_wiener_dev(self._h, x_ptr, cx, int(ldx), y_ptr, cy, int(ldy), int(N), int(stride),
+                                                 taps, int(lead), float(ridge), res_ptr, int(ld_res), ptr(h),
+                                                 ptr(var_y), ptr(var_res), ctypes.byref(singular)))
+        return {"h": h, "var_y": var_y, "var_res": var_res, "singular": bool(singular.value)}
 
     def set_host_slab_bytes(self, nbytes=0):
         """Slab size of the host-pointer entries (0: defaults); small values make a short record stream."""

@@ -8,7 +8,8 @@ INTEGRATION.md shows the opposite direction too: the reference's own façade poi
 signatures, default labels, the ``tau`` column, the error behaviour (log + ``None``) and the fields of the returned
 objects are those of the reference.  ``DeepFitObject.calc_csd`` is this package's addition: the cross-spectral estimate
 (CSD, coherence, transfer function) of one fit against another on the LPSD frequency plan; ``calc_conditioned`` is its
-multi-witness counterpart (joint transfer functions, residual PSD, multiple coherence).
+multi-witness counterpart (joint transfer functions, residual PSD, multiple coherence), and ``subtract_witnesses``
+performs that subtraction in the time domain (least-squares FIR filters, the cleaned series).
 """
 from __future__ import annotations
 
@@ -197,6 +198,22 @@ class DeepFitObject:
         (f, enbw, navs, Sxx, Syy, Sxy, H, Sres, mcoh) with this fit as the one target.  Stores nothing.  Every fit must
         have this fit's rate and number of buffers."""
         from .spectra import lcsd_conditioned
+        xs, y = self._witness_series(witness_fits, column)
+        return lcsd_conditioned(xs, y, self.fs, self.olap, self.bmin, self.Lmin, self.Jdes, self.Kdes, self.order,
+                                self.win, self.psll)
+
+    def subtract_witnesses(self, witness_fits, taps, lead=None, ridge=0.0, column="phi"):
+        """Time-domain witness subtraction of this fit's ``column`` on the device: the ``wiener_subtract`` dict (h,
+        offsets, n0, lead, residual, var_y, var_res, explained, singular) with the same column of every fit in
+        ``witness_fits`` (one fit or a sequence of up to 64) as witnesses and this fit as the one target.  Stores
+        nothing.  Every fit must have this fit's rate and number of buffers."""
+        from .spectra import wiener_subtract
+        xs, y = self._witness_series(witness_fits, column)
+        return wiener_subtract(xs, np.asarray(y, dtype=np.float64), taps, lead, ridge)
+
+    def _witness_series(self, witness_fits, column):
+        """([Cx, N] witness columns, this fit's column) after checking that there is at least one witness fit and that
+        every fit has this fit's rate and length."""
         if isinstance(witness_fits, DeepFitObject):
             witness_fits = [witness_fits]
         witness_fits = list(witness_fits)
@@ -215,8 +232,7 @@ class DeepFitObject:
             if len(x) != len(y):
                 raise ValueError(f"series lengths differ: {len(y)} and {len(x)}")
             xs.append(np.asarray(x, dtype=np.float64))
-        return lcsd_conditioned(np.stack(xs), y, self.fs, self.olap, self.bmin, self.Lmin, self.Jdes, self.Kdes,
-                                self.order, self.win, self.psll)
+        return np.stack(xs), y
 
 
 class DeepFitFramework:

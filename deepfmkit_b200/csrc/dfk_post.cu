@@ -1,10 +1,12 @@
-// Post-fit entries of the C ABI (include/dfk_b200.h, "post-fit step"): block means and log-frequency spectra.
+// Post-fit entries of the C ABI (include/dfk_b200.h, "post-fit step"): block means, log-frequency spectra and
+// time-domain witness subtraction.
 #include "dfk_host.h"
 
 #include <cmath>
 #include <vector>
 
 #include "dfk_spectra.cuh"
+#include "dfk_wiener.cuh"
 
 namespace {
 
@@ -403,6 +405,171 @@ int dfk_lcsd_cond_dev(dfk_ctx* ctx, const double* x_dev, int64_t Cx, int64_t ldx
     if (rc) return rc;
     DFK_CUDA(cudaStreamSynchronize(st));
     copy_plan_out(dp, f_host, navs_host);
+    return DFK_OK;
+}
+
+int dfk_wiener_dev(dfk_ctx* ctx, const double* x_dev, int64_t Cx, int64_t ldx, const double* y_dev, int64_t Cy,
+                   int64_t ldy, int64_t N, int64_t stride, int64_t L, int64_t lead, double ridge, double* res_dev,
+                   int64_t ld_res, double* h_host, double* var_y_host, double* var_res_host, int32_t* singular_out) {
+    DFK_ENTER(ctx);
+    if (!x_dev || !y_dev) return fail(DFK_ERR_ARG, "null pointer");
+    if (Cx < 1 || Cx > dfk::kWienerMaxWitnesses || Cy < 1 || Cx + Cy > 65535 || stride < 1)
+        return fail(DFK_ERR_ARG, "bad geometry: Cx=%lld (1..%d) Cy=%lld (Cx + Cy <= 65535) stride=%lld", (long long)Cx,
+                    dfk::kWienerMaxWitnesses, (long long)Cy, (long long)stride);
+    if (L < 1 || L > dfk::kWienerMaxUnknowns || Cx * L > dfk::kWienerMaxUnknowns)
+        return fail(DFK_ERR_ARG, "bad filter length: L=%lld, Cx L=%lld (at most %d)", (long long)L, (long long)(Cx * L),
+                    dfk::kWienerMaxUnknowns);
+    if (lead < 0 || lead > L - 1) return fail(DFK_ERR_ARG, "lead %lld outside 0..%lld", (long long)lead, (long long)(L - 1));
+    if (!(ridge >= 0.0) || !std::isfinite(ridge)) return fail(DFK_ERR_ARG, "ridge must be finite and >= 0");
+    const long long nu = Cx * L, M = N - L + 1, n0 = L - 1 - lead;
+    if (M < nu)
+        return fail(DFK_ERR_ARG, "N=%lld gives %lld rows for %lld unknowns (need N >= Cx L + L - 1)", (long long)N, M, nu);
+    if (res_dev && (Cy > 1 && ld_res < M))
+        return fail(DFK_ERR_ARG, "ld_res=%lld below the %lld residual samples", (long long)ld_res, M);
+    const long long ns = Cx + Cy;
+    // lag sums: column tiles, chunk length T sized so that the staging fits 48 KB, slices for about 2048 CTAs
+    dfk::LagParams P;
+    P.S.x = x_dev;
+    P.S.y = y_dev;
+    P.S.ldx = ldx;
+    P.S.ldy = ldy;
+    P.S.stride = stride;
+    P.S.cx = Cx;
+    P.S.cy = Cy;
+    P.S.N = N;
+    P.L = L;
+    P.k0 = lead;
+    P.ncx = Cx * (2 * L - 1);
+    P.ncols = P.ncx + Cy * L;
+    P.col_tiles = (P.ncols + dfk::kLagCols - 1) / dfk::kLagCols;
+    const long long row_tiles = (Cx + dfk::kLagRows - 1) / dfk::kLagRows, tiles = row_tiles * P.col_tiles;
+    long long nser = 1;
+    for (long long ct = 0; ct < P.col_tiles; ++ct) {
+        const long long c0 = ct * dfk::kLagCols, c1 = std::min(c0 + dfk::kLagCols, P.ncols) - 1;
+        nser = std::max(nser, dfk::lag_col_series(c1, Cx, P.ncx, L) - dfk::lag_col_series(c0, Cx, P.ncx, L) + 1);
+    }
+    constexpr long long kStage = 6144;
+    long long T = (kStage - dfk::kLagCols + nser) / (dfk::kLagRows + nser);
+    T = std::max(4ll, std::min(512ll, T & ~3ll));
+    P.T = static_cast<int>(T);
+    P.q_begin = L - 1;
+    P.q_end = N - L + 1;
+    const long long Q = P.q_end - P.q_begin;
+    long long nslices = std::max(1ll, std::min((2048 + tiles - 1) / tiles, (Q + T - 1) / T));
+    P.slice = (((Q + nslices - 1) / nslices + T - 1) / T) * T;
+    nslices = (Q + P.slice - 1) / P.slice;
+    P.part_stride = tiles * dfk::kLagTileEntries;
+    const size_t lag_smem =
+        sizeof(double) * static_cast<size_t>(std::max(dfk::kLagRows * T + nser * (T - 1) + dfk::kLagCols,
+                                                      static_cast<long long>(4 * dfk::kLagTileEntries)));
+    const long long apply_tiles = (M + dfk::kApplyTile - 1) / dfk::kApplyTile;
+    if (tiles > 0x7fffffffll || nslices > 65535 || apply_tiles > 0x7fffffffll)
+        return fail(DFK_ERR_ARG, "Wiener problem too large for one launch");
+    const bool apply = res_dev || var_res_host;
+    // post[0]: means [ns], var_y [Cy], var_res [Cy], diag0 [nu], the factored diagonal tile of the current Cholesky
+    // step [64][64], tile sums of e^2 [Cy][apply_tiles], flag
+    // post[1]: lag-sum slice partials; post[2]: G [nu][nu], then p / h [Cy][nu]
+    DevBuf& small_dev = ctx->post[0];
+    DevBuf& part_dev = ctx->post[1];
+    DevBuf& mat_dev = ctx->post[2];
+    const size_t small_doubles =
+        static_cast<size_t>(ns + 2 * Cy + nu + dfk::kCholBlock * dfk::kCholBlock + Cy * apply_tiles + 1);
+    int rc = ensure(ctx, small_dev, sizeof(double) * small_doubles);
+    if (!rc) rc = ensure(ctx, part_dev, sizeof(double) * static_cast<size_t>(nslices) * static_cast<size_t>(P.part_stride));
+    if (!rc) rc = ensure(ctx, mat_dev, sizeof(double) * static_cast<size_t>(nu) * static_cast<size_t>(nu + Cy));
+    if (rc) return rc;
+    double* mean_dev = static_cast<double*>(small_dev.ptr);
+    double* var_y_dev = mean_dev + ns;
+    double* var_res_dev = var_y_dev + Cy;
+    double* diag0_dev = var_res_dev + Cy;
+    double* lkk_dev = diag0_dev + nu;
+    double* vpart_dev = lkk_dev + dfk::kCholBlock * dfk::kCholBlock;
+    int* flag_dev = reinterpret_cast<int*>(vpart_dev + Cy * apply_tiles);
+    double* G_dev = static_cast<double*>(mat_dev.ptr);
+    double* rhs_dev = G_dev + nu * nu;
+    P.S.mean = mean_dev;
+    P.part = static_cast<double*>(part_dev.ptr);
+    cudaStream_t st = ctx->stream();
+    long long launches = 0;
+
+    dfk::wiener_means_kernel<<<static_cast<unsigned>(ns), dfk::kWMeanThreads, 0, st>>>(P.S, n0, M, mean_dev, var_y_dev);
+    DFK_CUDA(cudaGetLastError());
+    DFK_CUDA(cudaFuncSetAttribute(dfk::wiener_lag_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                                  static_cast<int>(lag_smem)));
+    dfk::wiener_lag_kernel<<<dim3(static_cast<unsigned>(tiles), static_cast<unsigned>(nslices)), dfk::kLagThreads,
+                             lag_smem, st>>>(P);
+    DFK_CUDA(cudaGetLastError());
+    dfk::AssembleParams A;
+    A.P = P;
+    A.nslices = nslices;
+    A.nu = nu;
+    A.G = G_dev;
+    A.rhs = rhs_dev;
+    const long long assemble_threads = nu * (nu + Cy);
+    dfk::wiener_assemble_kernel<<<static_cast<unsigned>((assemble_threads + dfk::kAssembleThreads - 1) /
+                                                        dfk::kAssembleThreads),
+                                  dfk::kAssembleThreads, 0, st>>>(A);
+    DFK_CUDA(cudaGetLastError());
+    dfk::wiener_load_kernel<<<1, dfk::kWMeanThreads, 0, st>>>(G_dev, nu, ridge, diag0_dev, flag_dev);
+    DFK_CUDA(cudaGetLastError());
+    launches += 4;
+    DFK_CUDA(cudaFuncSetAttribute(dfk::chol_panel_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                                  dfk::kCholPanelSmem));
+    for (long long k0 = 0; k0 < nu; k0 += dfk::kCholBlock) {
+        const long long below = nu - std::min(nu, k0 + dfk::kCholBlock);
+        const long long bt = (below + dfk::kCholBlock - 1) / dfk::kCholBlock;
+        dfk::chol_panel_kernel<<<static_cast<unsigned>(1 + bt), dfk::kCholThreads, dfk::kCholPanelSmem, st>>>(
+            G_dev, nu, k0, diag0_dev, flag_dev, lkk_dev);
+        DFK_CUDA(cudaGetLastError());
+        ++launches;
+        if (bt == 0) break;
+        const unsigned update_tiles = static_cast<unsigned>(bt * (bt + 1) / 2);
+        dfk::chol_update_kernel<<<update_tiles, dfk::kCholThreads, 0, st>>>(G_dev, nu, k0, lkk_dev);
+        DFK_CUDA(cudaGetLastError());
+        ++launches;
+    }
+    dfk::wiener_solve_kernel<<<static_cast<unsigned>(Cy), dfk::kSolveThreads, 0, st>>>(G_dev, nu, rhs_dev, flag_dev);
+    DFK_CUDA(cudaGetLastError());
+    ++launches;
+    if (apply) {
+        dfk::ApplyParams Y;
+        Y.S = P.S;
+        Y.L = L;
+        Y.nu = nu;
+        Y.n0 = n0;
+        Y.M = M;
+        const long long span = dfk::kApplyTile + L - 1;
+        Y.chunk = static_cast<int>(std::max(1ll, std::min(static_cast<long long>(Cx), dfk::kApplyStageDoubles / span)));
+        Y.h = rhs_dev;
+        Y.flag = flag_dev;
+        Y.res = res_dev;
+        Y.ld_res = ld_res;
+        Y.vpart = var_res_host ? vpart_dev : nullptr;
+        Y.tiles = apply_tiles;
+        const size_t apply_smem = sizeof(double) * static_cast<size_t>(dfk::kApplyTargets * nu + Y.chunk * span);
+        DFK_CUDA(cudaFuncSetAttribute(dfk::wiener_apply_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                                      static_cast<int>(apply_smem)));
+        const dim3 grid(static_cast<unsigned>(apply_tiles),
+                        static_cast<unsigned>((Cy + dfk::kApplyTargets - 1) / dfk::kApplyTargets));
+        dfk::wiener_apply_kernel<<<grid, dfk::kApplyThreads, apply_smem, st>>>(Y);
+        DFK_CUDA(cudaGetLastError());
+        ++launches;
+        if (var_res_host) {
+            dfk::wiener_var_kernel<<<static_cast<unsigned>((Cy + 127) / 128), 128, 0, st>>>(vpart_dev, apply_tiles, Cy,
+                                                                                           M, var_res_dev);
+            DFK_CUDA(cudaGetLastError());
+            ++launches;
+        }
+    }
+    ctx->launches += launches;
+    if (h_host) DFK_CUDA(cudaMemcpyAsync(h_host, rhs_dev, sizeof(double) * Cy * nu, cudaMemcpyDeviceToHost, st));
+    if (var_y_host) DFK_CUDA(cudaMemcpyAsync(var_y_host, var_y_dev, sizeof(double) * Cy, cudaMemcpyDeviceToHost, st));
+    if (var_res_host)
+        DFK_CUDA(cudaMemcpyAsync(var_res_host, var_res_dev, sizeof(double) * Cy, cudaMemcpyDeviceToHost, st));
+    int32_t flag = 0;
+    DFK_CUDA(cudaMemcpyAsync(&flag, flag_dev, sizeof(int32_t), cudaMemcpyDeviceToHost, st));
+    DFK_CUDA(cudaStreamSynchronize(st));
+    if (singular_out) *singular_out = flag;
     return DFK_OK;
 }
 

@@ -7,7 +7,8 @@ form, a 6-tuple whose first element is the frequency vector and whose third is t
 the reference stores as ``Sxx``.  ``lcsd`` is the cross-spectral counterpart on the same frequency plan: the CSD,
 coherence and transfer function between fitted channels.  ``lcsd_conditioned`` extends it to several witnesses at
 once: the joint transfer functions, the conditioned (residual) PSD and the multiple coherence of each target given all
-witnesses.  All run on the device only.
+witnesses.  ``wiener_subtract`` does that subtraction in the time domain: least-squares multi-input FIR filters and
+the cleaned target series.  All run on the device only.
 """
 from __future__ import annotations
 
@@ -233,3 +234,81 @@ def lcsd_conditioned(witnesses, targets, fs, olap="default", bmin=1, Lmin=0, Jde
         out["Syy"], out["Sres"], out["mcoh"] = out["Syy"][0], out["Sres"][0], out["mcoh"][0]
         out["Sxy"], out["H"] = out["Sxy"][:, 0], out["H"][:, 0]
     return out
+
+
+MAX_WIENER_UNKNOWNS = 1024  # Cx * taps: the normal matrix (8 MB) stays resident in L2 for the factorisation
+
+
+def wiener_subtract(witnesses, targets, taps, lead=None, ridge=0.0, device=0):
+    """Time-domain witness subtraction: the least-squares multi-input FIR (Wiener) filters that best predict each
+    target from all witnesses, and the targets with that prediction subtracted, on the device.
+
+    ``witnesses`` is ``[N]`` or ``[Cx, N]`` with 1 <= Cx <= 64, ``targets`` is ``[N]`` or ``[Cy, N]``; numpy arrays or
+    CUDA tensors, handled as by ``lcsd_conditioned``.  With x~, y~ the series less their means over all N samples,
+    L = ``taps``, k0 = ``lead`` (default (L - 1) // 2, a centred two-sided filter; 0 is causal), n0 = L - 1 - k0 and
+    M = N - L + 1 (the rows n0 .. n0 + M - 1 on which every tap is inside the record):
+
+    - model: yhat_t[n] = sum_a sum_k h[t, a, k] x~_a[n + k0 - k]; tap k looks ``offsets[k]`` = k0 - k samples away;
+    - ``h`` [Cy, Cx, L] solves (G + lambda I) h_t = p_t, the normal equations over the M rows
+      (G[(a,k),(b,l)] = sum_n x~_a[n+k0-k] x~_b[n+k0-l], p[(a,k),t] = sum_n x~_a[n+k0-k] y~_t[n]), with the diagonal
+      loading lambda = ``ridge`` * trace(G) / (Cx L);
+    - ``residual`` [Cy, M]: y~_t[n0 + i] - yhat_t[n0 + i]; a CUDA tensor when an input was one, numpy otherwise;
+    - ``var_y``, ``var_res`` [Cy]: mean squares of y~ and of the residual over the same rows; ``explained`` [Cy]:
+      1 - var_res / var_y, NaN where var_y is 0;
+    - ``offsets`` [L], ``n0``, ``lead``, and ``singular``: True when a Cholesky pivot of G + lambda I is not above
+      1e-10 times its diagonal entry (a duplicated or linearly dependent witness with ``ridge`` 0).  ``h``, the
+      residual, ``var_res`` and ``explained`` are then NaN; ``var_y`` stays finite.
+
+    Limits: Cx * L <= 1024 and M >= Cx * L (no underdetermined systems); Cx + Cy <= 65535.  Callers detrend beyond the
+    mean themselves.  A 1-D ``targets`` drops the Cy axis."""
+    import torch
+    nx, ny = (tuple(a.shape) if hasattr(a, "shape") else np.shape(a) for a in (witnesses, targets))
+    if len(nx) not in (1, 2) or len(ny) not in (1, 2) or nx[-1] != ny[-1]:
+        raise ValueError(f"witnesses and targets must be series of the same number of samples, got shapes {nx} and {ny}")
+    Cx, Cy, N = (1 if len(nx) == 1 else nx[0]), (1 if len(ny) == 1 else ny[0]), nx[-1]
+    if not 1 <= Cx <= MAX_WITNESSES:
+        raise ValueError(f"{Cx} witnesses: between 1 and {MAX_WITNESSES} are supported")
+    if Cy < 1 or Cx + Cy > 65535:
+        raise ValueError(f"{Cy} targets: at least 1, and at most 65535 series in all")
+    if not isinstance(taps, (int, np.integer)) or isinstance(taps, bool) or taps < 1:
+        raise ValueError(f"taps must be a positive integer, got {taps!r}")
+    L = int(taps)
+    if Cx * L > MAX_WIENER_UNKNOWNS:
+        raise ValueError(f"{Cx} witnesses x {L} taps = {Cx * L} unknowns: at most {MAX_WIENER_UNKNOWNS}")
+    if lead is None:
+        lead = (L - 1) // 2
+    if not isinstance(lead, (int, np.integer)) or isinstance(lead, bool) or not 0 <= lead <= L - 1:
+        raise ValueError(f"lead must be an integer in 0..{L - 1}, got {lead!r}")
+    lead = int(lead)
+    if isinstance(ridge, bool) or not np.isscalar(ridge) or not np.isfinite(ridge) or ridge < 0:
+        raise ValueError(f"ridge must be finite and >= 0, got {ridge!r}")
+    M = N - L + 1
+    if M < Cx * L:
+        raise ValueError(f"{N} samples give {M} rows for {Cx * L} unknowns: need N >= Cx L + L - 1")
+    tensors = [a for a in (witnesses, targets) if isinstance(a, torch.Tensor) and a.is_cuda]
+    if tensors:
+        device = tensors[0].device.index
+    xt, _ = _device_rows(witnesses, device)
+    yt, y1 = _device_rows(targets, device)
+    if xt.device != yt.device:
+        raise ValueError(f"witnesses and targets are on different devices ({xt.device}, {yt.device})")
+    res = torch.empty((Cy, M), dtype=torch.float64, device=xt.device)
+    ctx = _lib.get_context(device)
+    with torch.cuda.device(xt.device):
+        ctx.use_torch_stream()
+        try:
+            out = ctx.wiener_dev(xt.data_ptr(), Cx, N, yt.data_ptr(), Cy, N, N, 1, L, lead, float(ridge),
+                                 res.data_ptr(), M)
+        finally:
+            ctx.use_default_stream()
+    var_y, var_res = out["var_y"], out["var_res"]
+    explained = np.full(Cy, np.nan)
+    np.divide(var_res, var_y, out=explained, where=var_y != 0)
+    explained = np.where(var_y != 0, 1.0 - explained, np.nan)
+    result = {"h": out["h"], "offsets": lead - np.arange(L), "n0": L - 1 - lead, "lead": lead,
+              "residual": res if tensors else res.cpu().numpy(), "var_y": var_y, "var_res": var_res,
+              "explained": explained, "singular": out["singular"]}
+    if y1:
+        for k in ("h", "residual", "var_y", "var_res", "explained"):
+            result[k] = result[k][0]
+    return result

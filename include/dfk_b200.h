@@ -425,6 +425,24 @@ int dfk_lcsd_cond_dev(dfk_ctx* ctx, const double* x_dev, int64_t Cx, int64_t ldx
                       int64_t ldy, int64_t N, int64_t stride, double fs, const dfk_lpsd_opts* opts, int32_t cap,
                       int32_t* nf_out, double* f_host, double* sxx_host, double* syy_host, double* sxy_host,
                       double* h_host, double* sres_host, double* mcoh_host, double* enbw_host, int64_t* navs_host);
+/* Time-domain witness subtraction: the least-squares multi-input FIR (Wiener) filters that best predict each target
+ * y_t from the witnesses x_a, and the target with that prediction subtracted.  Series are read as by dfk_lcsd_dev
+ * (sample q of series u at x_dev[u ldx + q stride]).  With x~, y~ the series less their means over all N samples,
+ * L taps, lead k0 (0 <= k0 <= L-1; 0 is causal, (L-1)/2 a centred two-sided filter), n0 = L-1-k0, M = N-L+1:
+ *     yhat_t[n] = sum_a sum_{k<L} h[t,a,k] x~_a[n + k0 - k]          tap k looks k0 - k samples away
+ *     G[(a,k),(b,l)] = sum_n x~_a[n+k0-k] x~_b[n+k0-l],  p[(a,k),t] = sum_n x~_a[n+k0-k] y~_t[n],  n in [n0, n0+M)
+ *     (G + lambda I) h_t = p_t,  lambda = ridge trace(G) / (Cx L)
+ *     res[t][i] = y~_t[n0+i] - yhat_t[n0+i],  var_y = (1/M) sum y~_t^2,  var_res = (1/M) sum res^2  (i < M)
+ * A Cholesky pivot not above 1e-10 times its loaded diagonal entry (a duplicated or linearly dependent witness with
+ * ridge 0) sets *singular_out = 1; h, res and var_res are then NaN and var_y stays finite.  Limits: 1 <= Cx <= 64,
+ * Cy >= 1, Cx + Cy <= 65535, L >= 1, Cx L <= 1024, M >= Cx L, ridge finite and >= 0 (DFK_ERR_ARG otherwise).
+ * Outputs: res_dev [Cy][ld_res] on the device (M samples per target), h_host [Cy][Cx][L], var_y_host and var_res_host
+ * [Cy], singular_out; any may be NULL.  The sums are formed in a fixed order (bit-identical from run to run).
+ * Launches: 2 ceil(Cx L / 64) + 4, plus 1 when res_dev or var_res_host is given, plus 1 more for var_res_host.
+ * Synchronises like dfk_lpsd_dev. */
+int dfk_wiener_dev(dfk_ctx* ctx, const double* x_dev, int64_t Cx, int64_t ldx, const double* y_dev, int64_t Cy,
+                   int64_t ldy, int64_t N, int64_t stride, int64_t L, int64_t lead, double ridge, double* res_dev,
+                   int64_t ld_res, double* h_host, double* var_y_host, double* var_res_host, int32_t* singular_out);
 
 /* ---- introspection ------------------------------------------------------------------------ */
 /* Counters accumulated by the LM kernels since the last reset (device -> host copy, syncs). */
