@@ -95,6 +95,8 @@ SYMBOLS = {
     "dfk_ekf_dev": (ctypes.c_int, [_vp, _vp, _i64, _i64, _i64, _i64, _i64, _d, _d, ctypes.POINTER(EkfOpts), _vp]),
     "dfk_ekf_stream_dev": (ctypes.c_int, [_vp, _vp, _i64, _i64, _i64, _i64, _i64, _d, _d, ctypes.POINTER(EkfOpts), _i64,
                                           _vp, _vp]),
+    "dfk_ekf_smooth_dev": (ctypes.c_int, [_vp, _vp, _i64, _i64, _i64, _i64, _i64, _d, _d, ctypes.POINTER(EkfOpts), _i64,
+                                          _vp, _i64, _vp, _vp, _vp, _vp]),
     "dfk_synth_snr_slab_dev": (ctypes.c_int, [_vp, _vp, _i64, _i64, _i64, _i64, _d, _d, _d, _d, _d, _d, _d, _d, _d,
                                               ctypes.c_uint64]),
     "dfk_synth_snr_dev": (ctypes.c_int, [_vp, _vp, _i64, _i64, _d, _d, _d, _d, _d, _d, _d, _d, _d, ctypes.c_uint64]),
@@ -350,6 +352,15 @@ class Context:
         _check(self.lib, self.lib.dfk_ekf_stream_dev(self._h, z_ptr, T, C, ld_t, ld_c, R, f_samp, f_mod,
                                                      ctypes.byref(opts) if opts is not None else None, k0, state_ptr,
                                                      rows_ptr))
+
+    def ekf_smooth_dev(self, z_ptr, T, C, ld_t, ld_c, R, f_samp, f_mod, opts, k0, state_ptr, block, rows_ptr,
+                       var_ptr=None, filt_rows_ptr=None, filt_var_ptr=None):
+        """RTS smoother over a resident window (dfk_ekf_smooth_dev); outputs not wanted are None."""
+        _check(self.lib, self.lib.dfk_ekf_smooth_dev(self._h, z_ptr, int(T), int(C), int(ld_t), int(ld_c), int(R),
+                                                     float(f_samp), float(f_mod),
+                                                     ctypes.byref(opts) if opts is not None else None, int(k0),
+                                                     state_ptr, int(block), rows_ptr, var_ptr, filt_rows_ptr,
+                                                     filt_var_ptr))
 
     def synth_snr_slab_dev(self, x_ptr, T, C, ld_c, t0, f_samp, f_mod, m, amp=1.0, visibility=1.0, phi0=0.0, dphi=0.0,
                            psi0=0.0, snr_db=40.0, seed=0):

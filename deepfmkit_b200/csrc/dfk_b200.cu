@@ -19,6 +19,7 @@
 
 #include "dfk_demod.cuh"
 #include "dfk_ekf_kernels.cuh"
+#include "dfk_ekf_smooth.cuh"
 #include "dfk_lm_kernels.cuh"
 #include "dfk_synth.cuh"
 #include "dfk_sweep.cuh"
@@ -681,6 +682,17 @@ Schedule schedule_of(int32_t seeded) {
     return sc;
 }
 
+// Channels per one-warp block of the EKF kernels: the fewest that still leave every warp a scheduler (sub-partition)
+// of its own; the development setting DFK_EKF_CPW forces a power of two <= 32.
+int ekf_channels_per_warp(const dfk_ctx* ctx, int64_t C) {
+    const int64_t schedulers = static_cast<int64_t>(ctx->sm_count) * 4;
+    int cpw = 1;
+    while (cpw < 32 && (C + cpw - 1) / cpw > schedulers) cpw <<= 1;
+    const int forced = dev_int("DFK_EKF_CPW", 0);
+    if (forced == 1 || forced == 2 || forced == 4 || forced == 8 || forced == 16 || forced == 32) cpw = forced;
+    return cpw;
+}
+
 // Per-channel mean and variance of a device record (either layout); see dfk_ekf_kernels.cuh.
 int launch_channel_stats(dfk_ctx* ctx, const double* z, int64_t T, int64_t C, int64_t ld_t, int64_t ld_c, double* stats,
                          double* acc, cudaStream_t st) {
@@ -803,7 +815,7 @@ int dfk_destroy(dfk_ctx* ctx) {
     if (ctx->copy_stream) cudaStreamSynchronize(ctx->copy_stream);
     if (ctx->aux_stream) cudaStreamSynchronize(ctx->aux_stream);
     DevBuf* bufs[] = {&ctx->qi, &ctx->dc, &ctx->retry, &ctx->counters, &ctx->slab[0], &ctx->slab[1],
-                      &ctx->rows, &ctx->stats, &ctx->stats_part, &ctx->misc, &ctx->qi_seed, &ctx->dc_seed, &ctx->cov};
+                      &ctx->rows, &ctx->stats, &ctx->stats_part, &ctx->misc, &ctx->qi_seed, &ctx->dc_seed, &ctx->cov, &ctx->smooth};
     for (DevBuf* b : bufs)
         if (b->ptr) cudaFree(b->ptr);
     for (DevBuf& b : ctx->post)
@@ -1137,17 +1149,80 @@ int dfk_ekf_stream_dev(dfk_ctx* ctx, const double* z_dev, int64_t T, int64_t C, 
     a.r_val = opts->r_val;
     a.w_m = 2 * dfk::kPi * f_mod;  // fitters.py:262
     a.f_samp = f_samp;
-    // fewest channels per warp that still leaves every warp a scheduler (sub-partition) of its own
-    const int64_t schedulers = static_cast<int64_t>(ctx->sm_count) * 4;
-    int cpw = 1;
-    while (cpw < 32 && (C + cpw - 1) / cpw > schedulers) cpw <<= 1;
-    const int forced = dev_int("DFK_EKF_CPW", 0);
-    if (forced == 1 || forced == 2 || forced == 4 || forced == 8 || forced == 16 || forced == 32) cpw = forced;
+    const int cpw = ekf_channels_per_warp(ctx, C);
     a.cpw = cpw;
     const int64_t grid = (C + cpw - 1) / cpw;
     if (grid > std::numeric_limits<int>::max()) return fail(DFK_ERR_ARG, "too many channels");
     ProfScope ps(ctx, 3, st);
     return launch_kernel(ctx, dfk::ekf_kernel, static_cast<int>(grid), 32, 0, st, z_dev, T, C, ld_t, ld_c, R, a, stats, rows_dev);
+}
+
+int dfk_ekf_smooth_dev(dfk_ctx* ctx, const double* z_dev, int64_t T, int64_t C, int64_t ld_t, int64_t ld_c, int64_t R,
+                       double f_samp, double f_mod, const dfk_ekf_opts* opts, int64_t k0, const double* state_dev,
+                       int64_t block, double* rows_dev, double* var_dev, double* filt_rows_dev, double* filt_var_dev) {
+    DFK_ENTER(ctx);
+    if (k0 < 0 || (R > 0 && k0 % R != 0)) return fail(DFK_ERR_ARG, "k0 must be a non-negative multiple of R");
+    if (k0 > 0 && !state_dev) return fail(DFK_ERR_ARG, "a window that starts at k0 > 0 needs the carried state");
+    if (T < 0 || C < 0 || R <= 0) return fail(DFK_ERR_ARG, "bad geometry: T=%lld C=%lld R=%lld", (long long)T, (long long)C, (long long)R);
+    if (!(f_samp > 0.0) || !(f_mod > 0.0)) return fail(DFK_ERR_ARG, "f_samp and f_mod must be positive");
+    if (block < 0 || block % dfk::kEkfTile != 0)
+        return fail(DFK_ERR_ARG, "block must be 0 (library's choice) or a positive multiple of %d", dfk::kEkfTile);
+    if (T / R == 0 || C == 0) return DFK_OK;
+    if (!z_dev || !rows_dev) return fail(DFK_ERR_ARG, "null device pointer");
+    dfk_ekf_opts d;
+    if (!opts) {
+        dfk_default_ekf_opts(&d);
+        opts = &d;
+    }
+    const int64_t t_round = (T + dfk::kEkfTile - 1) / dfk::kEkfTile * dfk::kEkfTile;
+    const int64_t B = std::min<int64_t>(block ? block : dfk::kSmoothBlockDefault, t_round);
+    const int64_t nblk = (T + B - 1) / B;
+    // C (nblk + B) 20 doubles; C < 2^31 * 32 and nblk + B <= T + 32, so the product is formed in 128 bits
+    const unsigned __int128 want = static_cast<unsigned __int128>(C) * static_cast<unsigned __int128>(nblk + B) *
+                                   dfk::kSmoothDoubles * sizeof(double);
+    size_t free_b = 0, total_b = 0;
+    DFK_CUDA(cudaMemGetInfo(&free_b, &total_b));
+    if (want > static_cast<unsigned __int128>(free_b) + ctx->smooth.bytes)
+        return fail(DFK_ERR_NOMEM, "smoother scratch of %.0f bytes (checkpoints every %lld samples and a block store) does "
+                    "not fit the device's %zu free bytes", static_cast<double>(want), (long long)B, free_b + ctx->smooth.bytes);
+    int rc = ensure(ctx, ctx->smooth, static_cast<size_t>(want));
+    if (rc) return rc;
+    rc = ensure(ctx, ctx->stats, static_cast<size_t>(C) * 2 * sizeof(double));
+    if (rc) return rc;
+    cudaStream_t st = ctx->stream();
+    double* stats = static_cast<double*>(ctx->stats.ptr);
+    if (!state_dev && (std::isnan(opts->init_dc) || std::isnan(opts->r_val))) {
+        rc = launch_channel_stats(ctx, z_dev, T, C, ld_t, ld_c, stats, nullptr, st);
+        if (rc) return rc;
+    }
+    dfk::SmoothLaunch a;
+    a.f.k0 = k0;
+    a.f.state = const_cast<double*>(state_dev);  // read only: the smoother never writes the carried state
+    for (int i = 0; i < 4; ++i) a.f.init[i] = opts->init[i];
+    a.f.init_dc = opts->init_dc;
+    for (int i = 0; i < 5; ++i) {
+        a.f.p0[i] = opts->p0_diag[i];
+        a.f.q[i] = opts->q_diag[i];
+    }
+    a.f.r_val = opts->r_val;
+    a.f.w_m = 2 * dfk::kPi * f_mod;
+    a.f.f_samp = f_samp;
+    const int cpw = ekf_channels_per_warp(ctx, C);
+    a.f.cpw = cpw;
+    const int64_t grid = (C + cpw - 1) / cpw;
+    if (grid > std::numeric_limits<int>::max()) return fail(DFK_ERR_ARG, "too many channels");
+    a.B = B;
+    a.ckpt = static_cast<double*>(ctx->smooth.ptr);
+    a.store = a.ckpt + static_cast<size_t>(C) * nblk * dfk::kSmoothDoubles;
+    a.rows = rows_dev;
+    a.var = var_dev;
+    a.filt_rows = filt_rows_dev;
+    a.filt_var = filt_var_dev;
+    rc = launch_kernel(ctx, dfk::ekf_smooth_forward_kernel, static_cast<int>(grid), 32, 0, st, z_dev, T, C, ld_t, ld_c, R,
+                       a, stats);
+    if (rc) return rc;
+    return launch_kernel(ctx, dfk::ekf_smooth_backward_kernel, static_cast<int>(grid), 32, 0, st, z_dev, T, C, ld_t, ld_c,
+                         R, a, stats);
 }
 
 // EKFFitter.fit on host records [C][T].  A record that fits the device goes up whole.  A longer one (cfg 4 is 655 GB)

@@ -59,6 +59,7 @@ struct dfk_ctx {
     cudaEvent_t stager_free[kStagers] = {};
     DevBuf qi, dc, retry, counters, slab[2], rows, stats, stats_part, misc, qi_seed, dc_seed;
     DevBuf cov;  // covariance rows of a host record (dfk_nls_fit_cov_host)
+    DevBuf smooth;  // checkpoints and block store of dfk_ekf_smooth_dev
     static constexpr int kPostBufs = 8;
     DevBuf post[kPostBufs];  // scratch of the ingest / spectra / generator entries (dfk_post.cu, dfk_ingest.cu)
     int64_t launches = 0;

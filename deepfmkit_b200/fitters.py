@@ -150,7 +150,10 @@ class StandardNLSFitter(BaseFitter):
 
 
 class EKFFitter(BaseFitter):
-    """Time-domain 5-state EKF (fitters.py:210-320): one thread per channel, sequential in time."""
+    """Time-domain 5-state EKF (fitters.py:210-320): one thread per channel, sequential in time.
+
+    ``smooth=True`` returns the fixed-interval smoothed states instead of the filtered ones (see :func:`ekf_smooth`):
+    the state at each snapshot given the whole record, in the same columns."""
 
     def fit(self, main_raw, **kwargs) -> pd.DataFrame:
         if kwargs.get("uncertainties", False):
@@ -176,6 +179,12 @@ class EKFFitter(BaseFitter):
 
         R, _, nbuf = _calculate_fit_params(main_raw, n)
         zd = _device_record(main_raw)
+        if kwargs.get("smooth", False):
+            # the smoother needs the window resident: a host record is copied to the device whole
+            z = zd if zd is not None else _record_values(main_raw, column="ch0")
+            rows = _smooth(z[None, :], main_raw.f_samp, main_raw.f_mod, R, opts, 0, 0, None, False,
+                           zd.device.index if zd is not None else device)["rows"][0]
+            return rows_to_frame(rows)
         if zd is not None:
             import torch
             ctx = _lib.get_context(zd.device.index)
@@ -306,6 +315,20 @@ def ekf_fit_batch(z, f_samp, f_mod, n, time_major=False, device=0, return_tensor
         ld_t, ld_c = 1, T
     R = int(f_samp / f_mod * n)
     nbuf = T // R
+    opts = _batch_ekf_opts(kwargs)
+    rows = torch.empty((C, nbuf, _lib.ROW_STRIDE), dtype=torch.float64, device=dev)
+    with torch.cuda.device(dev):
+        ctx.use_torch_stream()
+        try:
+            ctx.ekf_dev(zt.data_ptr(), T, C, ld_t, ld_c, R, float(f_samp), float(f_mod), opts, rows.data_ptr())
+        finally:
+            ctx.use_default_stream()
+        torch.cuda.current_stream(dev).synchronize()
+    return rows if return_tensor else rows.cpu().numpy()
+
+
+def _batch_ekf_opts(kwargs):
+    """dfk_ekf_opts from ekf_fit_batch's keywords (init_a, init_m, init_phi, init_psi, P0_diag, Q_diag, R_val)."""
     opts = _lib.default_ekf_opts()
     for i, key in enumerate(("init_a", "init_m", "init_phi", "init_psi")):
         if key in kwargs:
@@ -317,12 +340,85 @@ def ekf_fit_batch(z, f_samp, f_mod, n, time_major=False, device=0, return_tensor
             opts.q_diag[i] = float(kwargs["Q_diag"][i])
     if kwargs.get("R_val") is not None:
         opts.r_val = float(kwargs["R_val"])
-    rows = torch.empty((C, nbuf, _lib.ROW_STRIDE), dtype=torch.float64, device=dev)
+    return opts
+
+
+def ekf_smooth(z, f_samp, f_mod, n, time_major=False, device=0, return_tensor=False, block=0, k0=0, state=None,
+               **kwargs):
+    """Fixed-interval (Rauch-Tung-Striebel) smoother of the EKF over C resident channels: the state at each snapshot
+    given the whole record, with its posterior variance.
+
+    z: ``[C, T]`` (or ``[T, C]`` with time_major=True), numpy or CUDA tensor; kwargs as :func:`ekf_fit_batch`.
+    With x_f[k], P_f[k] the filter's state and covariance after sample k (F = I): x_s[T-1] = x_f[T-1], and for
+    k = T-2 .. 0, with Pp = P_f[k] + diag(Q) and G = P_f[k] Pp^-1,
+
+        x_s[k] = x_f[k] + G (x_s[k+1] - x_f[k]),    P_s[k] = P_f[k] + G (P_s[k+1] - Pp) G^T,
+
+    the Kalman smoother of the linearisation the filter used.  Rows are taken at k_b = (b+1) R - 1 like the filter's,
+    R = int(f_samp / f_mod * n); samples after the last one still count as data.
+
+    k0, state: the window is samples k0 .. k0+T-1 of a longer record (k0 a multiple of R), started from ``state``
+    (``[C, 32]`` float64, the carried-state layout of ``dfk_ekf_stream_dev``: x, the covariance's upper triangle, r at
+    index 30), which is read and never written.  state=None (k0 = 0 only) starts from the options, NaN R_val / initial
+    dc from the record's variance / mean, as :func:`ekf_fit_batch` does.
+    block: the checkpoint interval (a positive multiple of 32, or 0 for the library's choice); results do not depend on it.
+
+    Returns a dict of ``rows`` and ``filtered`` ``[C, nbuf, 8]`` (the EKF row layout, so ``rows_to_frame`` takes them;
+    ``filtered`` is bit-identical to ``ekf_fit_batch``) and ``var`` and ``filtered_var`` ``[C, nbuf, 5]``, the
+    smoothed and filtered variances of a, m, phi, psi, dc.  A non-positive Cholesky pivot or a NaN sample makes that
+    channel's smoothed rows and variances NaN from there back to the start; filtered outputs and other channels are
+    unaffected.
+    """
+    shape = tuple(z.shape)
+    if len(shape) == 1:
+        shape = (1, shape[0]) if not time_major else (shape[0], 1)
+    C = shape[1] if time_major else shape[0]
+    R = int(f_samp / f_mod * n)
+    if isinstance(block, bool) or int(block) != block or block < 0 or block % 32:
+        raise ValueError("block must be 0 (library's choice) or a positive multiple of 32")
+    if isinstance(k0, bool) or int(k0) != k0 or k0 < 0 or (R > 0 and k0 % R):
+        raise ValueError(f"k0 must be a non-negative multiple of R = {R}")
+    if state is None:
+        if k0:
+            raise ValueError("a window that starts at k0 > 0 needs the carried state")
+    else:
+        sshape = tuple(state.shape) if hasattr(state, "shape") else np.shape(state)
+        if sshape != (C, 32):
+            raise ValueError(f"state must be [C, 32] = [{C}, 32], not {list(sshape)}")
+    return _smooth(z, f_samp, f_mod, R, _batch_ekf_opts(kwargs), int(block), int(k0), state, time_major, device,
+                   return_tensor)
+
+
+def _smooth(z, f_samp, f_mod, R, opts, block, k0, state, time_major, device, return_tensor=False):
+    import torch
+    ctx = _lib.get_context(device)
+    dev = torch.device("cuda", device)
+    zt = z if isinstance(z, torch.Tensor) else torch.from_numpy(np.ascontiguousarray(z, dtype=np.float64))
+    if zt.dim() == 1:
+        zt = zt[None, :]
+    zt = zt.to(dev).contiguous()
+    if time_major:
+        T, C = zt.shape
+        ld_t, ld_c = C, 1
+    else:
+        C, T = zt.shape
+        ld_t, ld_c = 1, T
+    nbuf = T // R
+    sd = None
+    if state is not None:
+        sd = state if isinstance(state, torch.Tensor) else torch.from_numpy(np.ascontiguousarray(state, dtype=np.float64))
+        sd = sd.to(dev, dtype=torch.float64).contiguous()
+    out = {"rows": torch.empty((C, nbuf, _lib.ROW_STRIDE), dtype=torch.float64, device=dev),
+           "var": torch.empty((C, nbuf, 5), dtype=torch.float64, device=dev),
+           "filtered": torch.empty((C, nbuf, _lib.ROW_STRIDE), dtype=torch.float64, device=dev),
+           "filtered_var": torch.empty((C, nbuf, 5), dtype=torch.float64, device=dev)}
     with torch.cuda.device(dev):
         ctx.use_torch_stream()
         try:
-            ctx.ekf_dev(zt.data_ptr(), T, C, ld_t, ld_c, R, float(f_samp), float(f_mod), opts, rows.data_ptr())
+            ctx.ekf_smooth_dev(zt.data_ptr(), T, C, ld_t, ld_c, R, float(f_samp), float(f_mod), opts, k0,
+                               sd.data_ptr() if sd is not None else None, block, out["rows"].data_ptr(),
+                               out["var"].data_ptr(), out["filtered"].data_ptr(), out["filtered_var"].data_ptr())
         finally:
             ctx.use_default_stream()
         torch.cuda.current_stream(dev).synchronize()
-    return rows if return_tensor else rows.cpu().numpy()
+    return out if return_tensor else {k: v.cpu().numpy() for k, v in out.items()}

@@ -230,6 +230,33 @@ int dfk_ekf_stream_dev(dfk_ctx* ctx, const double* z_dev, int64_t T, int64_t C, 
                        int64_t R, double f_samp, double f_mod, const dfk_ekf_opts* opts, int64_t k0,
                        double* state_dev, double* rows_dev);
 
+/* Fixed-interval (Rauch-Tung-Striebel) smoother of the same filter over a resident window: the state at each snapshot
+ * given the whole window, with its variance.  The window is the T samples k0 .. k0+T-1 of every channel (k0 a multiple
+ * of R; 0 for a whole record), laid out as for dfk_ekf_dev.  Let x_f[k], P_f[k] be the filter's state and covariance
+ * after the update with sample k, the pending update applied (exactly what dfk_ekf_dev's filter carries).  With F = I:
+ *     x_s[T-1] = x_f[T-1],  P_s[T-1] = P_f[T-1];  for k = T-2 .. 0:
+ *     Pp = P_f[k] + diag(q)   (the filter's own prediction for step k+1),   G = P_f[k] Pp^-1   (5x5 Cholesky of Pp),
+ *     x_s[k] = x_f[k] + G (x_s[k+1] - x_f[k]),   P_s[k] = P_f[k] + G (P_s[k+1] - Pp) G^T
+ * i.e. the Kalman smoother of the linearisation the filter used.  Outputs at the snapshots k_b = (b+1) R - 1, b < T / R
+ * (the samples after the last snapshot still count as data):
+ *     rows_dev      C x nbuf x DFK_ROW_STRIDE  smoothed [a, m, phi, psi, dc, 0, 1, 0] (the EKF row layout)
+ *     var_dev       C x nbuf x 5               diag P_s[k_b]
+ *     filt_rows_dev C x nbuf x DFK_ROW_STRIDE  filtered rows, bit-identical to dfk_ekf_dev's / dfk_ekf_stream_dev's
+ *     filt_var_dev  C x nbuf x 5               diag P_f[k_b]
+ * rows_dev is required; the others may be NULL.  Prior: state_dev == NULL (only allowed with k0 == 0) starts from opts
+ * as dfk_ekf_dev does, NaN init_dc / r_val taken from the window's mean and variance; otherwise the window starts from
+ * state_dev (C x 32, the layout of dfk_ekf_stream_dev), which is read and never written -- how the tail of a long
+ * record filtered slab by slab is smoothed.  A non-positive or NaN Cholesky pivot, or a NaN sample, makes that
+ * channel's smoothed states and variances NaN from that step back to the window's start; filtered outputs and other
+ * channels are unaffected.
+ * block: the checkpoint interval B, a positive multiple of 32, or 0 for the library's choice; results do not depend on
+ * it.  Scratch (context-owned): C (ceil(T / B) + B) 20 doubles, B capped at T rounded up to 32; DFK_ERR_NOMEM names
+ * the byte count when it does not fit.  Launches: the channel statistics when they are needed (one launch channel-
+ * major, three time-major), then a forward and a backward kernel.  T < R writes nothing. */
+int dfk_ekf_smooth_dev(dfk_ctx* ctx, const double* z_dev, int64_t T, int64_t C, int64_t ld_t, int64_t ld_c, int64_t R,
+                       double f_samp, double f_mod, const dfk_ekf_opts* opts, int64_t k0, const double* state_dev,
+                       int64_t block, double* rows_dev, double* var_dev, double* filt_rows_dev, double* filt_var_dev);
+
 /* 'snr'-mode synthetic record (physics.py:475-530) generated on the device with a counter-based
  * RNG: y = A(1 + C cos(phi0 + m cos(2 pi f_mod t + psi0))) + sigma N(0,1), sigma from snr_db.
  * Statistically (not bitwise) equivalent to the reference's MT19937 stream.  C channels,
