@@ -24,6 +24,9 @@ TRIAL_STATS_DOUBLES = 6
 SCHED_INDEPENDENT = 0   # every buffer a cold start from init
 SCHED_EACH = -1         # every buffer its own chunk, seeded from buffer 0 (pool schedule at n_cores >= nbuf - 1)
 ROW_COLUMNS = ("amp", "m", "phi", "psi", "dc", "ssq", "fitok")
+STAB_PHASE, STAB_FREQ = 0, 1                   # DFK_STAB_PHASE, DFK_STAB_FREQ
+STAB_KINDS = ("oadev", "mdev", "tdev", "ohdev")  # the slot order of dfk_stability_dev's outputs
+STAB_BITS = {"oadev": 1, "mdev": 2, "tdev": 4, "ohdev": 8}
 
 c_double_p = ctypes.POINTER(ctypes.c_double)
 
@@ -138,6 +141,7 @@ SYMBOLS = {
                                          _vp, _vp, _vp, _vp]),
     "dfk_wiener_dev": (ctypes.c_int, [_vp, _vp, _i64, _i64, _vp, _i64, _i64, _i64, _i64, _i64, _i64, _d, _vp, _i64, _vp,
                                       _vp, _vp, ctypes.POINTER(_i32)]),
+    "dfk_stability_dev": (ctypes.c_int, [_vp, _vp, _i64, _i64, _i64, _i64, _d, _i32, _i32, _vp, _i32, _vp, _vp]),
     "dfk_lm_counters_read": (ctypes.c_int, [_vp, ctypes.POINTER(LmCounters), _i32]),
     "dfk_profile_enable": (ctypes.c_int, [_vp, _i32]),
     "dfk_profile_read": (ctypes.c_int, [_vp, c_double_p, ctypes.POINTER(_i64), _i32]),
@@ -583,6 +587,18 @@ class Context:
                                                  taps, int(lead), float(ridge), res_ptr, int(ld_res), ptr(h),
                                                  ptr(var_y), ptr(var_res), ctypes.byref(singular)))
         return {"h": h, "var_y": var_y, "var_res": var_res, "singular": bool(singular.value)}
+
+    def stability_dev(self, v_ptr, N, stride, C, ld_c, fs, data_type, kinds, m):
+        """Stability deviations of C device-resident series (dfk_stability_dev) at the averaging factors ``m``.
+        ``data_type``: STAB_PHASE or STAB_FREQ; ``kinds``: a bitmask of STAB_BITS.  Returns host arrays dev[4, C, n_m]
+        and n[4, n_m] in STAB_KINDS order; slots of kinds not requested stay NaN and 0."""
+        ms = np.ascontiguousarray(m, dtype=np.int64)
+        dev = np.full((4, int(C), ms.size), np.nan)
+        n = np.zeros((4, ms.size), dtype=np.int64)
+        _check(self.lib, self.lib.dfk_stability_dev(self._h, v_ptr, int(N), int(stride), int(C), int(ld_c), float(fs),
+                                                    int(data_type), int(kinds), ms.ctypes.data, ms.size,
+                                                    dev.ctypes.data, n.ctypes.data))
+        return dev, n
 
     def set_host_slab_bytes(self, nbytes=0):
         """Slab size of the host-pointer entries (0: defaults); small values make a short record stream."""

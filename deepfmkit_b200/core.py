@@ -211,6 +211,16 @@ class DeepFitObject:
         xs, y = self._witness_series(witness_fits, column)
         return wiener_subtract(xs, np.asarray(y, dtype=np.float64), taps, lead, ridge)
 
+    def calc_stability(self, column="phi", kinds=("oadev", "mdev", "tdev", "ohdev"), taus="octave"):
+        """Time-domain stability of this fit's ``column`` on the device: the ``stability`` dict (taus, m and, per kind,
+        the deviation, its simple error and its term count) with the column as the averaged series (``data_type``
+        "freq") at the fit rate, so the deviations are in the column's units.  Stores nothing."""
+        from .spectra import stability
+        x = getattr(self, column)
+        if x is None:
+            raise ValueError(f"this fit has no '{column}' series")
+        return stability(np.asarray(x, dtype=np.float64), self.fs, kinds=kinds, taus=taus, data_type="freq")
+
     def _witness_series(self, witness_fits, column):
         """([Cx, N] witness columns, this fit's column) after checking that there is at least one witness fit and that
         every fit has this fit's rate and length."""

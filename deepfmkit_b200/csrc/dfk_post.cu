@@ -1,11 +1,12 @@
-// Post-fit entries of the C ABI (include/dfk_b200.h, "post-fit step"): block means, log-frequency spectra and
-// time-domain witness subtraction.
+// Post-fit entries of the C ABI (include/dfk_b200.h, "post-fit step"): block means, log-frequency spectra,
+// time-domain witness subtraction and time-domain stability.
 #include "dfk_host.h"
 
 #include <cmath>
 #include <vector>
 
 #include "dfk_spectra.cuh"
+#include "dfk_stability.cuh"
 #include "dfk_wiener.cuh"
 
 namespace {
@@ -570,6 +571,173 @@ int dfk_wiener_dev(dfk_ctx* ctx, const double* x_dev, int64_t Cx, int64_t ldx, c
     DFK_CUDA(cudaMemcpyAsync(&flag, flag_dev, sizeof(int32_t), cudaMemcpyDeviceToHost, st));
     DFK_CUDA(cudaStreamSynchronize(st));
     if (singular_out) *singular_out = flag;
+    return DFK_OK;
+}
+
+int dfk_stability_dev(dfk_ctx* ctx, const double* v_dev, int64_t N, int64_t stride, int64_t C, int64_t ld_c, double fs,
+                      int32_t data_type, int32_t kinds, const int64_t* m_host, int32_t n_m, double* dev_host,
+                      int64_t* n_host) {
+    DFK_ENTER(ctx);
+    if (!v_dev || !m_host || !dev_host || !n_host) return fail(DFK_ERR_ARG, "null pointer");
+    if (C < 1 || stride < 1) return fail(DFK_ERR_ARG, "bad geometry: C=%lld stride=%lld", (long long)C, (long long)stride);
+    if (!(fs > 0.0) || !std::isfinite(fs)) return fail(DFK_ERR_ARG, "fs must be positive and finite");
+    if (data_type != DFK_STAB_PHASE && data_type != DFK_STAB_FREQ)
+        return fail(DFK_ERR_ARG, "unknown data_type %d (0 phase, 1 freq)", data_type);
+    if (kinds == 0 || (kinds & ~DFK_STAB_ALL)) return fail(DFK_ERR_ARG, "kinds 0x%x: a non-empty subset of 0xf", kinds);
+    const bool freq = data_type == DFK_STAB_FREQ;
+    if (N < 1 || N > (int64_t(1) << 40)) return fail(DFK_ERR_ARG, "bad length N=%lld", (long long)N);
+    const long long Nx = freq ? N + 1 : N;
+    if (Nx < 3) return fail(DFK_ERR_ARG, "%lld phase points: at least 3 are needed", Nx);
+    if (n_m < 1) return fail(DFK_ERR_ARG, "no averaging factors");
+    for (int32_t t = 0; t < n_m; ++t)
+        if (m_host[t] < 1) return fail(DFK_ERR_ARG, "averaging factor m[%d] = %lld below 1", t, (long long)m_host[t]);
+    const bool want_a = kinds & DFK_STAB_OADEV, want_m = kinds & (DFK_STAB_MDEV | DFK_STAB_TDEV),
+               want_h = kinds & DFK_STAB_OHDEV;
+
+    // the slice table: every m gets ceil(n / 4096) slices of its largest requested term count n (none when m is
+    // outside every requested kind's range); an m above Nx is clamped there, where every count is already <= 0
+    std::vector<dfk::StabSlice> slices;
+    std::vector<dfk::StabTau> taus(n_m);
+    const int slot_bits[4] = {DFK_STAB_OADEV, DFK_STAB_MDEV, DFK_STAB_TDEV, DFK_STAB_OHDEV};
+    for (int32_t t = 0; t < n_m; ++t) {
+        const long long m = std::min<long long>(m_host[t], Nx);
+        const long long na = dfk::stab_n_oadev(Nx, m), nm = dfk::stab_n_mdev(Nx, m), nh = dfk::stab_n_ohdev(Nx, m);
+        long long nmax = 0;
+        if (want_a) nmax = std::max(nmax, na);
+        if (want_m) nmax = std::max(nmax, nm);
+        if (want_h) nmax = std::max(nmax, nh);
+        const long long ns = (nmax + dfk::kStabSlice - 1) / dfk::kStabSlice;
+        taus[t] = {m, static_cast<long long>(slices.size()), ns};
+        for (long long s = 0; s < ns; ++s) slices.push_back({m, s * dfk::kStabSlice});
+        if (slices.size() > (size_t(1) << 31)) return fail(DFK_ERR_ARG, "stability problem too large for one launch");
+        const long long n_slot[4] = {na, nm, nm, nh};
+        for (int k = 0; k < 4; ++k)
+            if (kinds & slot_bits[k]) n_host[k * n_m + t] = std::max(0ll, n_slot[k]);
+    }
+    const long long nslices = static_cast<long long>(slices.size());
+    const long long ld = Nx + 1;
+    const long long in_len = freq ? N : Nx;  // samples the X pass reads
+    const long long tiles_x = (in_len + dfk::kStabTile - 1) / dfk::kStabTile;
+    const long long tiles_s = (Nx + dfk::kStabTile - 1) / dfk::kStabTile;
+    if (nslices * C > 0x7fffffffll || tiles_s * C > 0x7fffffffll)
+        return fail(DFK_ERR_ARG, "stability problem too large for one launch");
+
+    // post[0]: X [C][Nx + 1] double-double; post[1]: S, the same, when mdev or tdev is requested; post[2]: tile sums
+    // [C][tiles], slices, taus, partials [C][nslices][3], outputs [4][C][n_m], flags [C]
+    const auto align = [](size_t b) { return (b + 255) & ~static_cast<size_t>(255); };
+    const size_t rows_b = static_cast<size_t>(C) * static_cast<size_t>(ld) * sizeof(double2);
+    const size_t tsum_b = align(sizeof(double2) * static_cast<size_t>(C) * static_cast<size_t>(std::max(tiles_x, tiles_s)));
+    const size_t slice_b = align(sizeof(dfk::StabSlice) * std::max<size_t>(1, slices.size()));
+    const size_t tau_b = align(sizeof(dfk::StabTau) * static_cast<size_t>(n_m));
+    const size_t part_b = align(sizeof(double) * dfk::kStabSums * static_cast<size_t>(std::max(1ll, nslices * C)));
+    const size_t out_b = align(sizeof(double) * 4 * static_cast<size_t>(C) * static_cast<size_t>(n_m));
+    const size_t small_b = tsum_b + slice_b + tau_b + part_b + out_b + sizeof(int) * static_cast<size_t>(C);
+    DevBuf& x_buf = ctx->post[0];
+    DevBuf& s_buf = ctx->post[1];
+    DevBuf& small_buf = ctx->post[2];
+    {
+        const size_t want = rows_b * (want_m ? 2 : 1) + small_b;
+        const size_t held = x_buf.bytes + (want_m ? s_buf.bytes : 0) + small_buf.bytes;
+        size_t free_b = 0, total_b = 0;
+        DFK_CUDA(cudaMemGetInfo(&free_b, &total_b));
+        if (want > free_b + held)
+            return fail(DFK_ERR_NOMEM, "stability scratch of %zu bytes (running sums of %lld x %lld points in "
+                        "double-double) does not fit the device's %zu free bytes", want, (long long)C, ld, free_b + held);
+    }
+    int rc = ensure(ctx, x_buf, rows_b);
+    if (!rc && want_m) rc = ensure(ctx, s_buf, rows_b);
+    if (!rc) rc = ensure(ctx, small_buf, small_b);
+    if (rc) return rc;
+    char* small = static_cast<char*>(small_buf.ptr);
+    double2* tsum_dev = reinterpret_cast<double2*>(small);
+    auto* slice_dev = reinterpret_cast<dfk::StabSlice*>(small + tsum_b);
+    auto* tau_dev = reinterpret_cast<dfk::StabTau*>(small + tsum_b + slice_b);
+    double* part_dev = reinterpret_cast<double*>(small + tsum_b + slice_b + tau_b);
+    double* out_dev = reinterpret_cast<double*>(small + tsum_b + slice_b + tau_b + part_b);
+    int* bad_dev = reinterpret_cast<int*>(small + tsum_b + slice_b + tau_b + part_b + out_b);
+    double2* X = static_cast<double2*>(x_buf.ptr);
+    double2* S = want_m ? static_cast<double2*>(s_buf.ptr) : nullptr;
+    cudaStream_t st = ctx->stream();
+    if (nslices)
+        DFK_CUDA(cudaMemcpyAsync(slice_dev, slices.data(), sizeof(dfk::StabSlice) * nslices, cudaMemcpyHostToDevice, st));
+    DFK_CUDA(cudaMemcpyAsync(tau_dev, taus.data(), sizeof(dfk::StabTau) * n_m, cudaMemcpyHostToDevice, st));
+    DFK_CUDA(cudaMemsetAsync(bad_dev, 0, sizeof(int) * C, st));
+    long long launches = 0;
+
+    // running sums as exclusive scans: out[0] = 0, out[k] = sum_{i<k} in_i (tile sums, carries, write)
+    auto scan = [&](dfk::StabScanParams P, bool dd) -> int {
+        const unsigned grid = static_cast<unsigned>(P.ntiles * C);
+        if (dd)
+            dfk::stab_scan_kernel<true, false><<<grid, dfk::kStabScanThreads, 0, st>>>(P);
+        else
+            dfk::stab_scan_kernel<false, false><<<grid, dfk::kStabScanThreads, 0, st>>>(P);
+        DFK_CUDA(cudaGetLastError());
+        dfk::stab_carry_kernel<<<static_cast<unsigned>((C + 3) / 4), 128, 0, st>>>(P.tsum, P.ntiles, C);
+        DFK_CUDA(cudaGetLastError());
+        if (dd)
+            dfk::stab_scan_kernel<true, true><<<grid, dfk::kStabScanThreads, 0, st>>>(P);
+        else
+            dfk::stab_scan_kernel<false, true><<<grid, dfk::kStabScanThreads, 0, st>>>(P);
+        DFK_CUDA(cudaGetLastError());
+        launches += 3;
+        return DFK_OK;
+    };
+    dfk::StabScanParams P;
+    P.v = v_dev;
+    P.X = nullptr;
+    P.ld_c = ld_c;
+    P.stride = stride;
+    P.L = in_len;
+    P.ntiles = tiles_x;
+    P.tsum = tsum_dev;
+    P.out = X;
+    P.ld_out = ld;
+    P.bad = bad_dev;
+    if (freq) {
+        rc = scan(P, false);
+        if (rc) return rc;
+    } else {
+        dfk::stab_load_kernel<<<static_cast<unsigned>(tiles_x * C), dfk::kStabScanThreads, 0, st>>>(P);
+        DFK_CUDA(cudaGetLastError());
+        ++launches;
+    }
+    if (want_m) {
+        dfk::StabScanParams Q = P;
+        Q.v = nullptr;
+        Q.X = X;
+        Q.ld_c = ld;
+        Q.stride = 1;
+        Q.L = Nx;
+        Q.ntiles = tiles_s;
+        Q.out = S;
+        rc = scan(Q, true);
+        if (rc) return rc;
+    }
+    dfk::StabTermsParams T;
+    T.X = X;
+    T.S = S;
+    T.ld = ld;
+    T.Nx = Nx;
+    T.slices = slice_dev;
+    T.nslices = nslices;
+    T.want_a = want_a;
+    T.want_m = want_m;
+    T.want_h = want_h;
+    T.part = part_dev;
+    dfk::stab_terms_kernel<<<static_cast<unsigned>(std::max(1ll, nslices * C)), dfk::kStabTermThreads, 0, st>>>(T);
+    DFK_CUDA(cudaGetLastError());
+    const long long nout = C * n_m;
+    dfk::stab_finish_kernel<<<static_cast<unsigned>((nout + dfk::kStabFinishThreads - 1) / dfk::kStabFinishThreads),
+                              dfk::kStabFinishThreads, 0, st>>>(tau_dev, n_m, C, part_dev, nslices, bad_dev, Nx, fs,
+                                                                freq ? 1.0 : fs, out_dev);
+    DFK_CUDA(cudaGetLastError());
+    launches += 2;
+    ctx->launches += launches;
+    for (int k = 0; k < 4; ++k)
+        if (kinds & slot_bits[k])
+            DFK_CUDA(cudaMemcpyAsync(dev_host + k * nout, out_dev + k * nout, sizeof(double) * nout,
+                                     cudaMemcpyDeviceToHost, st));
+    DFK_CUDA(cudaStreamSynchronize(st));
     return DFK_OK;
 }
 

@@ -8,7 +8,9 @@ the reference stores as ``Sxx``.  ``lcsd`` is the cross-spectral counterpart on 
 coherence and transfer function between fitted channels.  ``lcsd_conditioned`` extends it to several witnesses at
 once: the joint transfer functions, the conditioned (residual) PSD and the multiple coherence of each target given all
 witnesses.  ``wiener_subtract`` does that subtraction in the time domain: least-squares multi-input FIR filters and
-the cleaned target series.  All run on the device only.
+the cleaned target series.  ``stability`` (and its one-kind forms ``oadev``, ``mdev``, ``tdev``, ``ohdev``) gives the
+time-domain view: overlapping Allan, modified Allan, time and Hadamard deviations against the averaging time.  All run
+on the device only.
 """
 from __future__ import annotations
 
@@ -312,3 +314,142 @@ def wiener_subtract(witnesses, targets, taps, lead=None, ridge=0.0, device=0):
         for k in ("h", "residual", "var_y", "var_res", "explained"):
             result[k] = result[k][0]
     return result
+
+
+STABILITY_KINDS = _lib.STAB_KINDS
+
+
+def _stability_counts(Nx, m):
+    """Term counts [4, n_m] of each kind (STABILITY_KINDS order) at averaging factors m on Nx phase points."""
+    m = np.asarray(m, dtype=np.int64)
+    return np.stack([Nx - 2 * m, Nx - 3 * m + 1, Nx - 3 * m + 1, Nx - 3 * m])
+
+
+def _stability_m(Nx, fs, taus, kinds):
+    """The averaging factors of one call: the tau rule's m values that fall inside the range of at least one
+    requested kind (those outside every range are dropped), sorted and distinct."""
+    if isinstance(taus, str):
+        if taus == "octave":
+            m = 2 ** np.arange(int(np.floor(np.log2(Nx))) + 1, dtype=np.int64)
+        elif taus == "decade":
+            k = np.arange(int(np.floor(np.log10(Nx))) + 1, dtype=np.int64)
+            m = (np.array([1, 2, 4], dtype=np.int64)[None, :] * 10 ** k[:, None]).ravel()
+        elif taus == "all":
+            m = np.arange(1, Nx + 1, dtype=np.int64)
+        else:
+            raise ValueError(f"taus must be 'octave', 'decade', 'all' or an array of averaging times, got {taus!r}")
+    else:
+        try:
+            t = np.asarray(taus, dtype=np.float64)
+        except (TypeError, ValueError):
+            raise ValueError(f"taus must be 'octave', 'decade', 'all' or an array of averaging times, got {taus!r}")
+        if t.ndim != 1 or t.size == 0 or not np.all(np.isfinite(t)) or np.any(t <= 0):
+            raise ValueError("an array of taus must be a non-empty 1-D array of positive, finite averaging times")
+        m = np.unique(np.clip(np.rint(t * fs), 1, Nx + 1).astype(np.int64))
+    n = _stability_counts(Nx, m)[[STABILITY_KINDS.index(k) for k in kinds]]
+    return m[np.max(n, axis=0) >= 1]
+
+
+def _stability_series(x, device):
+    """(fp64 CUDA tensor [C, N] read in place where it already is one, whether the input was 1-D, ld_c, stride)."""
+    import torch
+    if isinstance(x, torch.Tensor) and x.is_cuda:
+        t = x if x.dtype == torch.float64 else x.to(torch.float64)
+    else:
+        h = np.ascontiguousarray(np.asarray(x, dtype=np.float64))
+        t = torch.from_numpy(h if h.flags.writeable else h.copy()).to(torch.device("cuda", device))
+    one = t.dim() == 1
+    if one:
+        t = t[None, :]
+    if t.stride(1) < 1:  # an expanded tensor
+        t = t.contiguous()
+    return t, one, int(t.stride(0)), int(t.stride(1))
+
+
+def stability(x, fs, kinds=STABILITY_KINDS, taus="octave", data_type="phase", device=0):
+    """Time-domain stability of one series or of every row of a 2-D array / tensor on the device: the overlapping
+    Allan ("oadev"), modified Allan ("mdev"), time ("tdev") and overlapping Hadamard ("ohdev") deviations against the
+    averaging time tau = m / fs (NIST SP 1065; the definitions and tau rules of allantools).
+
+    ``x`` is ``[N]`` or ``[C, N]``, a numpy array or a CUDA tensor (read in place on its device, strides included, so
+    a column of a row table needs no copy).  ``data_type`` "phase": x is phase-time, Nx = N points.  "freq": x is
+    fractional frequency (or any series whose averages are wanted, such as a fitted phase column), integrated as
+    x_0 = 0, x_n = sum_{i<n} y_i / fs, Nx = N + 1; the deviations come out in the series' own units.
+
+    ``taus``: "octave" (m = 1, 2, 4, ...), "decade" (m = 1, 2, 4 x 10^k), "all" (every m: O(N^2) work per series) or
+    an array of averaging times in seconds (m = round(tau fs), at least 1, sorted and distinct).  m values outside the
+    range of every requested kind are dropped; one inside some kind's range but not another's gives NaN and n = 0 for
+    the other.  Term counts n: oadev Nx - 2m, mdev and tdev Nx - 3m + 1, ohdev Nx - 3m.
+
+    Returns a dict of host arrays: ``taus`` and ``m`` [n_m], and per requested kind ``<kind>`` [C, n_m],
+    ``<kind>_err`` [C, n_m] (the simple error dev / sqrt(n) of allantools, not an EDF confidence interval) and
+    ``<kind>_n`` [n_m].  A 1-D input drops the C axis.  A NaN or infinite sample makes every deviation of its series
+    NaN.  The running sums are carried in double-double, so a drifting series keeps the differences that an fp64
+    cumulative sum would lose to cancellation; results are bit-identical between runs and for a series alone or in a
+    batch."""
+    import torch
+    if isinstance(kinds, str):
+        kinds = (kinds,)
+    kinds = tuple(kinds)
+    if not kinds or any(k not in STABILITY_KINDS for k in kinds):
+        raise ValueError(f"kinds must be a non-empty selection of {STABILITY_KINDS}, got {kinds!r}")
+    kinds = tuple(k for k in STABILITY_KINDS if k in kinds)
+    codes = {"phase": _lib.STAB_PHASE, "freq": _lib.STAB_FREQ}
+    if not isinstance(data_type, str) or data_type not in codes:
+        raise ValueError(f"data_type must be 'phase' or 'freq', got {data_type!r}")
+    if isinstance(fs, bool) or not np.isscalar(fs) or not np.isfinite(fs) or fs <= 0:
+        raise ValueError(f"fs must be positive and finite, got {fs!r}")
+    shape = tuple(x.shape) if hasattr(x, "shape") else np.shape(x)
+    if len(shape) not in (1, 2) or (len(shape) == 2 and shape[0] < 1):
+        raise ValueError(f"expected a series [N] or a batch of series [C, N], got shape {shape}")
+    N = shape[-1]
+    Nx = N + (data_type == "freq")
+    if Nx < 3:
+        raise ValueError(f"{N} samples give {Nx} phase points: at least 3 are needed")
+    m = _stability_m(Nx, float(fs), taus, kinds)
+    if m.size == 0:
+        raise ValueError(f"{N} samples are too short for any requested averaging factor of {kinds}")
+    if isinstance(x, torch.Tensor) and x.is_cuda:
+        device = x.device.index
+    t, one, ld_c, stride = _stability_series(x, device)
+    mask = sum(_lib.STAB_BITS[k] for k in kinds)
+    ctx = _lib.get_context(device)
+    with torch.cuda.device(t.device):
+        ctx.use_torch_stream()
+        try:
+            dev, n = ctx.stability_dev(t.data_ptr(), N, stride, t.shape[0], ld_c, float(fs), codes[data_type], mask, m)
+        finally:
+            ctx.use_default_stream()
+    out = {"taus": m / float(fs), "m": m}
+    for k in kinds:
+        i = STABILITY_KINDS.index(k)
+        err = np.full(dev[i].shape, np.nan)
+        np.divide(dev[i], np.sqrt(n[i].astype(np.float64)), out=err, where=n[i] > 0)
+        out[k], out[k + "_err"] = (dev[i][0], err[0]) if one else (dev[i], err)
+        out[k + "_n"] = n[i]
+    return out
+
+
+def _one_kind(kind, data, rate, data_type, taus):
+    out = stability(data, rate, kinds=(kind,), taus="octave" if taus is None else taus, data_type=data_type)
+    return out["taus"], out[kind], out[kind + "_err"], out[kind + "_n"]
+
+
+def oadev(data, rate=1.0, data_type="phase", taus=None):
+    """Overlapping Allan deviation with allantools' interface: ``(taus, dev, err, n)``; see ``stability``."""
+    return _one_kind("oadev", data, rate, data_type, taus)
+
+
+def mdev(data, rate=1.0, data_type="phase", taus=None):
+    """Modified Allan deviation with allantools' interface: ``(taus, dev, err, n)``; see ``stability``."""
+    return _one_kind("mdev", data, rate, data_type, taus)
+
+
+def tdev(data, rate=1.0, data_type="phase", taus=None):
+    """Time deviation, tau mdev / sqrt(3), with allantools' interface: ``(taus, dev, err, n)``; see ``stability``."""
+    return _one_kind("tdev", data, rate, data_type, taus)
+
+
+def ohdev(data, rate=1.0, data_type="phase", taus=None):
+    """Overlapping Hadamard deviation with allantools' interface: ``(taus, dev, err, n)``; see ``stability``."""
+    return _one_kind("ohdev", data, rate, data_type, taus)

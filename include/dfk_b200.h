@@ -503,6 +503,38 @@ int dfk_lcsd_cond_dev(dfk_ctx* ctx, const double* x_dev, int64_t Cx, int64_t ldx
 int dfk_wiener_dev(dfk_ctx* ctx, const double* x_dev, int64_t Cx, int64_t ldx, const double* y_dev, int64_t Cy,
                    int64_t ldy, int64_t N, int64_t stride, int64_t L, int64_t lead, double ridge, double* res_dev,
                    int64_t ld_res, double* h_host, double* var_y_host, double* var_res_host, int32_t* singular_out);
+/* Time-domain stability (NIST SP 1065, Riley 2008; the conventions of allantools): overlapping Allan (oadev),
+ * modified Allan (mdev), time (tdev) and overlapping Hadamard (ohdev) deviations of C device-resident series of N
+ * samples at rate fs, at the n_m averaging factors m_host (tau = m / fs).  Sample i of series c is
+ * v_dev[c * ld_c + i * stride]; stride = DFK_ROW_STRIDE reads a column of a row table in place.
+ * data_type DFK_STAB_PHASE: the series is phase-time x, Nx = N.  DFK_STAB_FREQ: the series is y, and x_0 = 0,
+ * x_n = tau0 sum_{i<n} y_i, Nx = N + 1; the deviations are in the series' own units.  With S_k = sum_{i<k} x_i:
+ *     oadev^2 = sum_{i<n} (x_{i+2m} - 2 x_{i+m} + x_i)^2 / (2 tau^2 n),                       n = Nx - 2m
+ *     mdev^2  = sum_{j<n} (S_{j+3m} - 3 S_{j+2m} + 3 S_{j+m} - S_j)^2 / (2 m^2 tau^2 n),     n = Nx - 3m + 1
+ *     tdev    = tau mdev / sqrt(3),                                                          mdev's n
+ *     ohdev^2 = sum_{i<n} (x_{i+3m} - 3 x_{i+2m} + 3 x_{i+m} - x_i)^2 / (6 tau^2 n),         n = Nx - 3m
+ * The running sums x and S are carried in double-double and every difference is rounded once to fp64 before it is
+ * squared: for a series on a grid the terms are exact while the sums stay below 2^106 grid steps, where fp64 running
+ * sums lose them to cancellation.  Where n <= 0 that kind's deviation is NaN and its n is 0.  A NaN or infinite sample
+ * makes every deviation of its series NaN.  kinds: a non-empty bitmask of DFK_STAB_OADEV .. DFK_STAB_OHDEV.
+ * Outputs: dev_host [4][C][n_m] and n_host [4][n_m] in the order oadev, mdev, tdev, ohdev; slots of kinds not
+ * requested are not written.  Sums are formed in a fixed order without atomics: results are bit-identical between
+ * runs, for a series alone or in a batch, over stride, and for an m alone or in a longer list.
+ * Scratch (context-owned): C (Nx + 1) 16 bytes for x, the same again for S when mdev or tdev is requested, plus tile
+ * sums and per-slice partials; DFK_ERR_NOMEM names the byte count when it does not fit.  DFK_ERR_ARG for a NULL
+ * pointer, C < 1, stride < 1, fs not positive, Nx < 3, unknown data_type or kinds, n_m < 1 or any m < 1.
+ * Launches: 2, plus 3 for DFK_STAB_FREQ or 1 for DFK_STAB_PHASE (x), plus 3 when mdev or tdev is requested (S).
+ * Synchronises like dfk_lpsd_dev. */
+#define DFK_STAB_PHASE 0
+#define DFK_STAB_FREQ 1
+#define DFK_STAB_OADEV 1
+#define DFK_STAB_MDEV 2
+#define DFK_STAB_TDEV 4
+#define DFK_STAB_OHDEV 8
+#define DFK_STAB_ALL 15
+int dfk_stability_dev(dfk_ctx* ctx, const double* v_dev, int64_t N, int64_t stride, int64_t C, int64_t ld_c, double fs,
+                      int32_t data_type, int32_t kinds, const int64_t* m_host, int32_t n_m, double* dev_host,
+                      int64_t* n_host);
 
 /* ---- introspection ------------------------------------------------------------------------ */
 /* Counters accumulated by the LM kernels since the last reset (device -> host copy, syncs). */
